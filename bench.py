@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg5|T|cfg1..cfg4]
     python bench.py --impl reference [...]          # the reference's CPU algorithm, host cores
+    python bench.py --dump-outputs DIR [...]        # also write the last timed step's output to DIR/*.npy
     torchrun ... bench.py --gpus N ...              # one rank per GPU (driver launches this)
 
 One JSON line on stdout (rank 0).  Metric: output Gpix/s, whole job.  ``value`` is timed over
@@ -106,19 +107,19 @@ def measured_peak_gbs():
 # --------------------------------------------------------------------------------------------
 # CPU arm: the reference's own implementation on the host cores.
 #
-# kind "reference": the UNMODIFIED reference package, copied by __graft_entry__.build() from
-# /root/reference/photonbend to the git-ignored baseline/_ref/ (it is pure Python + NumPy, so it
-# travels to the GPU box with the snapshot), driven through its own three-call protocol
+# kind "reference": the UNMODIFIED reference package, copied by __graft_entry__.build() to the
+# git-ignored oracle/_ref/ (it is pure Python + NumPy and imports as it lies), driven through its
+# own three-call protocol
 # (photonbend/core/__init__.py:66-92).  The reference is single-threaded; to use every host core
 # the coordinate map is cut into row bands, one worker process per band (the protocol takes any
 # (h, w, 3) slice of a map, bit-identically -- checked below against the golden hash).
-# kind "port": oracle/numpy_port.py, the stated fallback when baseline/_ref is absent.
+# kind "port": oracle/numpy_port.py, the stated fallback when oracle/_ref is absent.
 
-REF_DIR = os.path.join(REPO, "baseline", "_ref")
+REF_DIR = os.path.join(REPO, "oracle", "_ref")
 
 
 def live_reference():
-    """The reference's modules from baseline/_ref, or None."""
+    """The reference's modules from oracle/_ref, or None."""
     if not os.path.isdir(os.path.join(REF_DIR, "photonbend", "core")):
         return None
     if REF_DIR not in sys.path:
@@ -227,9 +228,9 @@ class CpuArm:
         return hashlib.sha256(_CPU["out"].tobytes()).hexdigest() == golden_info(self.name)["out_sha256"]
 
     def describe(self, band_rows, px, dt, steps=1):
-        what = ("the unmodified reference (baseline/_ref/photonbend, three-call protocol"
+        what = ("the unmodified reference (oracle/_ref/photonbend, three-call protocol"
                 + ("; coordinate map of the stream built once, outside the steps)" if self.stream else ")")
-                if self.ref else "oracle/numpy_port.py (NumPy restatement, bit-identical to the reference; baseline/_ref absent)")
+                if self.ref else "oracle/numpy_port.py (NumPy restatement, bit-identical to the reference; oracle/_ref absent)")
         frac = band_rows * self.procs / self.h
         return (f"{what}, {self.procs} worker processes, one row band of {band_rows} rows each per step "
                 f"({min(1.0, frac):.2f} of a {self.h}-row {self.name} frame), {dt / steps:.2f} s wall per step")
@@ -489,6 +490,32 @@ def timed_compressed_stream(torch, source, cmap, name, frames, steps):
     return dt, sum(len(j) for j in stream_in) // reps, sum(len(j) for j in out) // reps, fallbacks
 
 
+DUMP_MAX_BYTES = 48 << 20  # --dump-outputs stays under 64 MB in all
+
+
+def output_sample(torch, out):
+    """What --dump-outputs writes for one uint8 output tensor (..., C): the whole tensor as float32
+    when it fits DUMP_MAX_BYTES, else the channels of a fixed, seeded, sorted sample of its pixels
+    as ``values`` (n, C) and their coordinates, one column per leading axis (frame, row, column),
+    as ``pixels`` (float32 holds every index below 2^24 exactly)."""
+    if out.numel() * 4 <= DUMP_MAX_BYTES:
+        return {"": out.float().cpu().numpy()}
+    shape = tuple(out.shape)
+    flat = out.reshape(-1, shape[-1])
+    n = DUMP_MAX_BYTES // (4 * (shape[-1] + len(shape) - 1))
+    idx = np.sort(np.random.default_rng(0).choice(flat.shape[0], n, replace=False))
+    values = flat[torch.from_numpy(idx).to(out.device)].float().cpu().numpy()
+    pixels = np.stack(np.unravel_index(idx, shape[:-1]), axis=1).astype(np.float32)
+    return {"_values": values, "_pixels": pixels}
+
+
+def dump_outputs(directory, name, sample):
+    os.makedirs(directory, exist_ok=True)
+    for suffix, array in sample.items():
+        np.save(os.path.join(directory, f"{name}{suffix}.npy"), array)
+    log(f"[bench] wrote {', '.join(name + s + '.npy' for s in sample)} to {directory}")
+
+
 def parity_check(name, pairs):
     """Bit-compare remapped frames with the CPU oracle (oracle/pb_oracle.c on all cores; it is
     sha256-identical to the reference at full size, tests/golden).  pairs: (source HWC uint8
@@ -640,6 +667,7 @@ def run_gpu(args):
     total_ms, launch_ms = timed_kernel_steps(torch, source, cmap, batch, out, args.steps, args.warmup, dist, sampler)
     clocks = sampler.stop()
     gpu_launches = timed_kernel_steps.launches
+    dumped = output_sample(torch, out) if args.dump_outputs else None
 
     # the same steps back to back for >= --sustain-seconds: the K steps above are a burst of a few
     # milliseconds; this is what the kernel holds once the power limit has had time to act
@@ -760,6 +788,8 @@ def run_gpu(args):
         if also:
             line["also"] = also
         emit_line(line)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, "out" if world == 1 else f"out_rank{rank}", dumped)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -787,6 +817,8 @@ def run_gpu_rows(args, torch, dist, rank, local_rank, world, batch, source, cmap
     total_ms, launch_ms = timed_kernel_steps(torch, source, cmap, batch, None, args.steps, args.warmup, dist, sampler, step_fn=step)
     clocks = sampler.stop()
     gpu_launches = timed_kernel_steps.launches
+    if args.dump_outputs and len(rows) > 0:
+        dump_outputs(args.dump_outputs, "bands" if world == 1 else f"bands_rank{rank}", output_sample(torch, bands))
     (total_ms,) = max_over_ranks([total_ms], device="cuda")
     ms_per_step = total_ms / args.steps
     px_per_step = info["out_pixels"] * frames
@@ -906,7 +938,18 @@ def main():
     ap.add_argument("--no-also", action="store_true")
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per launch from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed to DIR/<name>.npy as float32 "
+                         "(a fixed, seeded sample of its pixels when the output is larger than 48 MB as float32); "
+                         "the synthetic inputs depend on the arguments only, so two builds can be compared. "
+                         "GPU path only: a step of --impl reference covers row bands whose height is chosen "
+                         "from a timing, so its output differs from run to run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: a step of --impl reference covers row bands sized from a "
+                 "timing, so what it computes is not the same from run to run")
     claim_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
