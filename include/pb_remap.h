@@ -19,7 +19,10 @@
  *    allocates and owns every buffer; the library allocates nothing that outlives a call, except
  *    the small tables owned by a pb_plan (see below);
  *  - source images may have at most 32767 rows and 65535 columns;
- *  - images are uint8, HWC, tightly packed (row pitch = width * channels);
+ *  - images are HWC, tightly packed (row pitch = width * channels elements): uint8 for the _u8
+ *    entry points; the _px entry points take elements of 1, 2, 4 or 8 bytes of any type (a pixel
+ *    is copied as bytes, never converted), except from a double-fisheye source, whose blend is
+ *    uint8 arithmetic;
  *  - coordinate maps are float64 (H, W, 3) = (latitude, longitude, invalid != 0), tightly packed
  *    (photonbend/core/__init__.py:42-49);
  *  - all work is enqueued on `stream` (a cudaStream_t, NULL = the default stream) and the call
@@ -93,7 +96,7 @@ typedef struct pb_image_desc {
 typedef struct pb_remap_desc {
     pb_image_desc out;
     pb_image_desc src;
-    int32_t channels;    /* 1..4 interleaved uint8 channels */
+    int32_t channels;    /* 1..4 interleaved channels (uint8, or the element width of a _px call) */
     int32_t n_rotations; /* 0..PB_MAX_ROTATIONS */
     double rotations[PB_MAX_ROTATIONS][9]; /* row-major Rotation.rotation_matrix, in order */
 } pb_remap_desc;
@@ -143,6 +146,21 @@ int pb_plan_remap_u8(const pb_plan *plan, const uint8_t *src, int64_t src_frame_
  */
 int pb_plan_remap_rows_u8(const pb_plan *plan, const uint8_t *src, uint8_t *dst_band,
                           int32_t row_begin, int32_t row_end, void *stream);
+/*
+ * Like the _u8 entry points, for pixels of desc->channels elements of elem_bytes (1, 2, 4 or 8)
+ * bytes each (uint16, float16, bfloat16, float32, int32, float64 ...); strides in bytes.  Every
+ * output pixel is a bit-for-bit copy of the source pixel the reference's index picks, or all-zero
+ * bytes.  elem_bytes == 1 is exactly the _u8 call.  src / dst aligned to elem_bytes.  One plan
+ * serves every element width: the width is a property of the call.  Errors, before any device
+ * work: elem_bytes not in {1, 2, 4, 8} -> PB_ERR_UNSUPPORTED; a double-fisheye source with
+ * elem_bytes > 1 -> PB_ERR_UNSUPPORTED (its blend is uint8 arithmetic, projection.py:459); a null
+ * pointer, or a pointer / stride not a multiple of elem_bytes -> PB_ERR_INVALID_ARGUMENT.  A batch
+ * is one kernel launch whatever n_frames is.
+ */
+int pb_plan_remap_px(const pb_plan *plan, int32_t elem_bytes, const void *src, int64_t src_frame_stride,
+                     void *dst, int64_t dst_frame_stride, int32_t n_frames, void *stream);
+int pb_plan_remap_rows_px(const pb_plan *plan, int32_t elem_bytes, const void *src, void *dst_band,
+                          int32_t row_begin, int32_t row_end, void *stream);
 void pb_plan_destroy(pb_plan *plan);
 
 /*
@@ -168,6 +186,9 @@ int pb_rotate_map_f64(const double matrix[9], double *map_in, double *map_out, i
 int pb_gather_from_map_u8(const pb_image_desc *src_desc, int32_t channels, double *map,
                           int32_t map_height, int32_t map_width, const uint8_t *src, uint8_t *dst,
                           void *stream);
+/* The same for elements of elem_bytes (1, 2, 4 or 8) bytes, with the errors of pb_plan_remap_px. */
+int pb_gather_from_map_px(const pb_image_desc *src_desc, int32_t channels, int32_t elem_bytes, double *map,
+                          int32_t map_height, int32_t map_width, const void *src, void *dst, void *stream);
 
 /*
  * map_projection (projection.py:550-599) on an explicit map (device, float64 map_height x

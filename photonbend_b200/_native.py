@@ -42,6 +42,9 @@ EXPORTS = (
     "pb_map_projection_u8",
     "pb_debug_fast32_stats",
     "pb_debug_plan_fast32",
+    "pb_plan_remap_px",
+    "pb_plan_remap_rows_px",
+    "pb_gather_from_map_px",
 )
 
 
@@ -123,6 +126,12 @@ def load():
     lib.pb_debug_fast32_stats.argtypes = [ctypes.POINTER(RemapDesc), ctypes.POINTER(ctypes.c_double), vp]
     lib.pb_debug_plan_fast32.restype = ctypes.c_int
     lib.pb_debug_plan_fast32.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
+    lib.pb_plan_remap_px.restype = ctypes.c_int
+    lib.pb_plan_remap_px.argtypes = [vp, i32, vp, i64, vp, i64, i32, vp]
+    lib.pb_plan_remap_rows_px.restype = ctypes.c_int
+    lib.pb_plan_remap_rows_px.argtypes = [vp, i32, vp, vp, i32, i32, vp]
+    lib.pb_gather_from_map_px.restype = ctypes.c_int
+    lib.pb_gather_from_map_px.argtypes = [ctypes.POINTER(ImageDesc), i32, i32, vp, i32, i32, vp, vp, vp]
     _lib = lib
     return lib
 

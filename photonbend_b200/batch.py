@@ -48,7 +48,8 @@ def shard_rows(height: int, rank: int, world_size: int, align: int = ROW_BAND_AL
 
 def remap_row_band(source, coordinate_map: CoordinateMap, frame, rows: range, out=None):
     """Rows ``rows`` (a contiguous range) of the remap of ONE device frame: the band alone, as a
-    (len(rows), Wo, C) CUDA tensor.  ``frame`` is the whole source image on this device."""
+    (len(rows), Wo, C) CUDA tensor of the frame's dtype.  ``frame`` is the whole source image on
+    this device."""
     if not (isinstance(coordinate_map, CoordinateMap) and coordinate_map.is_lazy):
         raise ValueError("remap_row_band needs the lazy CoordinateMap of get_coordinate_map()")
     if rows.step != 1:
@@ -70,10 +71,11 @@ def max_over_ranks(values, device="cpu"):
 
 
 def remap_batch(source, coordinate_map: CoordinateMap, frames, out=None):
-    """Remap a device batch ``frames`` (uint8 CUDA tensor (N, H, W, C)) that shares the geometry
+    """Remap a device batch ``frames`` (CUDA tensor (N, H, W, C) of any dtype the remap takes, see
+    ``engine.ELEM_BYTES``) that shares the geometry
     of ``source`` (a CameraImage / DoubleCameraImage / PanoramaImage whose own ``image`` is only
     used for its shape) along ``coordinate_map``.  One kernel launch; returns the (N, Ho, Wo, C)
-    CUDA tensor."""
+    CUDA tensor of the same dtype."""
     if not (isinstance(coordinate_map, CoordinateMap) and coordinate_map.is_lazy):
         raise ValueError("remap_batch needs the lazy CoordinateMap of get_coordinate_map()")
     if frames.dim() != 4 or not frames.is_cuda:
@@ -131,7 +133,7 @@ class FramePipeline:
             src_dev = self._src_bufs[slot]
             if self._dst_bufs[slot] is None:
                 oh, ow = self.output_shape
-                self._dst_bufs[slot] = torch.empty((self._batch, oh, ow) + tuple(src_dev.shape[3:]), dtype=torch.uint8,
+                self._dst_bufs[slot] = torch.empty((self._batch, oh, ow) + tuple(src_dev.shape[3:]), dtype=src_dev.dtype,
                                                    device=self._device)
             dst_dev = self._dst_bufs[slot]
             if n == 1:  # one frame: the single-frame kernels
@@ -147,16 +149,18 @@ class FramePipeline:
         return done
 
     def submit(self, host_frame, host_out):
-        """Enqueue one frame: host_frame (uint8 CPU tensor (H, W, C)) -> host_out (uint8 CPU
-        tensor (Ho, Wo, C)).  Returns immediately: the completion event of the launch when this
+        """Enqueue one frame: host_frame (CPU tensor (H, W, C) of any dtype the remap takes) ->
+        host_out (CPU tensor (Ho, Wo, C) of the same dtype).  Returns immediately: the completion event of the launch when this
         frame completed a batch, else None."""
         torch = self._torch
         slot = self._slot
         stream = self._streams[slot]
         with torch.cuda.device(self._device), torch.cuda.stream(stream):
             want = (self._batch,) + tuple(host_frame.shape)
-            if self._src_bufs[slot] is None or tuple(self._src_bufs[slot].shape) != want:
-                self._src_bufs[slot] = torch.empty(want, dtype=torch.uint8, device=self._device)
+            buf = self._src_bufs[slot]
+            if buf is None or tuple(buf.shape) != want or buf.dtype != host_frame.dtype:
+                engine.check_source(self._src_geom, host_frame)
+                self._src_bufs[slot] = torch.empty(want, dtype=host_frame.dtype, device=self._device)
                 self._dst_bufs[slot] = None
             self._src_bufs[slot][len(self._pending[slot])].copy_(host_frame, non_blocking=True)
         self._pending[slot].append(host_out)

@@ -6,10 +6,14 @@
     Rotation(...).rotate_coordinate_map(map)    -> lazy CoordinateMap with one more matrix
     source.process_coordinate_map(map)          -> ONE fused kernel: ray -> rotate -> index -> sample
 
-Images are uint8 HWC (or HW) and may be NumPy arrays, torch CPU tensors (pin them for truly
+Images are HWC (or HW) and may be NumPy arrays, torch CPU tensors (pin them for truly
 asynchronous copies) or torch CUDA tensors (device resident: no copies at all, and
-``(N, H, W, C)`` batches of frames that share the geometry are remapped by one launch).  The
-result comes back in the same flavour as the source image.
+``(N, H, W, C)`` batches of frames that share the geometry are remapped by one launch).  Their
+elements may be bool, int8, uint8, int16, uint16, float16, bfloat16 (torch), int32, uint32,
+float32, int64, uint64 or float64: like the reference's fancy indexing, every output pixel is a
+bit-for-bit copy of the source pixel its index picks (0 where there is none).  A double-fisheye
+source must be uint8 (the reference casts its blend to uint8).  The result comes back in the same
+dtype and flavour as the source image.
 """
 
 from __future__ import annotations
@@ -88,7 +92,7 @@ class _DeviceSampler:
         return CoordinateMap(engine.RayPlan(self._output_geometry()))
 
     def process_coordinate_map(self, coordinate_map, out=None):
-        """Sample this image along ``coordinate_map`` and return the new uint8 image.
+        """Sample this image along ``coordinate_map`` and return the new image (same dtype).
 
         Args:
             coordinate_map: a CoordinateMap from ``get_coordinate_map`` /
@@ -98,7 +102,8 @@ class _DeviceSampler:
                 (a pinned torch CPU tensor makes the device-to-host copy asynchronous).
         """
         src_geom = self._source_geometry()
-        src_dev = engine.to_device_u8(self.image)
+        engine.check_source(src_geom, self.image)  # before any device work
+        src_dev = engine.to_device(self.image)
 
         if isinstance(coordinate_map, CoordinateMap) and coordinate_map.is_lazy \
                 and len(coordinate_map.rays.rotations) <= _native.PB_MAX_ROTATIONS:
@@ -141,7 +146,7 @@ class CameraImage(_DeviceSampler):
     """A photo taken through a lens: maps pixels to (latitude, longitude) and back.
 
     Attributes:
-        image: the uint8 image, shape (height, width, channels).
+        image: the image, shape (height, width, channels), of any dtype the remap takes.
         fov (float): field of view in radians.
         forward_lens / reverse_lens: the lens functions.
         magnitude (float): distance in pixels from the image centre at which ``fov / 2`` is
@@ -184,7 +189,8 @@ class DoubleCameraImage(_DeviceSampler):
     """A 360-degree camera frame: two opposite fisheye sensors stored side by side.
 
     Attributes:
-        image: the uint8 image, shape (height, width, channels); each half is width // 2 wide.
+        image: the uint8 image, shape (height, width, channels); each half is width // 2 wide
+            (uint8 only: the reference blends the two lenses and casts the blend to uint8).
         sensor_fov (float): field of view of ONE sensor in radians (> pi for full coverage).
         lens (Lens), forward_lens, reverse_lens: the lens model of both sensors.
         magnitude (float): always height / 2 (a ``magnitude=`` keyword is accepted and ignored).
@@ -223,7 +229,7 @@ class PanoramaImage(_DeviceSampler):
     """An equirectangular panorama (width = 2 x height).
 
     Attributes:
-        image: the uint8 image, shape (height, width, channels).
+        image: the image, shape (height, width, channels), of any dtype the remap takes.
     """
 
     def __init__(self, image_arr) -> None:

@@ -19,6 +19,7 @@
 #include "pb_sep1.cuh"
 #include "pb_chunk.cuh"
 #include "pb_tiled2.cuh"
+#include "pb_wide.cuh"
 
 namespace pb {
 
@@ -374,14 +375,16 @@ struct RemapArgs {
     int row_begin, row_end;  // output rows this launch covers; dst_px points at row row_begin
 };
 
-template <int C>
-__device__ __forceinline__ void copy_px(unsigned char* __restrict__ d, const unsigned char* __restrict__ s) {
+// one pixel of C elements of T (uint8 images: T = unsigned char; wider elements: the unsigned
+// integer of their width, so that the bytes move unconverted)
+template <int C, typename T = unsigned char>
+__device__ __forceinline__ void copy_px(T* __restrict__ d, const T* __restrict__ s) {
 #pragma unroll
     for (int c = 0; c < C; ++c) d[c] = __ldg(s + c);
 }
 
-template <int C>
-__device__ __forceinline__ void zero_px(unsigned char* __restrict__ d) {
+template <int C, typename T = unsigned char>
+__device__ __forceinline__ void zero_px(T* __restrict__ d) {
 #pragma unroll
     for (int c = 0; c < C; ++c) d[c] = 0;
 }
@@ -628,11 +631,14 @@ __global__ void __launch_bounds__(256) rotate_map_kernel(const __grid_constant__
     out[p * 3 + 2] = r.invalid ? 1.0 : 0.0;
 }
 
-template <int SRC_KIND, int C>
+// T: one element of the image (unsigned char; for a camera / equirect source also the unsigned
+// integer of a 2, 4 or 8-byte element -- the copy moves bytes, it converts nothing)
+template <int SRC_KIND, int C, typename T = unsigned char>
 __global__ void __launch_bounds__(256) gather_from_map_kernel(const __grid_constant__ SrcGeom src,
                                                               double* __restrict__ map, long long n,
-                                                              const unsigned char* __restrict__ sp,
-                                                              unsigned char* __restrict__ dst) {
+                                                              const T* __restrict__ sp,
+                                                              T* __restrict__ dst) {
+    static_assert(SRC_KIND != PB_KIND_DOUBLE || sizeof(T) == 1, "the double-fisheye blend is uint8 arithmetic");
     const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
     Ray r;
@@ -646,10 +652,10 @@ __global__ void __launch_bounds__(256) gather_from_map_kernel(const __grid_const
     const Lookup L = source_lookup<SRC_KIND>(src, r);
     const int off0 = xy_to_offset(L.xy0, src.W);
     const int off1 = xy_to_offset(L.xy1, src.W);
-    unsigned char* dp = dst + p * C;
-    if (SRC_KIND != PB_KIND_DOUBLE) {
-        if (off0 >= 0) copy_px<C>(dp, sp + (long long)off0 * C);
-        else zero_px<C>(dp);
+    T* dp = dst + p * C;
+    if constexpr (SRC_KIND != PB_KIND_DOUBLE) {
+        if (off0 >= 0) copy_px<C, T>(dp, sp + (long long)off0 * C);
+        else zero_px<C, T>(dp);
     } else {
         if (r.invalid) {
             zero_px<C>(dp);
@@ -840,6 +846,63 @@ static void launch_gather_c(const SrcGeom& s, double* map, long long n, const un
         case 3: gather_from_map_kernel<SRC_KIND, 3><<<grid, block, 0, st>>>(s, map, n, sp, dst); PB_COUNT_LAUNCH(); break;
         default: gather_from_map_kernel<SRC_KIND, 4><<<grid, block, 0, st>>>(s, map, n, sp, dst); PB_COUNT_LAUNCH(); break;
     }
+}
+
+// the same for elements of T (2, 4 or 8 bytes), camera / equirect sources
+template <int SRC_KIND, typename T>
+static void launch_gather_wide(const SrcGeom& s, double* map, long long n, const void* src, void* dst, cudaStream_t st) {
+    const int block = 256;
+    const unsigned grid = (unsigned)((n + block - 1) / block);
+    const T* sp = static_cast<const T*>(src);
+    T* dp = static_cast<T*>(dst);
+    switch (s.C) {
+        case 1: gather_from_map_kernel<SRC_KIND, 1, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
+        case 2: gather_from_map_kernel<SRC_KIND, 2, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
+        case 3: gather_from_map_kernel<SRC_KIND, 3, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
+        default: gather_from_map_kernel<SRC_KIND, 4, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
+    }
+    PB_COUNT_LAUNCH();
+}
+
+template <int SRC_KIND>
+static void launch_gather_e(const SrcGeom& s, int elem_bytes, double* map, long long n, const void* src, void* dst,
+                            cudaStream_t st) {
+    switch (elem_bytes) {
+        case 2: launch_gather_wide<SRC_KIND, unsigned short>(s, map, n, src, dst, st); break;
+        case 4: launch_gather_wide<SRC_KIND, unsigned>(s, map, n, src, dst, st); break;
+        default: launch_gather_wide<SRC_KIND, unsigned long long>(s, map, n, src, dst, st); break;
+    }
+}
+
+// fused remap of pixels wider than one byte (pb_wide.cuh): VEC-byte words
+template <int OUT_KIND, int SRC_KIND, bool SEP>
+static void launch_wide_v(const WideArgs& a, int vec, dim3 grid, cudaStream_t st) {
+    switch (vec) {
+        case 16: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 16><<<grid, 256, 0, st>>>(a); break;
+        case 8: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 8><<<grid, 256, 0, st>>>(a); break;
+        case 4: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 4><<<grid, 256, 0, st>>>(a); break;
+        default: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 2><<<grid, 256, 0, st>>>(a); break;
+    }
+    PB_COUNT_LAUNCH();
+}
+
+template <int OUT_KIND>
+static void launch_wide_s(const WideArgs& a, int vec, dim3 grid, cudaStream_t st) {
+    if (a.src.kind == PB_KIND_CAMERA) launch_wide_v<OUT_KIND, PB_KIND_CAMERA, false>(a, vec, grid, st);
+    else launch_wide_v<OUT_KIND, PB_KIND_EQUIRECT, false>(a, vec, grid, st);
+}
+
+// The widest word (a power of two, at most 16 bytes) that divides the pixel size and every address
+// the gather forms: the base pointers, and the frame strides when there is more than one frame
+// (row pitches are whole pixels).
+static int wide_vec(int px_bytes, const void* src, const void* dst, long long src_stride, long long dst_stride,
+                    bool multi) {
+    unsigned long long bits = (unsigned long long)px_bytes | (unsigned long long)reinterpret_cast<uintptr_t>(src) |
+                              (unsigned long long)reinterpret_cast<uintptr_t>(dst);
+    if (multi) bits |= (unsigned long long)src_stride | (unsigned long long)dst_stride;
+    int vec = 16;
+    while (vec > 2 && (bits & (unsigned long long)(vec - 1)) != 0) vec >>= 1;
+    return vec;
 }
 
 // ------------------------------------------------------------------------------------ tiled path
@@ -1719,6 +1782,69 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
     return PB_OK;
 }
 
+// plan_run for pixels of channels x elem_bytes (2, 4 or 8) bytes, camera / equirect sources: ONE
+// launch of remap_wide_kernel for the whole batch (the plan's state is only read: no lock needed)
+static int plan_run_wide(const pb_plan& p, int elem_bytes, const void* src, int64_t src_frame_stride, void* dst,
+                         int64_t dst_frame_stride, int32_t n_frames, cudaStream_t st, int row_begin = 0,
+                         int row_end = -1) {
+    if (row_end < 0) row_end = p.out.H;
+    const long long tiles_y = (row_end - row_begin + kTileH - 1) / kTileH;
+    if (tiles_y >= 65536) return fail(PB_ERR_UNSUPPORTED, "wide remap: more than 65535 x 64 output rows in one call");
+    WideArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.out = p.out;
+    a.src = p.src;
+    a.rot = p.rot;
+    a.fast = p.fast;
+    const bool sep = p.separable && p.tables != nullptr;
+    a.col_tab = sep ? p.tables : nullptr;
+    a.row_tab = sep ? p.tables + 2 * (size_t)p.out.W : nullptr;
+    a.src_px = static_cast<const unsigned char*>(src);
+    a.dst_px = static_cast<unsigned char*>(dst);
+    a.src_frame_stride = src_frame_stride;
+    a.dst_frame_stride = dst_frame_stride;
+    a.n_frames = n_frames;
+    a.row_begin = row_begin;
+    a.row_end = row_end;
+    a.px_bytes = p.desc.channels * elem_bytes;
+    const int vec = wide_vec(a.px_bytes, src, dst, src_frame_stride, dst_frame_stride, n_frames > 1);
+    a.words = a.px_bytes / vec;
+    const dim3 grid((p.out.W + kTileW - 1) / kTileW, (unsigned)tiles_y);
+    if (sep) {
+        launch_wide_v<PB_KIND_EQUIRECT, PB_KIND_CAMERA, true>(a, vec, grid, st);
+    } else {
+        switch (p.out.kind) {
+            case PB_KIND_CAMERA: launch_wide_s<PB_KIND_CAMERA>(a, vec, grid, st); break;
+            case PB_KIND_DOUBLE: launch_wide_s<PB_KIND_DOUBLE>(a, vec, grid, st); break;
+            default: launch_wide_s<PB_KIND_EQUIRECT>(a, vec, grid, st); break;
+        }
+    }
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "wide remap launch");
+    return PB_OK;
+}
+
+// Arguments of the _px entry points that need no device: the element width, then pointers and
+// strides against it.  -> PB_OK, or the code with pb_last_error set.
+static int check_elem_bytes(int32_t elem_bytes, const char* who) {
+    if (elem_bytes != 1 && elem_bytes != 2 && elem_bytes != 4 && elem_bytes != 8)
+        return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": elem_bytes must be 1, 2, 4 or 8 (got " +
+                                            std::to_string(elem_bytes) + ")");
+    return PB_OK;
+}
+static int check_double_source(int src_kind, const char* who) {
+    if (src_kind == PB_KIND_DOUBLE)
+        return fail(PB_ERR_UNSUPPORTED, std::string(who) +
+                                            ": a double-fisheye source blends its two lenses into uint8 "
+                                            "(projection.py:459); only elem_bytes == 1 is supported for it");
+    return PB_OK;
+}
+static int check_aligned(const void* p, long long stride, int32_t elem_bytes, const char* who) {
+    if ((reinterpret_cast<uintptr_t>(p) % (uintptr_t)elem_bytes) != 0 || stride % elem_bytes != 0)
+        return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": pointer or stride not a multiple of elem_bytes");
+    return PB_OK;
+}
+
 }  // namespace pb
 
 // ------------------------------------------------------------------------------------ C ABI
@@ -1889,6 +2015,45 @@ int pb_plan_remap_rows_u8(const pb_plan* plan, const uint8_t* src, uint8_t* dst_
                     row_end);
 }
 
+int pb_plan_remap_px(const pb_plan* plan, int32_t elem_bytes, const void* src, int64_t src_frame_stride, void* dst,
+                     int64_t dst_frame_stride, int32_t n_frames, void* stream) {
+    const char* who = "pb_plan_remap_px";
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!plan || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_px: null pointer");
+    if (elem_bytes == 1)
+        return pb_plan_remap_u8(plan, static_cast<const uint8_t*>(src), src_frame_stride, static_cast<uint8_t*>(dst),
+                                dst_frame_stride, n_frames, stream);
+    if (int rc = check_double_source(plan->src.kind, who)) return rc;
+    if (int rc = check_aligned(src, src_frame_stride, elem_bytes, who)) return rc;
+    if (int rc = check_aligned(dst, dst_frame_stride, elem_bytes, who)) return rc;
+    if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_px: negative n_frames");
+    if (n_frames == 0) return PB_OK;
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
+        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_px: plan belongs to another device");
+    return plan_run_wide(*plan, elem_bytes, src, src_frame_stride, dst, dst_frame_stride, n_frames, (cudaStream_t)stream);
+}
+
+int pb_plan_remap_rows_px(const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band, int32_t row_begin,
+                          int32_t row_end, void* stream) {
+    const char* who = "pb_plan_remap_rows_px";
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!plan || !src || !dst_band) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_px: null pointer");
+    if (elem_bytes == 1)
+        return pb_plan_remap_rows_u8(plan, static_cast<const uint8_t*>(src), static_cast<uint8_t*>(dst_band), row_begin,
+                                     row_end, stream);
+    if (int rc = check_double_source(plan->src.kind, who)) return rc;
+    if (int rc = check_aligned(src, 0, elem_bytes, who)) return rc;
+    if (int rc = check_aligned(dst_band, 0, elem_bytes, who)) return rc;
+    if (row_begin < 0 || row_end > plan->out.H || row_begin > row_end)
+        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_px: rows outside the output image");
+    if (row_begin == row_end) return PB_OK;
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
+        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_px: plan belongs to another device");
+    return plan_run_wide(*plan, elem_bytes, src, 0, dst_band, 0, 1, (cudaStream_t)stream, row_begin, row_end);
+}
+
 void pb_plan_destroy(pb_plan* plan) {
     if (!plan) return;
     if (plan->tables) cudaFree(plan->tables);
@@ -2034,6 +2199,38 @@ int pb_gather_from_map_u8(const pb_image_desc* src_desc, int32_t channels, doubl
     cudaError_t e = cudaGetLastError();
     if (luts) cudaFreeAsync(luts, st);
     if (e != cudaSuccess) return cuda_fail(e, "pb_gather_from_map_u8 launch");
+    return PB_OK;
+}
+
+int pb_gather_from_map_px(const pb_image_desc* src_desc, int32_t channels, int32_t elem_bytes, double* map,
+                          int32_t map_height, int32_t map_width, const void* src, void* dst, void* stream) {
+    const char* who = "pb_gather_from_map_px";
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!src_desc || !map || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, "pb_gather_from_map_px: null pointer");
+    if (elem_bytes == 1)
+        return pb_gather_from_map_u8(src_desc, channels, map, map_height, map_width, static_cast<const uint8_t*>(src),
+                                     static_cast<uint8_t*>(dst), stream);
+    if (int rc = check_image(*src_desc, "src")) return rc;
+    if (int rc = check_double_source(src_desc->kind, who)) return rc;
+    if (int rc = check_aligned(src, 0, elem_bytes, who)) return rc;
+    if (int rc = check_aligned(dst, 0, elem_bytes, who)) return rc;
+    if (src_desc->height > 32767 || src_desc->width > 65535)
+        return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_px: source larger than 32767 rows x 65535 columns");
+    if (channels < 1 || channels > 4) return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_px: channels must be 1..4");
+    if (map_height < 0 || map_width < 0) return fail(PB_ERR_INVALID_ARGUMENT, "pb_gather_from_map_px: negative map size");
+    const long long n = (long long)map_height * map_width;
+    if (n == 0) return PB_OK;
+    if ((n + 255) / 256 > 0x7fffffffLL) return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_px: map too large");
+    SrcGeom s = derive_src(*src_desc, channels);
+    cudaStream_t st = (cudaStream_t)stream;
+    double* luts = nullptr;
+    if (cudaError_t eu = upload_lens_tables(nullptr, nullptr, src_desc, &s, &luts, st, true))
+        return cuda_fail(eu, "pb_gather_from_map_px lens table");
+    if (s.kind == PB_KIND_CAMERA) launch_gather_e<PB_KIND_CAMERA>(s, elem_bytes, map, n, src, dst, st);
+    else launch_gather_e<PB_KIND_EQUIRECT>(s, elem_bytes, map, n, src, dst, st);
+    cudaError_t e = cudaGetLastError();
+    if (luts) cudaFreeAsync(luts, st);
+    if (e != cudaSuccess) return cuda_fail(e, "pb_gather_from_map_px launch");
     return PB_OK;
 }
 

@@ -196,7 +196,7 @@ def is_torch_tensor(x) -> bool:
 
 
 def image_layout(image) -> Tuple[int, int, int, bool]:
-    """(height, width, channels, had_channel_axis) of an HWC / HW uint8 image."""
+    """(height, width, channels, had_channel_axis) of an HWC / HW image."""
     shape = tuple(image.shape)
     if len(shape) == 2:
         return shape[0], shape[1], 1, False
@@ -205,17 +205,52 @@ def image_layout(image) -> Tuple[int, int, int, bool]:
     raise ValueError(f"expected an (H, W, C) or (H, W) image, got shape {shape}")
 
 
-def _check_u8(image) -> None:
+# Element types the remap takes, by NumPy / torch name, and their width in bytes.  The remap copies
+# a pixel's bytes and converts nothing, so only the width matters (bfloat16: torch tensors only).
+ELEM_BYTES = {
+    "bool": 1, "int8": 1, "uint8": 1,
+    "int16": 2, "uint16": 2, "float16": 2, "bfloat16": 2,
+    "int32": 4, "uint32": 4, "float32": 4,
+    "int64": 8, "uint64": 8, "float64": 8,
+}
+
+
+def _dtype_name(image) -> str:
     name = str(image.dtype)
-    if name not in ("uint8", "torch.uint8"):
-        raise NotImplementedError(f"only uint8 images are supported by the B200 path (got {name})")
+    return name[len("torch."):] if name.startswith("torch.") else name
 
 
-def to_device_u8(image):
-    """uint8 image (numpy / torch CPU / torch CUDA) -> contiguous CUDA tensor (async H2D on the
-    current stream; pinned host memory makes it a true async copy)."""
+def elem_bytes(image) -> int:
+    """Bytes per element of an image the remap takes (see ELEM_BYTES); NotImplementedError naming
+    the dtype for anything else (complex, object, structured, non-native byte order ...)."""
+    name = _dtype_name(image)
+    width = ELEM_BYTES.get(name)
+    if width is None or (name == "bfloat16" and not is_torch_tensor(image)):
+        raise NotImplementedError(f"images of dtype {name} are not supported: the remap takes bool, int8, uint8, "
+                                  "int16, uint16, float16, bfloat16 (torch), int32, uint32, float32, int64, uint64 "
+                                  "and float64 images")
+    return width
+
+
+def check_source(src: ImageGeometry, image) -> int:
+    """elem_bytes(image), after refusing what a source of geometry ``src`` cannot be: a
+    double-fisheye source must be uint8.  The reference blends its two lenses in float64 and casts
+    the blend to uint8 whatever the input dtype (projection.py:459), so a wider source would come
+    back as a uint8 image wrapped mod 256; neither that nor a dtype-preserving blend is offered."""
+    width = elem_bytes(image)
+    name = _dtype_name(image)
+    if src.kind == _native.KIND_DOUBLE and name != "uint8":
+        raise NotImplementedError(
+            f"a double-fisheye source must be uint8 (got {name}): the reference blends the two lenses and "
+            "casts the blend to uint8 whatever the input dtype, which would wrap other values mod 256")
+    return width
+
+
+def to_device(image):
+    """Image of an accepted dtype (numpy / torch CPU / torch CUDA) -> contiguous CUDA tensor of the
+    same dtype (async H2D on the current stream; pinned host memory makes it a true async copy)."""
     torch = _torch()
-    _check_u8(image)
+    elem_bytes(image)
     if is_torch_tensor(image):
         t = image
     else:
@@ -254,11 +289,19 @@ def from_device_like(result, like, out=None):
 # ----------------------------------------------------------------------------- calls
 
 
+def _check_out(out_dev, out_shape, src_dev) -> None:
+    if tuple(out_dev.shape) != out_shape or not out_dev.is_contiguous() or out_dev.dtype != src_dev.dtype:
+        name = _dtype_name(src_dev)
+        raise ValueError(f"out must be a contiguous {name} tensor of shape {out_shape}")
+
+
 def remap_device(rays: RayPlan, src: ImageGeometry, src_dev, out_dev=None):
-    """Fused remap on device tensors.  src_dev: uint8 CUDA tensor (H, W[, C]) or a batch
-    (N, H, W, C); returns (and fills) the uint8 CUDA output tensor."""
+    """Fused remap on device tensors.  src_dev: CUDA tensor (H, W[, C]) or a batch (N, H, W, C) of
+    an accepted dtype (ELEM_BYTES); returns (and fills) the CUDA output tensor of the same dtype.
+    One-byte elements take the uint8 kernels (pb_plan_remap_u8), wider ones pb_plan_remap_px."""
     torch = _torch()
     lib = _native.load()
+    e = check_source(src, src_dev)
     batched = src_dev.dim() == 4
     frames = src_dev.shape[0] if batched else 1
     h, w, c, had_c = image_layout(src_dev[0] if batched else src_dev)
@@ -269,26 +312,31 @@ def remap_device(rays: RayPlan, src: ImageGeometry, src_dev, out_dev=None):
     if batched:
         out_shape = (frames,) + out_shape
     if out_dev is None:
-        out_dev = torch.empty(out_shape, dtype=torch.uint8, device=src_dev.device)
-    elif tuple(out_dev.shape) != out_shape or not out_dev.is_contiguous() or out_dev.dtype != torch.uint8:
-        raise ValueError(f"out must be a contiguous uint8 tensor of shape {out_shape}")
+        out_dev = torch.empty(out_shape, dtype=src_dev.dtype, device=src_dev.device)
+    else:
+        _check_out(out_dev, out_shape, src_dev)
     desc = _remap_desc(rays, src, c)
     with torch.cuda.device(src_dev.device):
         plan = _plans.get(lib, desc, src_dev.device.index or 0, torch)
         stream = _stream_ptr(torch)
-        _native.check(lib.pb_plan_remap_u8(
-            plan,
-            ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_int64(h * w * c),
-            ctypes.c_void_p(out_dev.data_ptr()), ctypes.c_int64(oh * ow * c),
-            ctypes.c_int32(frames), stream))
+        src_ptr, dst_ptr = ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_void_p(out_dev.data_ptr())
+        src_stride, dst_stride = ctypes.c_int64(h * w * c * e), ctypes.c_int64(oh * ow * c * e)
+        if e == 1:  # uint8, int8, bool: the same bytes
+            _native.check(lib.pb_plan_remap_u8(plan, src_ptr, src_stride, dst_ptr, dst_stride,
+                                               ctypes.c_int32(frames), stream))
+        else:
+            _native.check(lib.pb_plan_remap_px(plan, ctypes.c_int32(e), src_ptr, src_stride, dst_ptr, dst_stride,
+                                               ctypes.c_int32(frames), stream))
     return out_dev
 
 
 def remap_rows_device(rays: RayPlan, src: ImageGeometry, src_dev, row_begin: int, row_end: int, out_dev=None):
-    """Output rows [row_begin, row_end) of one frame (pb_plan_remap_rows_u8): src_dev is the WHOLE
-    source image on this device, the result is the band alone, (row_end - row_begin, Wo[, C])."""
+    """Output rows [row_begin, row_end) of one frame (pb_plan_remap_rows_u8 / _px): src_dev is the
+    WHOLE source image on this device, the result is the band alone, (row_end - row_begin, Wo[, C]),
+    of the source's dtype."""
     torch = _torch()
     lib = _native.load()
+    e = check_source(src, src_dev)
     if src_dev.dim() == 4:
         raise ValueError("a row band is cut from ONE frame, not from a batch")
     h, w, c, had_c = image_layout(src_dev)
@@ -299,17 +347,20 @@ def remap_rows_device(rays: RayPlan, src: ImageGeometry, src_dev, row_begin: int
         raise ValueError(f"rows [{row_begin}, {row_end}) outside an output of {oh} rows")
     out_shape = (row_end - row_begin, ow, c) if had_c else (row_end - row_begin, ow)
     if out_dev is None:
-        out_dev = torch.empty(out_shape, dtype=torch.uint8, device=src_dev.device)
-    elif tuple(out_dev.shape) != out_shape or not out_dev.is_contiguous() or out_dev.dtype != torch.uint8:
-        raise ValueError(f"out must be a contiguous uint8 tensor of shape {out_shape}")
+        out_dev = torch.empty(out_shape, dtype=src_dev.dtype, device=src_dev.device)
+    else:
+        _check_out(out_dev, out_shape, src_dev)
     if row_begin == row_end:
         return out_dev
     desc = _remap_desc(rays, src, c)
     with torch.cuda.device(src_dev.device):
         plan = _plans.get(lib, desc, src_dev.device.index or 0, torch)
-        _native.check(lib.pb_plan_remap_rows_u8(
-            plan, ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_void_p(out_dev.data_ptr()),
-            ctypes.c_int32(row_begin), ctypes.c_int32(row_end), _stream_ptr(torch)))
+        src_ptr, dst_ptr = ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_void_p(out_dev.data_ptr())
+        rows = (ctypes.c_int32(row_begin), ctypes.c_int32(row_end), _stream_ptr(torch))
+        if e == 1:
+            _native.check(lib.pb_plan_remap_rows_u8(plan, src_ptr, dst_ptr, *rows))
+        else:
+            _native.check(lib.pb_plan_remap_rows_px(plan, ctypes.c_int32(e), src_ptr, dst_ptr, *rows))
     return out_dev
 
 
@@ -345,9 +396,10 @@ def rotate_map_device(cmap_dev, matrix):
 
 
 def gather_from_map_device(src: ImageGeometry, cmap_dev, src_dev, out_dev=None):
-    """process_coordinate_map on an explicit float64 CUDA map."""
+    """process_coordinate_map on an explicit float64 CUDA map; the result has the source's dtype."""
     torch = _torch()
     lib = _native.load()
+    e = check_source(src, src_dev)
     h, w, c, had_c = image_layout(src_dev)
     if (h, w) != (src.height, src.width):
         raise ValueError(f"source image is {h}x{w} but its geometry says {src.height}x{src.width}")
@@ -362,17 +414,23 @@ def gather_from_map_device(src: ImageGeometry, cmap_dev, src_dev, out_dev=None):
     mh, mw = cmap_dev.shape[0], cmap_dev.shape[1]
     out_shape = (mh, mw, c) if had_c else (mh, mw)
     if out_dev is None:
-        out_dev = torch.empty(out_shape, dtype=torch.uint8, device=src_dev.device)
-    elif (tuple(out_dev.shape) != out_shape or not out_dev.is_contiguous() or out_dev.dtype != torch.uint8
+        out_dev = torch.empty(out_shape, dtype=src_dev.dtype, device=src_dev.device)
+    elif (tuple(out_dev.shape) != out_shape or not out_dev.is_contiguous() or out_dev.dtype != src_dev.dtype
           or out_dev.device != src_dev.device):
-        raise ValueError(f"out must be a contiguous uint8 tensor of shape {out_shape} on {src_dev.device}")
+        raise ValueError(f"out must be a contiguous {_dtype_name(src_dev)} tensor of shape {out_shape} on {src_dev.device}")
     d = _native.ImageDesc()
     src.fill(d)
     with torch.cuda.device(src_dev.device):
-        _native.check(lib.pb_gather_from_map_u8(
-            ctypes.byref(d), ctypes.c_int32(c), ctypes.c_void_p(cmap_dev.data_ptr()),
-            ctypes.c_int32(mh), ctypes.c_int32(mw), ctypes.c_void_p(src_dev.data_ptr()),
-            ctypes.c_void_p(out_dev.data_ptr()), _stream_ptr(torch)))
+        if e == 1:
+            _native.check(lib.pb_gather_from_map_u8(
+                ctypes.byref(d), ctypes.c_int32(c), ctypes.c_void_p(cmap_dev.data_ptr()),
+                ctypes.c_int32(mh), ctypes.c_int32(mw), ctypes.c_void_p(src_dev.data_ptr()),
+                ctypes.c_void_p(out_dev.data_ptr()), _stream_ptr(torch)))
+        else:
+            _native.check(lib.pb_gather_from_map_px(
+                ctypes.byref(d), ctypes.c_int32(c), ctypes.c_int32(e), ctypes.c_void_p(cmap_dev.data_ptr()),
+                ctypes.c_int32(mh), ctypes.c_int32(mw), ctypes.c_void_p(src_dev.data_ptr()),
+                ctypes.c_void_p(out_dev.data_ptr()), _stream_ptr(torch)))
     return out_dev
 
 
