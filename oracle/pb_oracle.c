@@ -241,10 +241,13 @@ static int camera_lookup(int lens, double f, int h, int w, double lat, double lo
     return 1;
 }
 
-/* ndarray.astype(np.uint8) from float64: truncate, keep the low byte */
+/* ndarray.astype(np.uint8) from float64 on x86-64: truncation to a 32-bit integer
+ * (cvttsd2si), low byte kept; NaN and |v| >= 2^31 give INT32_MIN, whose low byte is 0 */
 static uint8_t wrap_u8(double v)
 {
-    return (uint8_t)(trunc_i64(v) & 0xFF);
+    if (!(fabs(v) < 2147483648.0))
+        return 0;
+    return (uint8_t)((int32_t)v & 0xFF);
 }
 
 /* projection.py:439-456 */

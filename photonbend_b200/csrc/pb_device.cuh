@@ -288,10 +288,16 @@ __device__ __forceinline__ int xy_to_offset(int xy, int width) {
     return xy < 0 ? -1 : (xy >> 16) * width + (xy & 0xffff);
 }
 
-// (left*wl + right*wr).astype(np.uint8): truncate, keep the low byte  (projection.py:459)
+// numpy's float64 -> uint8 cast on x86-64: truncation to a 32-bit integer (cvttsd2si), low byte
+// kept; NaN and |v| >= 2^31 give 0x80000000, whose low byte is 0
+__device__ __forceinline__ unsigned char cast_u8(double v) {
+    if (!(fabs(v) < 2147483648.0)) return 0;
+    return (unsigned char)(__double2int_rz(v) & 0xff);
+}
+
+// (left*wl + right*wr).astype(np.uint8)  (projection.py:459)
 __device__ __forceinline__ unsigned char blend_u8(unsigned a, double wa, unsigned b, double wb) {
-    const double v = __dadd_rn(__dmul_rn((double)a, wa), __dmul_rn((double)b, wb));
-    return (unsigned char)(trunc_i64(v) & 0xFF);
+    return cast_u8(__dadd_rn(__dmul_rn((double)a, wa), __dmul_rn((double)b, wb)));
 }
 
 }  // namespace pb

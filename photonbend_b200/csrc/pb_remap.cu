@@ -723,11 +723,6 @@ __global__ void __launch_bounds__(256) map_range_kernel(double* __restrict__ map
         if (nan) atomicOr(&range->any_nan, 1);
     }
 }
-// numpy's float64 -> uint8 cast on x86-64: truncation to a 32-bit integer, low byte kept
-__device__ __forceinline__ unsigned char cast_u8(double v) {
-    if (!(fabs(v) < 2147483648.0)) return 0;  // NaN / out of range: 0x80000000
-    return (unsigned char)(__double2int_rz(v) & 0xff);
-}
 __global__ void __launch_bounds__(256) map_projection_kernel(const double* __restrict__ map, long long n,
                                                              const MapRange* __restrict__ range, unsigned char* __restrict__ dst) {
     const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;

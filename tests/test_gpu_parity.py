@@ -317,19 +317,22 @@ def test_tiled_fast_path_mid_size_batches(torch_cuda, src_kind):
         (src_kind, n_bad1, max_abs1)
 
 
-@pytest.mark.parametrize("fov_deg", [195, 180, 181, 210, 170, 250])
+@pytest.mark.parametrize("fov_deg", [195, 180, 181, 210, 170, 250, 180.00000000001, 179.99999999999])
 def test_double_source_batches_blend_band(torch_cuda, fov_deg, monkeypatch):
     """Batches through a double-fisheye source (csrc/pb_tiled.cuh: two launches by tile class,
     blend band through the guarded fixed-point blend) on frames chosen to sit ON the blend's
     truncation boundaries: flat frames (left == right, weights adding up to 1 -> the float64 sum is
     an integer up to its last bits), black frames, a ramp, and noise; several sensor fovs (180:
-    zero-width band, division by zero in the weights; 170: negative range), against the NumPy oracle."""
+    zero-width band, division by zero in the weights; 170: negative range; within 2e-13 rad of
+    180: a band so narrow that the weights grow past 2^31 and the blend leaves the int32 range of
+    NumPy's uint8 cast), against the NumPy oracle."""
     torch = torch_cuda
     from oracle import numpy_port
 
     sg = {"kind": "double", "height": 336, "width": 672, "lens": "equidistant", "fov": case_matrix.rad(fov_deg)}
     og = {"kind": "equirect", "height": 336 + 16, "width": 672 + 32}
-    rng = np.random.default_rng(fov_deg)
+    seed = round(fov_deg)
+    rng = np.random.default_rng(seed)
     h, w = sg["height"], sg["width"]
     ramp = (np.arange(h * w * 3, dtype=np.int64).reshape(h, w, 3) // 7 % 256).astype(np.uint8)
     frames = np.stack([
@@ -337,7 +340,7 @@ def test_double_source_batches_blend_band(torch_cuda, fov_deg, monkeypatch):
         np.zeros((h, w, 3), np.uint8),
         np.full((h, w, 3), 255, np.uint8),
         ramp,
-        case_matrix.case_image(sg, 500 + fov_deg),
+        case_matrix.case_image(sg, 500 + seed),
         (rng.integers(0, 4, (h, w, 3)) * 85).astype(np.uint8),
     ])
     want = [numpy_port.remap(og, (), sg, f) for f in frames]

@@ -11,6 +11,7 @@
 import hashlib
 import json
 import os
+import platform
 
 import numpy as np
 import pytest
@@ -127,6 +128,77 @@ def test_c_port_threads_equal_single_thread():
     c = c_port.remap(og, rots, sg, image, rows=(5, 17), threads=2)
     assert np.array_equal(a, b)
     assert np.array_equal(a[5:17], c)
+
+
+def numpy_u8_cast_model(v):
+    """NumPy's float64 -> uint8 cast on x86-64, as the kernels (cast_u8 in csrc/pb_device.cuh) and
+    pb_oracle.c restate it: truncation to a 32-bit integer (cvttsd2si), low byte kept; NaN and
+    |v| >= 2^31 become INT32_MIN, whose low byte is 0."""
+    v = np.asarray(v, dtype=np.float64)
+    with np.errstate(invalid="ignore"):
+        fits = np.abs(v) < 2.0**31
+    t = np.where(fits, np.trunc(np.where(fits, v, 0.0)), -(2.0**31)).astype(np.int64)
+    return (t & 0xFF).astype(np.uint8)
+
+
+@pytest.mark.skipif(platform.machine().lower() not in ("x86_64", "amd64"),
+                    reason="the kernels restate NumPy's x86-64 cast; other hosts saturate")
+def test_numpy_uint8_cast_is_the_32_bit_truncation_the_kernels_restate():
+    """ndarray.astype(np.uint8) of float64 on this host against numpy_u8_cast_model, over the
+    values where 8-, 32- and 64-bit truncations part ways, contiguous, strided and 3-D."""
+    tiny = np.finfo(np.float64).smallest_subnormal
+    edges = [np.nan, -np.nan, np.inf, -np.inf, 0.0, -0.0, tiny, -tiny, 1e-310, -1e-310,
+             0.5, -0.5, 0.999999, -0.999999, 1.5, -1.5, 255.0, 255.5, 255.9999999, 256.0, 256.5,
+             -255.9999, -256.0, -256.5, 300.7, -300.7, 2.0**63, -(2.0**63), 2.0**64, 1e300, -1e300]
+    for base in (2.0**31, 2.0**32, 2.0**52, 2.0**53):
+        for d in (-7.0, -1.0, -0.5, 0.0, 0.5, 1.0, 7.0):
+            edges += [base + d, -(base + d)]
+        edges += [np.nextafter(base, 0), np.nextafter(base, np.inf), -np.nextafter(base, 0), -np.nextafter(base, np.inf)]
+    edges = np.array(edges, dtype=np.float64)
+    want = numpy_u8_cast_model(edges)
+    assert want[np.isnan(edges)].tolist() == [0, 0]
+    assert numpy_u8_cast_model([2.0**31 + 7, 300.7, -1.5, 255.9999999, -256.5]).tolist() == [0, 44, 255, 255, 0]
+    rng = np.random.default_rng(31)
+    mags = 10.0 ** rng.uniform(-323, 308, 200_000)
+    sweep = np.concatenate([edges, mags * rng.choice([-1.0, 1.0], mags.size),
+                            rng.uniform(-2.0**33, 2.0**33, 100_000), rng.uniform(-600, 600, 100_000)])
+    with np.errstate(invalid="ignore"):
+        assert np.array_equal(sweep.astype(np.uint8), numpy_u8_cast_model(sweep))
+        assert np.array_equal(np.repeat(sweep, 2)[1::2].astype(np.uint8), numpy_u8_cast_model(sweep))
+        cube = sweep[: (sweep.size // 60) * 60].reshape(-1, 20, 3)
+        assert np.array_equal(cube.astype(np.uint8), numpy_u8_cast_model(cube))
+        assert np.array_equal(cube[:, ::2, 1:].astype(np.uint8), numpy_u8_cast_model(cube[:, ::2, 1:]))
+
+
+# Double-fisheye sensor fovs within 1e-9 rad of pi: the blend band 2 * (fov/2 - pi/2) nearly
+# vanishes and its weights reach 1e7 .. 1e13, beyond the 32 bits of NumPy's uint8 cast.
+NEAR_180_FOVS = {
+    "nextafter_up": float(np.nextafter(np.pi, np.inf)),
+    "nextafter_down": float(np.nextafter(np.pi, 0.0)),
+    "pi_plus_1e-12": np.pi + 1e-12,
+    "pi_minus_1e-12": np.pi - 1e-12,
+    "180.000000001": case_matrix.rad(180.000000001),
+    "180.00000000001": case_matrix.rad(180.00000000001),
+    "179.99999999999": case_matrix.rad(179.99999999999),
+    "pi": np.pi,
+    "180.0000001": case_matrix.rad(180.0000001),
+}
+
+
+@pytest.mark.parametrize("fov_name", list(NEAR_180_FOVS))
+def test_c_port_blend_of_near_180_degree_double_sources(fov_name):
+    """oracle/pb_oracle.c against the NumPy oracle (bit-identical to the reference) on double
+    sources whose blend weights overflow int32: the C oracle has to cast the blend to uint8 the
+    way NumPy does, or every pixel of the band rows differs."""
+    fov = NEAR_180_FOVS[fov_name]
+    for (h, w), og in (((336, 672), {"kind": "equirect", "height": 352, "width": 704}),
+                       ((200, 400), {"kind": "equirect", "height": 400, "width": 800})):
+        sg = {"kind": "double", "height": h, "width": w, "lens": "equidistant", "fov": fov}
+        for image in (np.full((h, w, 3), 200, np.uint8), case_matrix.case_image(sg, 7)):
+            for rots in ((), ((0.3, -0.7, 1.1),)):
+                got = c_port.remap(og, rots, sg, image)
+                want = numpy_port.remap(og, rots, sg, image)
+                assert np.array_equal(got, want), (fov_name, h, len(rots), mismatch_report(got, want))
 
 
 @pytest.mark.parametrize("bad_fov_deg", [179.0, 180.0])
