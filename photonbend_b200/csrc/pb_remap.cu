@@ -12,6 +12,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "pb_device.cuh"
@@ -172,6 +173,19 @@ static cudaError_t upload_lens_tables(const pb_image_desc* od, OutGeom* og, cons
     return e;
 }
 
+// radius (in focal units) at which the latitude of an output lens crosses hf = fov / 2; inf = never
+static double lens_d_star(int lens, double hf) {
+    const double inf = INFINITY;
+    switch (lens) {
+        case PB_LENS_EQUIDISTANT: return hf;
+        case PB_LENS_EQUISOLID: return hf < kPi ? 2.0 * std::sin(hf / 2.0) : inf;
+        case PB_LENS_ORTHOGRAPHIC: return hf < kPi / 2 ? std::sin(hf) : inf;
+        case PB_LENS_STEREOGRAPHIC: return hf < kPi ? 2.0 * std::tan(hf / 2.0) : inf;
+        case PB_LENS_RECTILINEAR: return hf < kPi / 2 ? std::tan(hf) : inf;
+        default: return 0.713 * hf < kPi / 2 ? 1.47 * std::sin(0.713 * hf) : inf;
+    }
+}
+
 // Constants of the guarded short cut (pb_fast.cuh).  Nothing here has to be bit-identical to
 // the reference: these are decision thresholds with a guard band, not values that reach a pixel.
 static FastGeom derive_fast(const pb_image_desc& od, const OutGeom& o, const pb_image_desc& sd, const SrcGeom& s,
@@ -216,16 +230,7 @@ static FastGeom derive_fast(const pb_image_desc& od, const OutGeom& o, const pb_
         const double f = o.f, hf = o.half_fov;
         if (!(f > 0.0) || !std::isfinite(f) || !std::isfinite(hf)) g.enabled = 0;
         g.inv_f = 1.0 / f;
-        // radius (in focal units) at which the latitude crosses fov / 2; inf = never
-        double d_star = inf;
-        switch (o.lens) {
-            case PB_LENS_EQUIDISTANT: d_star = hf; break;
-            case PB_LENS_EQUISOLID: d_star = hf < kPi ? 2.0 * std::sin(hf / 2.0) : inf; break;
-            case PB_LENS_ORTHOGRAPHIC: d_star = hf < kPi / 2 ? std::sin(hf) : inf; break;
-            case PB_LENS_STEREOGRAPHIC: d_star = hf < kPi ? 2.0 * std::tan(hf / 2.0) : inf; break;
-            case PB_LENS_RECTILINEAR: d_star = hf < kPi / 2 ? std::tan(hf) : inf; break;
-            default: d_star = 0.713 * hf < kPi / 2 ? 1.47 * std::sin(0.713 * hf) : inf; break;
-        }
+        const double d_star = lens_d_star(o.lens, hf);
         if (hf < 0.0) {  // every ray is outside the fov
             g.r2_valid = -1.0;
             g.r2_invalid = -1.0;
@@ -303,15 +308,7 @@ static Fast32GeomT<double> derive_fast32(const OutGeom& o, const SrcGeom& s, con
         d.y0 = o.y_start;
         d.inv_f = 1.0 / f;
         d.quarter_inv_f2 = 0.25 / (f * f);
-        double d_star = inf;
-        switch (o.lens) {
-            case PB_LENS_EQUIDISTANT: d_star = hf; break;
-            case PB_LENS_EQUISOLID: d_star = hf < kPi ? 2.0 * std::sin(hf / 2.0) : inf; break;
-            case PB_LENS_ORTHOGRAPHIC: d_star = hf < kPi / 2 ? std::sin(hf) : inf; break;
-            case PB_LENS_STEREOGRAPHIC: d_star = hf < kPi ? 2.0 * std::tan(hf / 2.0) : inf; break;
-            case PB_LENS_RECTILINEAR: d_star = hf < kPi / 2 ? std::tan(hf) : inf; break;
-            default: d_star = 0.713 * hf < kPi / 2 ? 1.47 * std::sin(0.713 * hf) : inf; break;
-        }
+        const double d_star = lens_d_star(o.lens, hf);
         if (hf < 0.0) {
             d.r2_valid = d.r2_invalid = -1.0;
         } else if (d_star < inf) {
@@ -742,149 +739,105 @@ __global__ void __launch_bounds__(256) map_projection_kernel(const double* __res
 
 // ------------------------------------------------------------------------------------ launchers
 
-template <int OUT_KIND, int SRC_KIND>
-static void launch_generic_c(const RemapArgs& a, cudaStream_t st) {
-    dim3 block(32, 8);
-    dim3 grid((a.out.W + block.x - 1) / block.x, (a.row_end - a.row_begin + block.y - 1) / block.y);
-    switch (a.src.C) {
-        case 1: remap_generic_kernel<OUT_KIND, SRC_KIND, 1><<<grid, block, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
-        case 2: remap_generic_kernel<OUT_KIND, SRC_KIND, 2><<<grid, block, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
-        case 3: remap_generic_kernel<OUT_KIND, SRC_KIND, 3><<<grid, block, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
-        default: remap_generic_kernel<OUT_KIND, SRC_KIND, 4><<<grid, block, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
+// Runtime values as compile-time constants: each with_* helper calls f(Int<V>{}) for the value V
+// the runtime value selects, so that f can instantiate the kernel template for it.
+template <int V>
+using Int = std::integral_constant<int, V>;
+
+// an unknown kind runs as an equirect image
+template <typename F>
+static auto with_kind(int kind, F&& f) {
+    switch (kind) {
+        case PB_KIND_CAMERA: return f(Int<PB_KIND_CAMERA>{});
+        case PB_KIND_DOUBLE: return f(Int<PB_KIND_DOUBLE>{});
+        default: return f(Int<PB_KIND_EQUIRECT>{});
     }
 }
 
-template <int OUT_KIND>
-static void launch_generic_s(const RemapArgs& a, cudaStream_t st) {
-    switch (a.src.kind) {
-        case PB_KIND_CAMERA: launch_generic_c<OUT_KIND, PB_KIND_CAMERA>(a, st); break;
-        case PB_KIND_DOUBLE: launch_generic_c<OUT_KIND, PB_KIND_DOUBLE>(a, st); break;
-        default: launch_generic_c<OUT_KIND, PB_KIND_EQUIRECT>(a, st); break;
+// kernels without a double-fisheye instantiation: a camera source, anything else as equirect
+template <typename F>
+static auto with_single_kind(int kind, F&& f) {
+    if (kind == PB_KIND_CAMERA) return f(Int<PB_KIND_CAMERA>{});
+    return f(Int<PB_KIND_EQUIRECT>{});
+}
+
+template <typename F>
+static auto with_kinds(int out_kind, int src_kind, F&& f) {
+    return with_kind(out_kind, [&](auto o) { return with_kind(src_kind, [&](auto s) { return f(o, s); }); });
+}
+
+// 1, 2 or 3 channels; anything else as 4
+template <typename F>
+static auto with_channels(int channels, F&& f) {
+    switch (channels) {
+        case 1: return f(Int<1>{});
+        case 2: return f(Int<2>{});
+        case 3: return f(Int<3>{});
+        default: return f(Int<4>{});
     }
 }
 
-template <int OUT_KIND>
-static void launch_direct_s(const RemapArgs& a, dim3 grid, cudaStream_t st) {
-    switch (a.src.kind) {
-        case PB_KIND_CAMERA: remap_direct_kernel<OUT_KIND, PB_KIND_CAMERA><<<grid, 256, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
-        case PB_KIND_DOUBLE: remap_direct_kernel<OUT_KIND, PB_KIND_DOUBLE><<<grid, 256, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
-        default: remap_direct_kernel<OUT_KIND, PB_KIND_EQUIRECT><<<grid, 256, 0, st>>>(a); PB_COUNT_LAUNCH(); break;
+// f(T{}) with T the unsigned integer of a 2- or 4-byte element; anything else as 8 bytes
+template <typename F>
+static auto with_elem(int elem_bytes, F&& f) {
+    switch (elem_bytes) {
+        case 2: return f((unsigned short)0);
+        case 4: return f(0u);
+        default: return f(0ull);
     }
 }
 
-template <int OUT_KIND>
-static void launch_direct32_s(const RemapArgs& a, dim3 grid, cudaStream_t st) {
-    if (a.src.kind == PB_KIND_CAMERA) remap_direct32_kernel<OUT_KIND, PB_KIND_CAMERA><<<grid, 256, 0, st>>>(a);
-    else remap_direct32_kernel<OUT_KIND, PB_KIND_EQUIRECT><<<grid, 256, 0, st>>>(a);
-    PB_COUNT_LAUNCH();
-}
-
-template <int OUT_KIND>
-static void launch_stats_s(const RemapArgs& a, const Fast32GeomT<double>& gd, unsigned* maxima, unsigned long long* counters,
-                           cudaStream_t st) {
-    dim3 block(32, 8);
-    dim3 grid((a.out.W + 31) / 32, (a.out.H + 7) / 8);
-    switch (a.src.kind) {
-        case PB_KIND_CAMERA: fast32_stats_kernel<OUT_KIND, PB_KIND_CAMERA><<<grid, block, 0, st>>>(a, gd, maxima, counters); break;
-        case PB_KIND_DOUBLE: fast32_stats_kernel<OUT_KIND, PB_KIND_DOUBLE><<<grid, block, 0, st>>>(a, gd, maxima, counters); break;
-        default: fast32_stats_kernel<OUT_KIND, PB_KIND_EQUIRECT><<<grid, block, 0, st>>>(a, gd, maxima, counters); break;
+// 16-, 8- or 4-byte words; anything else as 2
+template <typename F>
+static auto with_vec(int vec, F&& f) {
+    switch (vec) {
+        case 16: return f(Int<16>{});
+        case 8: return f(Int<8>{});
+        case 4: return f(Int<4>{});
+        default: return f(Int<2>{});
     }
-    PB_COUNT_LAUNCH();
-}
-
-template <int OUT_KIND>
-static void launch_ratio_s(const RemapArgs& a, const Fast32GeomT<double>& gd, unsigned* maxima, cudaStream_t st) {
-    dim3 block(32, 8);
-    dim3 grid((a.out.W + block.x - 1) / block.x, (a.out.H + block.y - 1) / block.y);
-    switch (a.src.kind) {
-        case PB_KIND_CAMERA: fast32_ratio_kernel<OUT_KIND, PB_KIND_CAMERA><<<grid, block, 0, st>>>(a, gd, maxima); break;
-        case PB_KIND_DOUBLE: fast32_ratio_kernel<OUT_KIND, PB_KIND_DOUBLE><<<grid, block, 0, st>>>(a, gd, maxima); break;
-        default: fast32_ratio_kernel<OUT_KIND, PB_KIND_EQUIRECT><<<grid, block, 0, st>>>(a, gd, maxima); break;
-    }
-    PB_COUNT_LAUNCH();
 }
 
 static void launch_direct(const RemapArgs& a, cudaStream_t st) {
     dim3 grid((a.out.W + kTileW - 1) / kTileW, (a.row_end - a.row_begin + kTileH - 1) / kTileH);
     static const bool compact_off = std::getenv("PB_COMPACT") && std::atoi(std::getenv("PB_COMPACT")) == 0;  // experiments
     if (a.src.kind != PB_KIND_DOUBLE && a.fast.f32.enabled && !compact_off) {
-        switch (a.out.kind) {
-            case PB_KIND_CAMERA: launch_direct32_s<PB_KIND_CAMERA>(a, grid, st); break;
-            case PB_KIND_DOUBLE: launch_direct32_s<PB_KIND_DOUBLE>(a, grid, st); break;
-            default: launch_direct32_s<PB_KIND_EQUIRECT>(a, grid, st); break;
-        }
-        return;
+        with_kind(a.out.kind, [&](auto o) {
+            with_single_kind(a.src.kind, [&](auto s) { remap_direct32_kernel<o, s><<<grid, 256, 0, st>>>(a); });
+        });
+    } else {
+        with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) { remap_direct_kernel<o, s><<<grid, 256, 0, st>>>(a); });
     }
-    switch (a.out.kind) {
-        case PB_KIND_CAMERA: launch_direct_s<PB_KIND_CAMERA>(a, grid, st); break;
-        case PB_KIND_DOUBLE: launch_direct_s<PB_KIND_DOUBLE>(a, grid, st); break;
-        default: launch_direct_s<PB_KIND_EQUIRECT>(a, grid, st); break;
-    }
+    PB_COUNT_LAUNCH();
 }
 
 static void launch_generic(const RemapArgs& a, cudaStream_t st) {
-    switch (a.out.kind) {
-        case PB_KIND_CAMERA: launch_generic_s<PB_KIND_CAMERA>(a, st); break;
-        case PB_KIND_DOUBLE: launch_generic_s<PB_KIND_DOUBLE>(a, st); break;
-        default: launch_generic_s<PB_KIND_EQUIRECT>(a, st); break;
-    }
-}
-
-template <int SRC_KIND>
-static void launch_gather_c(const SrcGeom& s, double* map, long long n, const unsigned char* sp,
-                            unsigned char* dst, cudaStream_t st) {
-    const int block = 256;
-    const unsigned grid = (unsigned)((n + block - 1) / block);
-    switch (s.C) {
-        case 1: gather_from_map_kernel<SRC_KIND, 1><<<grid, block, 0, st>>>(s, map, n, sp, dst); PB_COUNT_LAUNCH(); break;
-        case 2: gather_from_map_kernel<SRC_KIND, 2><<<grid, block, 0, st>>>(s, map, n, sp, dst); PB_COUNT_LAUNCH(); break;
-        case 3: gather_from_map_kernel<SRC_KIND, 3><<<grid, block, 0, st>>>(s, map, n, sp, dst); PB_COUNT_LAUNCH(); break;
-        default: gather_from_map_kernel<SRC_KIND, 4><<<grid, block, 0, st>>>(s, map, n, sp, dst); PB_COUNT_LAUNCH(); break;
-    }
-}
-
-// the same for elements of T (2, 4 or 8 bytes), camera / equirect sources
-template <int SRC_KIND, typename T>
-static void launch_gather_wide(const SrcGeom& s, double* map, long long n, const void* src, void* dst, cudaStream_t st) {
-    const int block = 256;
-    const unsigned grid = (unsigned)((n + block - 1) / block);
-    const T* sp = static_cast<const T*>(src);
-    T* dp = static_cast<T*>(dst);
-    switch (s.C) {
-        case 1: gather_from_map_kernel<SRC_KIND, 1, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
-        case 2: gather_from_map_kernel<SRC_KIND, 2, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
-        case 3: gather_from_map_kernel<SRC_KIND, 3, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
-        default: gather_from_map_kernel<SRC_KIND, 4, T><<<grid, block, 0, st>>>(s, map, n, sp, dp); break;
-    }
+    dim3 block(32, 8);
+    dim3 grid((a.out.W + block.x - 1) / block.x, (a.row_end - a.row_begin + block.y - 1) / block.y);
+    with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
+        with_channels(a.src.C, [&](auto c) { remap_generic_kernel<o, s, c><<<grid, block, 0, st>>>(a); });
+    });
     PB_COUNT_LAUNCH();
 }
 
-template <int SRC_KIND>
-static void launch_gather_e(const SrcGeom& s, int elem_bytes, double* map, long long n, const void* src, void* dst,
-                            cudaStream_t st) {
-    switch (elem_bytes) {
-        case 2: launch_gather_wide<SRC_KIND, unsigned short>(s, map, n, src, dst, st); break;
-        case 4: launch_gather_wide<SRC_KIND, unsigned>(s, map, n, src, dst, st); break;
-        default: launch_gather_wide<SRC_KIND, unsigned long long>(s, map, n, src, dst, st); break;
-    }
-}
-
-// fused remap of pixels wider than one byte (pb_wide.cuh): VEC-byte words
-template <int OUT_KIND, int SRC_KIND, bool SEP>
-static void launch_wide_v(const WideArgs& a, int vec, dim3 grid, cudaStream_t st) {
-    switch (vec) {
-        case 16: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 16><<<grid, 256, 0, st>>>(a); break;
-        case 8: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 8><<<grid, 256, 0, st>>>(a); break;
-        case 4: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 4><<<grid, 256, 0, st>>>(a); break;
-        default: remap_wide_kernel<OUT_KIND, SRC_KIND, SEP, 2><<<grid, 256, 0, st>>>(a); break;
-    }
+// explicit-map gather: uint8 elements from any source, or elements of 2, 4 or 8 bytes from a
+// camera / equirect source
+static void launch_gather(const SrcGeom& s, int elem_bytes, double* map, long long n, const void* src, void* dst,
+                          cudaStream_t st) {
+    const int block = 256;
+    const unsigned grid = (unsigned)((n + block - 1) / block);
+    auto gather = [&](auto k, auto t) {
+        using T = decltype(t);
+        with_channels(s.C, [&](auto c) {
+            gather_from_map_kernel<k, c, T><<<grid, block, 0, st>>>(s, map, n, static_cast<const T*>(src),
+                                                                      static_cast<T*>(dst));
+        });
+    };
+    if (elem_bytes == 1)
+        with_kind(s.kind, [&](auto k) { gather(k, (unsigned char)0); });
+    else
+        with_single_kind(s.kind, [&](auto k) { with_elem(elem_bytes, [&](auto t) { gather(k, t); }); });
     PB_COUNT_LAUNCH();
-}
-
-template <int OUT_KIND>
-static void launch_wide_s(const WideArgs& a, int vec, dim3 grid, cudaStream_t st) {
-    if (a.src.kind == PB_KIND_CAMERA) launch_wide_v<OUT_KIND, PB_KIND_CAMERA, false>(a, vec, grid, st);
-    else launch_wide_v<OUT_KIND, PB_KIND_EQUIRECT, false>(a, vec, grid, st);
 }
 
 // The widest word (a power of two, at most 16 bytes) that divides the pixel size and every address
@@ -941,19 +894,24 @@ static bool encode_frames_map(CUtensorMap* map, const void* base, long long pitc
 constexpr int kMaxTiledSmem = 200 * 1024;
 constexpr int kMaxDevices = 64;
 
+// Raises Kernel's dynamic shared-memory limit on the current device to smem when it was given less
+// so far.  The state is per kernel and per device: the attribute belongs to the function on one device.
+template <auto Kernel>
+static cudaError_t reserve_smem(int smem) {
+    static int given[kMaxDevices] = {0};
+    int dev = 0;
+    if (cudaError_t e = cudaGetDevice(&dev)) return e;
+    const bool tracked = dev >= 0 && dev < kMaxDevices;
+    if (tracked && smem <= given[dev]) return cudaSuccess;
+    cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e == cudaSuccess && tracked) given[dev] = smem;
+    return e;
+}
+
 template <int OUT_KIND, int SRC_KIND, int MODE, int CLS = 0>
 static cudaError_t launch_tiled_one(const TiledArgs& a, cudaStream_t st) {
     const int smem = tiled_smem_bytes<SRC_KIND, MODE>(a.stage_bytes, a.n_buffers, a.n_out);
-    // per instantiation and per device: the attribute belongs to the function on one device
-    static bool configured[kMaxDevices] = {false};
-    int dev = 0;
-    if (cudaError_t e = cudaGetDevice(&dev)) return e;
-    if (dev < 0 || dev >= kMaxDevices || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(remap_tiled_kernel<OUT_KIND, SRC_KIND, MODE, CLS>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxTiledSmem);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < kMaxDevices) configured[dev] = true;
-    }
+    if (cudaError_t e = reserve_smem<remap_tiled_kernel<OUT_KIND, SRC_KIND, MODE, CLS>>(kMaxTiledSmem)) return e;
     const int grid = a.tile_list ? a.n_list : a.tiles_x * a.tiles_y;
     if (grid <= 0) return cudaSuccess;
     remap_tiled_kernel<OUT_KIND, SRC_KIND, MODE, CLS><<<grid, kTileThreads, smem, st>>>(a);
@@ -961,39 +919,19 @@ static cudaError_t launch_tiled_one(const TiledArgs& a, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-template <int OUT_KIND>
-static cudaError_t launch_tiled_generic_s(const TiledArgs& a, cudaStream_t st) {
-    switch (a.src.kind) {
-        case PB_KIND_CAMERA: return launch_tiled_one<OUT_KIND, PB_KIND_CAMERA, 0>(a, st);
-        case PB_KIND_DOUBLE: return launch_tiled_one<OUT_KIND, PB_KIND_DOUBLE, 0>(a, st);
-        default: return launch_tiled_one<OUT_KIND, PB_KIND_EQUIRECT, 0>(a, st);
-    }
-}
-
 static cudaError_t launch_tiled(const TiledArgs& a, bool separable, cudaStream_t st) {
     if (separable) {
         if (a.src.kind == PB_KIND_CAMERA) return launch_tiled_one<PB_KIND_EQUIRECT, PB_KIND_CAMERA, 1>(a, st);
         return launch_tiled_one<PB_KIND_EQUIRECT, PB_KIND_DOUBLE, 1>(a, st);
     }
-    switch (a.out.kind) {
-        case PB_KIND_CAMERA: return launch_tiled_generic_s<PB_KIND_CAMERA>(a, st);
-        case PB_KIND_DOUBLE: return launch_tiled_generic_s<PB_KIND_DOUBLE>(a, st);
-        default: return launch_tiled_generic_s<PB_KIND_EQUIRECT>(a, st);
-    }
+    return with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) { return launch_tiled_one<o, s, 0>(a, st); });
 }
 
 // batches with the source staged as a chunk list (pb_chunk.cuh)
 template <int SRC_KIND, int CLS>
 static cudaError_t launch_chunk_one(const TiledArgs& a, cudaStream_t st) {
     const int smem = chunk_smem_bytes(a.stage_bytes);
-    static int max_smem_set[kMaxDevices] = {0};
-    int dev = 0;
-    if (cudaError_t e = cudaGetDevice(&dev)) return e;
-    if (dev < 0 || dev >= kMaxDevices || smem > max_smem_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(remap_chunk_kernel<SRC_KIND, CLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < kMaxDevices) max_smem_set[dev] = smem;
-    }
+    if (cudaError_t e = reserve_smem<remap_chunk_kernel<SRC_KIND, CLS>>(smem)) return e;
     const int grid = a.tile_list ? a.n_list : a.tiles_x * a.tiles_y;
     if (grid <= 0) return cudaSuccess;
     remap_chunk_kernel<SRC_KIND, CLS><<<grid, kTileThreads, smem, st>>>(a);
@@ -1004,14 +942,7 @@ static cudaError_t launch_chunk_one(const TiledArgs& a, cudaStream_t st) {
 // the two-lens / blend-band class of a batch with 512 threads per CTA (pb_tiled2.cuh)
 static cudaError_t launch_two_lens(const TiledArgs& a, cudaStream_t st) {
     const int smem = two_lens_smem_bytes(a.stage_bytes);
-    static int max_smem_set[kMaxDevices] = {0};
-    int dev = 0;
-    if (cudaError_t e = cudaGetDevice(&dev)) return e;
-    if (dev < 0 || dev >= kMaxDevices || smem > max_smem_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(remap_two_lens_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < kMaxDevices) max_smem_set[dev] = smem;
-    }
+    if (cudaError_t e = reserve_smem<remap_two_lens_kernel>(smem)) return e;
     if (a.n_list <= 0) return cudaSuccess;
     remap_two_lens_kernel<<<a.n_list, kTile2Threads, smem, st>>>(a);
     PB_COUNT_LAUNCH();
@@ -1031,15 +962,10 @@ static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 template <int SRC_KIND, int NB, int CLS = 0>
 static cudaError_t launch_sep1_one(const TiledArgs& a, cudaStream_t st) {
     const int smem = sep1_smem_bytes(a.sep1_cap, SRC_KIND == PB_KIND_DOUBLE, NB);
-    static int max_smem_set[kMaxDevices] = {0};  // per device: the attribute belongs to the function on one device
     int dev = 0, sms = 0, per_sm = 0;
-    cudaError_t e = cudaGetDevice(&dev);
+    cudaError_t e = reserve_smem<remap_sep1_kernel<SRC_KIND, NB, CLS>>(smem);
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
-    if (dev < 0 || dev >= kMaxDevices || smem > max_smem_set[dev]) {
-        e = cudaFuncSetAttribute(remap_sep1_kernel<SRC_KIND, NB, CLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < kMaxDevices) max_smem_set[dev] = smem;
-    }
     e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (e == cudaSuccess)
         e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, remap_sep1_kernel<SRC_KIND, NB, CLS>, kTileThreads, smem);
@@ -1217,6 +1143,50 @@ static const int4* footprint_table(const pb_plan& p, const double* tables) {
     return reinterpret_cast<const int4*>(tables + 2 * (size_t)p.out.W + 4 * (size_t)p.out.H);
 }
 
+// Kernel arguments of a plan: what every launch through it sets the same way
+static RemapArgs remap_args(const pb_plan& p) {
+    RemapArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.out = p.out;
+    a.src = p.src;
+    a.rot = p.rot;
+    a.fast = p.fast;
+    return a;
+}
+// tables: the plan's own, a transient copy, or null (generic rays)
+static TiledArgs tiled_args(const pb_plan& p, const double* tables) {
+    TiledArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.out = p.out;
+    a.src = p.src;
+    a.rot = p.rot;
+    a.fast = p.fast;
+    a.col_tab = tables;
+    a.row_tab = tables ? tables + 2 * (size_t)p.out.W : nullptr;
+    a.tile_fp = tables ? footprint_table(p, tables) : nullptr;
+    a.sep1_tab = tables ? sep1_table(p, tables) : nullptr;
+    a.sep1_col = tables ? sep1_col(p, tables) : nullptr;
+    a.sep1_row = tables ? sep1_row(p, tables) : nullptr;
+    a.tiles_x = tiles_x(p);
+    a.tiles_y = tiles_y(p);
+    a.raster_band = p.raster_band;
+    return a;
+}
+
+// The smallest bin k of the histogram h[0, n) such that bins 0..k hold all but 1/200 of its items;
+// -1 for an empty histogram.
+static int covering_bin(const int* h, int n) {
+    long long items = 0;
+    for (int k = 0; k < n; ++k) items += h[k];
+    if (items <= 0) return -1;
+    long long acc = 0;
+    for (int k = 0; k < n; ++k) {
+        acc += h[k];
+        if (acc >= items - items / 200) return k;
+    }
+    return n - 1;
+}
+
 // Picks the stage-buffer capacity from the census h (see kProbeSizeBins): the smallest size that
 // holds the footprint of all but 0.5 % of the (tile, slot) items -- the rest gather straight from
 // global memory -- so that the buffers are as small, and the occupancy as high, as the geometry
@@ -1225,16 +1195,8 @@ static const int4* footprint_table(const pb_plan& p, const double* tables) {
 // them, which is what the gather of a tile whose footprint runs down the source image would
 // otherwise do (tests/analysis/stage_sim.py: 4.4 -> 2.3 wavefronts per LDS at pitch 256 -> 272).
 static void pick_stage(pb_plan& p, const int* h) {
-    long long items = 0;
-    for (int k = 0; k < kProbeSizeBins; ++k) items += h[k];
-    if (items <= 0) return;
-    const long long need = items - items / 200;
-    long long acc = 0;
-    int kib = kProbeSizeBins - 1;
-    for (int k = 0; k < kProbeSizeBins; ++k) {
-        acc += h[k];
-        if (acc >= need) { kib = k; break; }
-    }
+    int kib = covering_bin(h, kProbeSizeBins);
+    if (kib < 0) return;
     if (kib < 2) kib = 2;
     if (kib > 48) kib = 48;
     if (const char* e = std::getenv("PB_STAGE_KIB")) kib = std::atoi(e);  // tuning experiments
@@ -1304,29 +1266,30 @@ static void classify_tiles(pb_plan& p, const int4* fp, cudaStream_t st) {
         (void)cudaGetLastError();
         return;
     }
-    if (p.n_one > 0)
+    if (p.n_one > 0) {
         pb_sep1_table_kernel<<<(p.n_one + 255) / 256, 256, 0, st>>>(footprint_table(p, p.tables), cls, tx, ty, p.raster_band,
                                                                    2, lists, p.n_one, 1);
-    if (p.n_rest > 0)
+        PB_COUNT_LAUNCH();
+    }
+    if (p.n_rest > 0) {
         pb_sep1_table_kernel<<<(p.n_rest + 255) / 256, 256, 0, st>>>(footprint_table(p, p.tables), cls + p.n_one, tx, ty,
                                                                     p.raster_band, 2, lists + p.n_one, p.n_rest, 0);
+        PB_COUNT_LAUNCH();
+    }
     if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) {
         (void)cudaGetLastError();
         cudaFree(cls);
         return;
     }
-    std::vector<int> kib;
+    std::vector<int> hist(129);  // KiB; 128: that or more, or not stageable
     for (int i = 0; i < p.n_one; ++i) {
         const int t = one[i];
         const int4& f = fp[2 * t].z > 0 ? fp[2 * t] : fp[2 * t + 1];
         const int units = stage_units(f.w >> 1);
-        kib.push_back(units <= kMaxStageUnits ? (f.z * kBoxRows * 16 * units + 1023) >> 10 : 1 << 20);
+        hist[units <= kMaxStageUnits ? std::min((f.z * kBoxRows * 16 * units + 1023) >> 10, 128) : 128] += 1;
     }
-    if (!kib.empty()) {
-        std::sort(kib.begin(), kib.end());
-        int k = kib[kib.size() - 1 - kib.size() / 200];
-        p.sep1_cap_one = std::min(std::max(k, 4), 96) * 1024;
-    }
+    const int k = covering_bin(hist.data(), 129);
+    if (k >= 0) p.sep1_cap_one = std::min(std::max(k, 4), 96) * 1024;
     p.sep1_cls = cls;
     // the side stream carries the latency-bound grid (two-lens tiles) at the highest priority: its
     // CTAs are dispatched first wherever an SM has room, so they mix with the bandwidth-bound
@@ -1463,11 +1426,7 @@ static void tune_stage(pb_plan& p, cudaStream_t st) {
                     hist[kib > 128 ? 128 : (int)kib] += 1;
                     counted += 1;
                 }
-                int acc = 0, kib = 128;
-                for (int k = 0; k <= 128; ++k) {
-                    acc += hist[k];
-                    if (acc >= counted - counted / 200) { kib = k; break; }
-                }
+                int kib = covering_bin(hist, 129);
                 if (kib < 4) kib = 4;
                 if (kib > 96) kib = 96;
                 if (const char* e = std::getenv("PB_SEP1_KIB")) kib = std::atoi(e);  // tuning experiments
@@ -1506,14 +1465,7 @@ static void tune_stage(pb_plan& p, cudaStream_t st) {
         return;
     }
     cudaMemsetAsync(census, 0, sizeof(h), st);
-    TiledArgs a;
-    std::memset(&a, 0, sizeof(a));
-    a.out = p.out;
-    a.src = p.src;
-    a.rot = p.rot;
-    a.fast = p.fast;
-    a.col_tab = p.tables;
-    a.row_tab = p.tables ? p.tables + 2 * (size_t)p.out.W : nullptr;
+    TiledArgs a = tiled_args(p, p.tables);
     a.n_frames = 0;
     a.src_pitch = p.src.W * 3;
     a.stage_bytes = 256;
@@ -1521,8 +1473,6 @@ static void tune_stage(pb_plan& p, cudaStream_t st) {
     a.n_buffers = 1;
     a.n_out = 1;
     a.probe = census;
-    a.tiles_x = tiles_x(p);
-    a.tiles_y = tiles_y(p);
     a.raster_band = 0;
     if (launch_tiled(a, p.separable && p.tables != nullptr, st) == cudaSuccess &&
         cudaMemcpyAsync(h, census, sizeof(h), cudaMemcpyDeviceToHost, st) == cudaSuccess &&
@@ -1540,15 +1490,10 @@ static cudaError_t fill_tables(const pb_plan& p, double* tables, cudaStream_t st
     PB_COUNT_LAUNCH();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    TiledArgs a;
-    std::memset(&a, 0, sizeof(a));
-    a.out = p.out;
-    a.src = p.src;
-    a.col_tab = tables;
-    a.row_tab = tables + 2 * (size_t)p.out.W;
     const int n_entries = footprint_entries(p);
-    pb_footprint_kernel<<<(n_entries + 7) / 8, 256, 0, st>>>(a, const_cast<int4*>(footprint_table(p, tables)),
-                                                           tiles_x(p), n_entries);
+    pb_footprint_kernel<<<(n_entries + 7) / 8, 256, 0, st>>>(tiled_args(p, tables),
+                                                           const_cast<int4*>(footprint_table(p, tables)), tiles_x(p),
+                                                           n_entries);
     PB_COUNT_LAUNCH();
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
@@ -1592,49 +1537,33 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
     static const bool direct_off = std::getenv("PB_DIRECT") && std::atoi(std::getenv("PB_DIRECT")) == 0;  // experiments
     // (a separable geometry takes the tiled kernels when the band starts on a tile row)
     const bool separable_run = p.separable && tables != nullptr && row_begin % kTileH == 0;
+    // the arguments of the direct and the generic kernel
+    RemapArgs ra = remap_args(p);
+    ra.src_px = src;
+    ra.dst_px = dst;
+    ra.src_frame_stride = src_frame_stride;
+    ra.dst_frame_stride = dst_frame_stride;
+    ra.n_frames = n_frames;
+    ra.row_begin = row_begin;
+    ra.row_end = row_end;
     if (n_frames == 1 && !separable_run && !direct_off && C == 3 && p.out.W % 4 == 0 &&
         (reinterpret_cast<uintptr_t>(dst) & 3u) == 0 && src_pitch * p.src.H < (1LL << 31) &&
         (p.out.H + kTileH - 1) / kTileH < 65536) {
-        RemapArgs a;
-        a.out = p.out;
-        a.src = p.src;
-        a.rot = p.rot;
-        a.fast = p.fast;
-        a.src_px = src;
-        a.dst_px = dst;
-        a.src_frame_stride = src_frame_stride;
-        a.dst_frame_stride = dst_frame_stride;
-        a.n_frames = 1;
-        a.row_begin = row_begin;
-        a.row_end = row_end;
-        launch_direct(a, st);
+        launch_direct(ra, st);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return cuda_fail(e, "direct remap launch");
         return PB_OK;
     }
     static const bool tiled_off = std::getenv("PB_TILED") && std::atoi(std::getenv("PB_TILED")) == 0;  // experiments
     if (tiled_ok && !tiled_off && row_begin % kTileH == 0) {
-        TiledArgs a;
-        std::memset(&a, 0, sizeof(a));
-        a.out = p.out;
-        a.src = p.src;
-        a.rot = p.rot;
-        a.fast = p.fast;
-        a.col_tab = tables;
-        a.row_tab = tables ? tables + 2 * (size_t)p.out.W : nullptr;
-        a.tile_fp = tables ? footprint_table(p, tables) : nullptr;
-        a.sep1_tab = tables ? sep1_table(p, tables) : nullptr;
-        a.sep1_col = tables ? sep1_col(p, tables) : nullptr;
-        a.sep1_row = tables ? sep1_row(p, tables) : nullptr;
+        TiledArgs a = tiled_args(p, tables);
         a.sep1_cap = p.sep1_cap;
         a.src_px = src;
         a.src_frame_stride = src_frame_stride;
         a.n_frames = n_frames;
         a.src_pitch = (int)src_pitch;
-        a.tiles_x = tiles_x(p);
         a.tile_y0 = row_begin / kTileH;
         a.tiles_y = (row_end - row_begin + kTileH - 1) / kTileH;
-        a.raster_band = p.raster_band;
         // L2 prefetch (UTMAPF) of frames beyond those in flight: worth +7 % on a single-lens source
         // while tiles kept two frames in flight; with the ring of frame groups it is neutral
         // (8K target) or harmful (double source, -8 %), so it is off  (gpurun_out/run3.log, run12.log)
@@ -1759,19 +1688,7 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
         }
         // no tensor-map encoder in this driver: the generic kernel below needs none
     }
-    RemapArgs a;
-    a.out = p.out;
-    a.src = p.src;
-    a.rot = p.rot;
-    a.fast = p.fast;
-    a.src_px = src;
-    a.dst_px = dst;
-    a.src_frame_stride = src_frame_stride;
-    a.dst_frame_stride = dst_frame_stride;
-    a.n_frames = n_frames;
-    a.row_begin = row_begin;
-    a.row_end = row_end;
-    launch_generic(a, st);
+    launch_generic(ra, st);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "generic remap launch");
     return PB_OK;
@@ -1805,38 +1722,107 @@ static int plan_run_wide(const pb_plan& p, int elem_bytes, const void* src, int6
     const int vec = wide_vec(a.px_bytes, src, dst, src_frame_stride, dst_frame_stride, n_frames > 1);
     a.words = a.px_bytes / vec;
     const dim3 grid((p.out.W + kTileW - 1) / kTileW, (unsigned)tiles_y);
-    if (sep) {
-        launch_wide_v<PB_KIND_EQUIRECT, PB_KIND_CAMERA, true>(a, vec, grid, st);
-    } else {
-        switch (p.out.kind) {
-            case PB_KIND_CAMERA: launch_wide_s<PB_KIND_CAMERA>(a, vec, grid, st); break;
-            case PB_KIND_DOUBLE: launch_wide_s<PB_KIND_DOUBLE>(a, vec, grid, st); break;
-            default: launch_wide_s<PB_KIND_EQUIRECT>(a, vec, grid, st); break;
+    with_vec(vec, [&](auto v) {
+        if (sep) {
+            remap_wide_kernel<PB_KIND_EQUIRECT, PB_KIND_CAMERA, true, v><<<grid, 256, 0, st>>>(a);
+        } else {
+            with_kind(p.out.kind, [&](auto o) {
+                with_single_kind(p.src.kind,
+                                 [&](auto s) { remap_wide_kernel<o, s, false, v><<<grid, 256, 0, st>>>(a); });
+            });
         }
-    }
+    });
+    PB_COUNT_LAUNCH();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "wide remap launch");
     return PB_OK;
 }
 
-// Arguments of the _px entry points that need no device: the element width, then pointers and
-// strides against it.  -> PB_OK, or the code with pb_last_error set.
+// Arguments of the entry points that need no device: the element width, then for elements wider
+// than a byte the source kind, and pointers and strides against the width.  -> PB_OK, or the code
+// with pb_last_error set.
 static int check_elem_bytes(int32_t elem_bytes, const char* who) {
     if (elem_bytes != 1 && elem_bytes != 2 && elem_bytes != 4 && elem_bytes != 8)
         return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": elem_bytes must be 1, 2, 4 or 8 (got " +
                                             std::to_string(elem_bytes) + ")");
     return PB_OK;
 }
-static int check_double_source(int src_kind, const char* who) {
+static int check_wide(int32_t elem_bytes, int src_kind, const void* src, long long src_stride, const void* dst,
+                      long long dst_stride, const char* who) {
+    if (elem_bytes == 1) return PB_OK;
     if (src_kind == PB_KIND_DOUBLE)
         return fail(PB_ERR_UNSUPPORTED, std::string(who) +
                                             ": a double-fisheye source blends its two lenses into uint8 "
                                             "(projection.py:459); only elem_bytes == 1 is supported for it");
+    auto whole = [&](const void* q, long long stride) {
+        return reinterpret_cast<uintptr_t>(q) % (uintptr_t)elem_bytes == 0 && stride % elem_bytes == 0;
+    };
+    if (!whole(src, src_stride) || !whole(dst, dst_stride))
+        return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": pointer or stride not a multiple of elem_bytes");
     return PB_OK;
 }
-static int check_aligned(const void* p, long long stride, int32_t elem_bytes, const char* who) {
-    if ((reinterpret_cast<uintptr_t>(p) % (uintptr_t)elem_bytes) != 0 || stride % elem_bytes != 0)
-        return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": pointer or stride not a multiple of elem_bytes");
+static int check_plan_device(const pb_plan* plan, const char* who) {
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
+        return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": plan belongs to another device");
+    return PB_OK;
+}
+
+// The bodies of the _u8 (elem_bytes == 1) and _px entry points; who names the entry point.
+static int plan_remap(const char* who, const pb_plan* plan, int32_t elem_bytes, const void* src,
+                      int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames, void* stream) {
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!plan || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
+    if (int rc = check_wide(elem_bytes, plan->src.kind, src, src_frame_stride, dst, dst_frame_stride, who)) return rc;
+    if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": negative n_frames");
+    if (n_frames == 0) return PB_OK;
+    if (int rc = check_plan_device(plan, who)) return rc;
+    if (elem_bytes > 1)
+        return plan_run_wide(*plan, elem_bytes, src, src_frame_stride, dst, dst_frame_stride, n_frames,
+                             (cudaStream_t)stream);
+    return plan_run(*const_cast<pb_plan*>(plan), plan->tables, static_cast<const uint8_t*>(src), src_frame_stride,
+                    static_cast<uint8_t*>(dst), dst_frame_stride, n_frames, (cudaStream_t)stream);
+}
+
+static int plan_remap_rows(const char* who, const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band,
+                           int32_t row_begin, int32_t row_end, void* stream) {
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!plan || !src || !dst_band) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
+    if (int rc = check_wide(elem_bytes, plan->src.kind, src, 0, dst_band, 0, who)) return rc;
+    if (row_begin < 0 || row_end > plan->out.H || row_begin > row_end)
+        return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": rows outside the output image");
+    if (row_begin == row_end) return PB_OK;
+    if (int rc = check_plan_device(plan, who)) return rc;
+    if (elem_bytes > 1)
+        return plan_run_wide(*plan, elem_bytes, src, 0, dst_band, 0, 1, (cudaStream_t)stream, row_begin, row_end);
+    return plan_run(*const_cast<pb_plan*>(plan), plan->tables, static_cast<const uint8_t*>(src), 0,
+                    static_cast<uint8_t*>(dst_band), 0, 1, (cudaStream_t)stream, row_begin, row_end);
+}
+
+static int gather_from_map(const char* who, const pb_image_desc* src_desc, int32_t channels, int32_t elem_bytes,
+                           double* map, int32_t map_height, int32_t map_width, const void* src, void* dst,
+                           void* stream) {
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!src_desc || !map || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
+    if (int rc = check_image(*src_desc, "src")) return rc;
+    if (int rc = check_wide(elem_bytes, src_desc->kind, src, 0, dst, 0, who)) return rc;
+    // source_lookup packs a source pixel as row << 16 | column
+    if (src_desc->height > 32767 || src_desc->width > 65535)
+        return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": source larger than 32767 rows x 65535 columns");
+    if (channels < 1 || channels > 4) return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": channels must be 1..4");
+    if (map_height < 0 || map_width < 0) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": negative map size");
+    const long long n = (long long)map_height * map_width;
+    if (n == 0) return PB_OK;
+    if ((n + 255) / 256 > 0x7fffffffLL) return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": map too large");
+    SrcGeom s = derive_src(*src_desc, channels);
+    cudaStream_t st = (cudaStream_t)stream;
+    double* luts = nullptr;
+    if (cudaError_t eu = upload_lens_tables(nullptr, nullptr, src_desc, &s, &luts, st, true))
+        return cuda_fail(eu, (std::string(who) + " lens table").c_str());
+    launch_gather(s, elem_bytes, map, n, src, dst, st);
+    cudaError_t e = cudaGetLastError();
+    if (luts) cudaFreeAsync(luts, st);
+    if (e != cudaSuccess) return cuda_fail(e, (std::string(who) + " launch").c_str());
     return PB_OK;
 }
 
@@ -1906,23 +1892,19 @@ static void calibrate_fast32(pb_plan& p, cudaStream_t st) {
         if (std::atoi(e) == 0) return;
     }
     const Fast32GeomT<double> gd = derive_fast32(p.out, p.src, p.fast);
-    RemapArgs a;
-    std::memset(&a, 0, sizeof(a));
-    a.out = p.out;
-    a.src = p.src;
-    a.rot = p.rot;
-    a.fast = p.fast;
+    const RemapArgs a = remap_args(p);
     unsigned* dev = nullptr;
     if (cudaMalloc((void**)&dev, sizeof(unsigned)) != cudaSuccess) {
         (void)cudaGetLastError();
         return;
     }
     cudaMemsetAsync(dev, 0, sizeof(unsigned), st);
-    switch (a.out.kind) {
-        case PB_KIND_CAMERA: launch_ratio_s<PB_KIND_CAMERA>(a, gd, dev, st); break;
-        case PB_KIND_DOUBLE: launch_ratio_s<PB_KIND_DOUBLE>(a, gd, dev, st); break;
-        default: launch_ratio_s<PB_KIND_EQUIRECT>(a, gd, dev, st); break;
-    }
+    dim3 block(32, 8);
+    dim3 grid((a.out.W + block.x - 1) / block.x, (a.out.H + block.y - 1) / block.y);
+    with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
+        fast32_ratio_kernel<o, s><<<grid, block, 0, st>>>(a, gd, dev);
+    });
+    PB_COUNT_LAUNCH();
     unsigned bits = 0;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(&bits, dev, sizeof(bits), cudaMemcpyDeviceToHost, st);
@@ -1987,66 +1969,23 @@ int pb_debug_plan_fast32(const pb_plan* plan, double out[2]) {
 
 int pb_plan_remap_u8(const pb_plan* plan, const uint8_t* src, int64_t src_frame_stride, uint8_t* dst,
                      int64_t dst_frame_stride, int32_t n_frames, void* stream) {
-    if (!plan || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_u8: null pointer");
-    if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_u8: negative n_frames");
-    if (n_frames == 0) return PB_OK;
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
-        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_u8: plan belongs to another device");
-    return plan_run(*const_cast<pb_plan*>(plan), plan->tables, src, src_frame_stride, dst, dst_frame_stride, n_frames,
-                    (cudaStream_t)stream);
+    return plan_remap("pb_plan_remap_u8", plan, 1, src, src_frame_stride, dst, dst_frame_stride, n_frames, stream);
 }
 
 int pb_plan_remap_rows_u8(const pb_plan* plan, const uint8_t* src, uint8_t* dst_band, int32_t row_begin, int32_t row_end,
                           void* stream) {
-    if (!plan || !src || !dst_band) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_u8: null pointer");
-    if (row_begin < 0 || row_end > plan->out.H || row_begin > row_end)
-        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_u8: rows outside the output image");
-    if (row_begin == row_end) return PB_OK;
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
-        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_u8: plan belongs to another device");
-    return plan_run(*const_cast<pb_plan*>(plan), plan->tables, src, 0, dst_band, 0, 1, (cudaStream_t)stream, row_begin,
-                    row_end);
+    return plan_remap_rows("pb_plan_remap_rows_u8", plan, 1, src, dst_band, row_begin, row_end, stream);
 }
 
 int pb_plan_remap_px(const pb_plan* plan, int32_t elem_bytes, const void* src, int64_t src_frame_stride, void* dst,
                      int64_t dst_frame_stride, int32_t n_frames, void* stream) {
-    const char* who = "pb_plan_remap_px";
-    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
-    if (!plan || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_px: null pointer");
-    if (elem_bytes == 1)
-        return pb_plan_remap_u8(plan, static_cast<const uint8_t*>(src), src_frame_stride, static_cast<uint8_t*>(dst),
-                                dst_frame_stride, n_frames, stream);
-    if (int rc = check_double_source(plan->src.kind, who)) return rc;
-    if (int rc = check_aligned(src, src_frame_stride, elem_bytes, who)) return rc;
-    if (int rc = check_aligned(dst, dst_frame_stride, elem_bytes, who)) return rc;
-    if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_px: negative n_frames");
-    if (n_frames == 0) return PB_OK;
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
-        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_px: plan belongs to another device");
-    return plan_run_wide(*plan, elem_bytes, src, src_frame_stride, dst, dst_frame_stride, n_frames, (cudaStream_t)stream);
+    return plan_remap("pb_plan_remap_px", plan, elem_bytes, src, src_frame_stride, dst, dst_frame_stride, n_frames,
+                      stream);
 }
 
 int pb_plan_remap_rows_px(const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band, int32_t row_begin,
                           int32_t row_end, void* stream) {
-    const char* who = "pb_plan_remap_rows_px";
-    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
-    if (!plan || !src || !dst_band) return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_px: null pointer");
-    if (elem_bytes == 1)
-        return pb_plan_remap_rows_u8(plan, static_cast<const uint8_t*>(src), static_cast<uint8_t*>(dst_band), row_begin,
-                                     row_end, stream);
-    if (int rc = check_double_source(plan->src.kind, who)) return rc;
-    if (int rc = check_aligned(src, 0, elem_bytes, who)) return rc;
-    if (int rc = check_aligned(dst_band, 0, elem_bytes, who)) return rc;
-    if (row_begin < 0 || row_end > plan->out.H || row_begin > row_end)
-        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_px: rows outside the output image");
-    if (row_begin == row_end) return PB_OK;
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev != plan->device)
-        return fail(PB_ERR_INVALID_ARGUMENT, "pb_plan_remap_rows_px: plan belongs to another device");
-    return plan_run_wide(*plan, elem_bytes, src, 0, dst_band, 0, 1, (cudaStream_t)stream, row_begin, row_end);
+    return plan_remap_rows("pb_plan_remap_rows_px", plan, elem_bytes, src, dst_band, row_begin, row_end, stream);
 }
 
 void pb_plan_destroy(pb_plan* plan) {
@@ -2079,11 +2018,8 @@ int pb_materialize_map_f64(const pb_remap_desc* desc, double* map, void* stream)
     double* luts = nullptr;
     if (cudaError_t eu = upload_lens_tables(&desc->out, &g, nullptr, nullptr, &luts, st, true))
         return cuda_fail(eu, "pb_materialize_map_f64 lens table");
-    switch (g.kind) {
-        case PB_KIND_CAMERA: materialize_map_kernel<PB_KIND_CAMERA><<<grid, block, 0, st>>>(g, rot, map); PB_COUNT_LAUNCH(); break;
-        case PB_KIND_DOUBLE: materialize_map_kernel<PB_KIND_DOUBLE><<<grid, block, 0, st>>>(g, rot, map); PB_COUNT_LAUNCH(); break;
-        default: materialize_map_kernel<PB_KIND_EQUIRECT><<<grid, block, 0, st>>>(g, rot, map); PB_COUNT_LAUNCH(); break;
-    }
+    with_kind(g.kind, [&](auto k) { materialize_map_kernel<k><<<grid, block, 0, st>>>(g, rot, map); });
+    PB_COUNT_LAUNCH();
     cudaError_t e = cudaGetLastError();
     if (luts) cudaFreeAsync(luts, st);
     if (e != cudaSuccess) return cuda_fail(e, "pb_materialize_map_f64 launch");
@@ -2121,23 +2057,19 @@ int pb_debug_fast32_stats(const pb_remap_desc* desc, double stats[6], void* stre
     pb_plan p;
     plan_init(p, *desc);
     const Fast32GeomT<double> gd = derive_fast32(p.out, p.src, p.fast);
-    RemapArgs a;
-    std::memset(&a, 0, sizeof(a));
-    a.out = p.out;
-    a.src = p.src;
-    a.rot = p.rot;
-    a.fast = p.fast;
+    const RemapArgs a = remap_args(p);
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long* dev = nullptr;
     cudaError_t e = cudaMalloc((void**)&dev, 8 * sizeof(unsigned long long));
     if (e != cudaSuccess) return cuda_fail(e, "pb_debug_fast32_stats");
     cudaMemsetAsync(dev, 0, 8 * sizeof(unsigned long long), st);
     unsigned* maxima = reinterpret_cast<unsigned*>(dev + 4);
-    switch (a.out.kind) {
-        case PB_KIND_CAMERA: launch_stats_s<PB_KIND_CAMERA>(a, gd, maxima, dev, st); break;
-        case PB_KIND_DOUBLE: launch_stats_s<PB_KIND_DOUBLE>(a, gd, maxima, dev, st); break;
-        default: launch_stats_s<PB_KIND_EQUIRECT>(a, gd, maxima, dev, st); break;
-    }
+    dim3 block(32, 8);
+    dim3 grid((a.out.W + block.x - 1) / block.x, (a.out.H + block.y - 1) / block.y);
+    with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
+        fast32_stats_kernel<o, s><<<grid, block, 0, st>>>(a, gd, maxima, dev);
+    });
+    PB_COUNT_LAUNCH();
     unsigned long long host[8];
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(host, dev, sizeof(host), cudaMemcpyDeviceToHost, st);
@@ -2171,62 +2103,13 @@ int pb_rotate_map_f64(const double matrix[9], double* map_in, double* map_out, i
 
 int pb_gather_from_map_u8(const pb_image_desc* src_desc, int32_t channels, double* map, int32_t map_height,
                           int32_t map_width, const uint8_t* src, uint8_t* dst, void* stream) {
-    if (!src_desc || !map || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, "pb_gather_from_map_u8: null pointer");
-    if (int rc = check_image(*src_desc, "src")) return rc;
-    // source_lookup packs a source pixel as row << 16 | column
-    if (src_desc->height > 32767 || src_desc->width > 65535)
-        return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_u8: source larger than 32767 rows x 65535 columns");
-    if (channels < 1 || channels > 4) return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_u8: channels must be 1..4");
-    if (map_height < 0 || map_width < 0) return fail(PB_ERR_INVALID_ARGUMENT, "pb_gather_from_map_u8: negative map size");
-    const long long n = (long long)map_height * map_width;
-    if (n == 0) return PB_OK;
-    if ((n + 255) / 256 > 0x7fffffffLL) return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_u8: map too large");
-    SrcGeom s = derive_src(*src_desc, channels);
-    cudaStream_t st = (cudaStream_t)stream;
-    double* luts = nullptr;
-    if (cudaError_t eu = upload_lens_tables(nullptr, nullptr, src_desc, &s, &luts, st, true))
-        return cuda_fail(eu, "pb_gather_from_map_u8 lens table");
-    switch (s.kind) {
-        case PB_KIND_CAMERA: launch_gather_c<PB_KIND_CAMERA>(s, map, n, src, dst, st); break;
-        case PB_KIND_DOUBLE: launch_gather_c<PB_KIND_DOUBLE>(s, map, n, src, dst, st); break;
-        default: launch_gather_c<PB_KIND_EQUIRECT>(s, map, n, src, dst, st); break;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (luts) cudaFreeAsync(luts, st);
-    if (e != cudaSuccess) return cuda_fail(e, "pb_gather_from_map_u8 launch");
-    return PB_OK;
+    return gather_from_map("pb_gather_from_map_u8", src_desc, channels, 1, map, map_height, map_width, src, dst, stream);
 }
 
 int pb_gather_from_map_px(const pb_image_desc* src_desc, int32_t channels, int32_t elem_bytes, double* map,
                           int32_t map_height, int32_t map_width, const void* src, void* dst, void* stream) {
-    const char* who = "pb_gather_from_map_px";
-    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
-    if (!src_desc || !map || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, "pb_gather_from_map_px: null pointer");
-    if (elem_bytes == 1)
-        return pb_gather_from_map_u8(src_desc, channels, map, map_height, map_width, static_cast<const uint8_t*>(src),
-                                     static_cast<uint8_t*>(dst), stream);
-    if (int rc = check_image(*src_desc, "src")) return rc;
-    if (int rc = check_double_source(src_desc->kind, who)) return rc;
-    if (int rc = check_aligned(src, 0, elem_bytes, who)) return rc;
-    if (int rc = check_aligned(dst, 0, elem_bytes, who)) return rc;
-    if (src_desc->height > 32767 || src_desc->width > 65535)
-        return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_px: source larger than 32767 rows x 65535 columns");
-    if (channels < 1 || channels > 4) return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_px: channels must be 1..4");
-    if (map_height < 0 || map_width < 0) return fail(PB_ERR_INVALID_ARGUMENT, "pb_gather_from_map_px: negative map size");
-    const long long n = (long long)map_height * map_width;
-    if (n == 0) return PB_OK;
-    if ((n + 255) / 256 > 0x7fffffffLL) return fail(PB_ERR_UNSUPPORTED, "pb_gather_from_map_px: map too large");
-    SrcGeom s = derive_src(*src_desc, channels);
-    cudaStream_t st = (cudaStream_t)stream;
-    double* luts = nullptr;
-    if (cudaError_t eu = upload_lens_tables(nullptr, nullptr, src_desc, &s, &luts, st, true))
-        return cuda_fail(eu, "pb_gather_from_map_px lens table");
-    if (s.kind == PB_KIND_CAMERA) launch_gather_e<PB_KIND_CAMERA>(s, elem_bytes, map, n, src, dst, st);
-    else launch_gather_e<PB_KIND_EQUIRECT>(s, elem_bytes, map, n, src, dst, st);
-    cudaError_t e = cudaGetLastError();
-    if (luts) cudaFreeAsync(luts, st);
-    if (e != cudaSuccess) return cuda_fail(e, "pb_gather_from_map_px launch");
-    return PB_OK;
+    return gather_from_map("pb_gather_from_map_px", src_desc, channels, elem_bytes, map, map_height, map_width, src, dst,
+                           stream);
 }
 
 }  // extern "C"
