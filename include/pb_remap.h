@@ -220,6 +220,16 @@ int pb_debug_fast32_stats(const pb_remap_desc *desc, double stats[6], void *stre
  */
 int pb_debug_plan_fast32(const pb_plan *plan, double out[2]);
 
+/*
+ * The per-box extents a plan of a separable double-fisheye geometry stages for batches (csrc/pb_boxes.cuh),
+ * synchronous: dims = {tiles_y, tiles_x, boxes per (tile, slot)}, all 0 when the plan has no such table.
+ * With table non-null (capacity >= tiles_y * tiles_x * 2 * boxes * 4 int32) it receives one entry per
+ * (tile in raster order, slot: left / right lens, box): {first staged byte of the box's rows, width in
+ * 16-byte units (0: nothing staged; -1 in every entry of a tile that is not described), byte offset of
+ * the box inside a frame group, first source row of its 16}.  No reference counterpart.
+ */
+int pb_debug_plan_boxes(const pb_plan *plan, int32_t *table, int64_t capacity, int32_t dims[3]);
+
 #ifdef __cplusplus
 }
 #endif

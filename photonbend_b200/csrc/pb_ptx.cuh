@@ -26,6 +26,14 @@ __device__ __forceinline__ void mbarrier_arrive_expect_tx(uint64_t* bar, uint32_
                  : "memory");
 }
 
+// a plain arrival (release: this thread's earlier shared-memory accesses are ordered before it)
+__device__ __forceinline__ void mbarrier_arrive(uint64_t* bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_addr(bar)) : "memory");
+}
+__device__ __forceinline__ void mbarrier_arrive_sa(uint32_t bar_sa) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar_sa) : "memory");
+}
+
 __device__ __forceinline__ bool mbarrier_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
     asm volatile(

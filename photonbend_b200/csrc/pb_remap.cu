@@ -20,6 +20,7 @@
 #include "pb_sep1.cuh"
 #include "pb_chunk.cuh"
 #include "pb_tiled2.cuh"
+#include "pb_boxes.cuh"
 #include "pb_wide.cuh"
 
 namespace pb {
@@ -949,6 +950,17 @@ static cudaError_t launch_two_lens(const TiledArgs& a, cudaStream_t st) {
     return cudaGetLastError();
 }
 
+// both tile classes of a batch through a double-fisheye source, staged box by box (pb_boxes.cuh)
+template <int CLS>
+static cudaError_t launch_boxes(const TiledArgs& a, cudaStream_t st) {
+    const int smem = boxes_smem_bytes(a.stage_bytes);
+    if (cudaError_t e = reserve_smem<remap_boxes_kernel<CLS>>(smem)) return e;
+    if (a.n_list <= 0) return cudaSuccess;
+    remap_boxes_kernel<CLS><<<a.n_list, BoxKernel<CLS>::kThreads, smem, st>>>(a);
+    PB_COUNT_LAUNCH();
+    return cudaGetLastError();
+}
+
 // tuning experiments
 static int env_int(const char* name, int fallback) {
     const char* e = std::getenv(name);
@@ -1024,6 +1036,7 @@ struct pb_plan {
     int* tile_lists;
     int n_one, n_rest;
     int4* sep1_cls;      // single-frame kernel: descriptor tables of the two classes ([n_one] then [n_rest][2])
+    int4* boxes;         // batches: per (tile, slot, box) extents of the staged footprints (pb_box_kernel); null: rectangles
     int sep1_cap_one;    // ... and the stage-buffer capacity of the one-lens class
     // the two grids of a double-fisheye remap are independent (disjoint tiles): the second one is
     // forked onto a stream of the plan's own and joined back, so that it fills the SMs the first
@@ -1104,6 +1117,7 @@ static void plan_init(pb_plan& p, const pb_remap_desc& d) {
     p.tile_lists = nullptr;
     p.n_one = p.n_rest = 0;
     p.sep1_cls = nullptr;
+    p.boxes = nullptr;
     p.sep1_cap_one = 24 * 1024;
     std::memset(p.lanes, 0, sizeof(p.lanes));
     p.n_lanes = p.next_lane = 0;
@@ -1259,6 +1273,18 @@ static void classify_tiles(pb_plan& p, const int4* fp, cudaStream_t st) {
     p.tile_lists = lists;
     p.n_rest = (int)rest.size();
     p.n_one = n_tiles - p.n_rest;
+    // batches: the extents of every 16-row box of the footprints (what pb_boxes.cuh stages); without
+    // them the batched kernels stage bounding rectangles
+    int4* boxes = nullptr;
+    if (cudaMalloc((void**)&boxes, sizeof(int4) * 2 * kMaxBoxes * (size_t)n_tiles) == cudaSuccess) {
+        pb_box_kernel<<<(n_tiles + 7) / 8, 256, 0, st>>>(tiled_args(p, p.tables), footprint_table(p, p.tables), boxes, tx,
+                                                        n_tiles);
+        PB_COUNT_LAUNCH();
+        if (cudaGetLastError() == cudaSuccess) p.boxes = boxes;
+        else cudaFree(boxes);
+    } else {
+        (void)cudaGetLastError();
+    }
     // single-frame kernel: per-class descriptor tables, and a buffer size that holds the one
     // rectangle of (all but 0.5 % of) the one-lens tiles
     int4* cls = nullptr;
@@ -1653,11 +1679,18 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
                 // rectangles (pb_chunk.cuh); PB_CHUNK: bit 0 = that class, bit 1 = the one-lens class too
                 const int chunk = env_int("PB_CHUNK", 0);
                 const int skip = env_int("PB_SKIP_CLASS", 0);  // timing experiments: leave one grid out (wrong output)
+                // each 16-row box staged at its own extents, a producer warp per CTA (pb_boxes.cuh);
+                // PB_BOX_EXTENTS=0: bounding rectangles issued by thread 0 (pb_tiled.cuh, pb_tiled2.cuh)
+                const bool boxed = p.boxes && env_int("PB_BOX_EXTENTS", 1) != 0;
+                a.tile_box = b.tile_box = p.boxes;
                 if (skip == 2) {
                     e = cudaSuccess;
                 } else if (chunk & 1) {
                     a.stage_bytes = env_int("PB_CHUNK_REST_KIB", 94) * 1024;
                     e = launch_chunk_one<PB_KIND_DOUBLE, 2>(a, lane ? lane->side : st);
+                } else if (boxed) {
+                    a.stage_bytes = 2 * a.stage_bytes;  // the ring of frame groups of remap_two_lens_kernel
+                    e = launch_boxes<2>(a, lane ? lane->side : st);
                 } else if (env_int("PB_CLS2_THREADS", 512) == 512) {
                     // 16 warps per CTA, one quad per thread: twice the warps per SM for the same shared memory
                     // (cfg5 x16: the class alone 0.321 -> 0.301 ms, the step 0.628 -> 0.612 ms)
@@ -1670,6 +1703,9 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
                     if (chunk & 2) {
                         b.stage_bytes = env_int("PB_CHUNK_ONE_KIB", 38) * 1024;
                         e = launch_chunk_one<PB_KIND_DOUBLE, 1>(b, st);
+                    } else if (boxed) {
+                        b.stage_bytes = 2 * b.stage_bytes + 128;  // the ring of the two stage buffers of remap_tiled_kernel
+                        e = launch_boxes<1>(b, st);
                     } else {
                         e = launch_tiled_one<PB_KIND_EQUIRECT, PB_KIND_DOUBLE, 1, 1>(b, st);
                     }
@@ -1967,6 +2003,21 @@ int pb_debug_plan_fast32(const pb_plan* plan, double out[2]) {
     return PB_OK;
 }
 
+int pb_debug_plan_boxes(const pb_plan* plan, int32_t* table, int64_t capacity, int32_t dims[3]) {
+    if (!plan || !dims) return fail(PB_ERR_INVALID_ARGUMENT, "pb_debug_plan_boxes: null pointer");
+    dims[0] = dims[1] = dims[2] = 0;
+    if (!plan->boxes) return PB_OK;
+    dims[0] = tiles_y(*plan);
+    dims[1] = tiles_x(*plan);
+    dims[2] = kMaxBoxes;
+    const int64_t n = (int64_t)dims[0] * dims[1] * 2 * kMaxBoxes * 4;
+    if (!table) return PB_OK;
+    if (capacity < n) return fail(PB_ERR_INVALID_ARGUMENT, "pb_debug_plan_boxes: table too small");
+    cudaError_t e = cudaMemcpy(table, plan->boxes, sizeof(int32_t) * n, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return cuda_fail(e, "pb_debug_plan_boxes");
+    return PB_OK;
+}
+
 int pb_plan_remap_u8(const pb_plan* plan, const uint8_t* src, int64_t src_frame_stride, uint8_t* dst,
                      int64_t dst_frame_stride, int32_t n_frames, void* stream) {
     return plan_remap("pb_plan_remap_u8", plan, 1, src, src_frame_stride, dst, dst_frame_stride, n_frames, stream);
@@ -1994,6 +2045,7 @@ void pb_plan_destroy(pb_plan* plan) {
     if (plan->luts) cudaFree(plan->luts);
     if (plan->tile_lists) cudaFree(plan->tile_lists);
     if (plan->sep1_cls) cudaFree(plan->sep1_cls);
+    if (plan->boxes) cudaFree(plan->boxes);
     for (int k = 0; k < plan->n_lanes; ++k) {
         cudaStreamDestroy(plan->lanes[k].side);
         cudaEventDestroy(plan->lanes[k].ev_fork);

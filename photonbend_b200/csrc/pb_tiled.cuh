@@ -90,6 +90,7 @@ struct TiledArgs {
     const int* tile_list;  // non-null: CTA b remaps tile tile_list[b] (a class of tiles, in raster order; n_list CTAs)
     int n_list;
     const int4* tile_fp;  // separable: per (tile, slot) footprint {by0, xb0, nbox, all_valid | need_bytes << 1}
+    const int4* tile_box; // separable double-fisheye plan: per (tile, slot, box) extents (pb_boxes.cuh)
     const int4* sep1_tab; // separable: the same per (tile in launch order, slot), pre-decoded (pb_sep1.cuh)
     const double* sep1_col;  // single-frame kernel: per-tile column / row table slices (pb_sep1_slices_kernel)
     const double* sep1_row;
