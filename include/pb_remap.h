@@ -109,6 +109,31 @@ const char *pb_last_error(void);
  * state how many of their own kernels ran inside a timed region. */
 int64_t pb_kernel_launches(void);
 
+/* Kernel families of pb_debug_launch_counts: which kernel a launch ran. */
+enum {
+    PB_LAUNCH_DIRECT = 0,     /* remap_direct_kernel: one frame, float64 tiers per pixel */
+    PB_LAUNCH_DIRECT32 = 1,   /* remap_direct32_kernel: one frame, FP32-first tier */
+    PB_LAUNCH_GENERIC = 2,    /* remap_generic_kernel: any layout, alignment or stride */
+    PB_LAUNCH_TILED = 3,      /* remap_tiled_kernel, generic rays (MODE 0) */
+    PB_LAUNCH_TILED_SEP = 4,  /* remap_tiled_kernel, separable tables (MODE 1), every tile class */
+    PB_LAUNCH_TWO_LENS = 5,   /* remap_two_lens_kernel */
+    PB_LAUNCH_BOXES1 = 6,     /* remap_boxes_kernel, one-lens tiles */
+    PB_LAUNCH_BOXES2 = 7,     /* remap_boxes_kernel, two-lens and blend-band tiles */
+    PB_LAUNCH_SEP1 = 8,       /* remap_sep1_kernel: one frame, separable */
+    PB_LAUNCH_CHUNK = 9,      /* remap_chunk_kernel */
+    PB_LAUNCH_WIDE = 10,      /* remap_wide_kernel: elements wider than a byte */
+    PB_LAUNCH_GATHER = 11,    /* gather_from_map_kernel: explicit maps */
+    PB_LAUNCH_PLAN = 12,      /* plan-time kernels: tables, footprints, boxes, census, calibration */
+    PB_LAUNCH_MAP = 13,       /* coordinate-map kernels: materialise, rotate, map_projection */
+    PB_LAUNCH_DIAGNOSTIC = 14, /* pb_debug_fast32_stats */
+    PB_LAUNCH_FAMILIES = 15
+};
+
+/* Kernels launched per family since the process started, for tests that must know which kernel
+ * a call ran.  Fills counts[0 .. min(capacity, PB_LAUNCH_FAMILIES)) (nothing when counts is NULL)
+ * and returns PB_LAUNCH_FAMILIES.  The families add up to pb_kernel_launches(). */
+int pb_debug_launch_counts(int64_t *counts, int32_t capacity);
+
 /* Width of the image a geometry produces: 2*(width/2) for PB_KIND_DOUBLE (projection.py:389-397),
  * width otherwise. */
 int32_t pb_output_width(const pb_image_desc *out);

@@ -25,11 +25,16 @@ PB_ERR_UNSUPPORTED = 2
 PB_ERR_CUDA = 3
 PB_ERR_TOO_MANY_ROTATIONS = 4
 
+# kernel families of pb_debug_launch_counts, in the order of the PB_LAUNCH_* enum
+LAUNCH_FAMILIES = ("direct", "direct32", "generic", "tiled", "tiled_sep", "two_lens", "boxes1", "boxes2", "sep1",
+                   "chunk", "wide", "gather", "plan", "map", "diagnostic")
+
 # every symbol include/pb_remap.h declares
 EXPORTS = (
     "pb_version",
     "pb_last_error",
     "pb_kernel_launches",
+    "pb_debug_launch_counts",
     "pb_output_width",
     "pb_remap_u8",
     "pb_plan_create",
@@ -103,6 +108,8 @@ def load():
     lib.pb_last_error.argtypes = []
     lib.pb_kernel_launches.restype = ctypes.c_int64
     lib.pb_kernel_launches.argtypes = []
+    lib.pb_debug_launch_counts.restype = ctypes.c_int
+    lib.pb_debug_launch_counts.argtypes = [ctypes.POINTER(ctypes.c_int64), i32]
     lib.pb_output_width.restype = i32
     lib.pb_output_width.argtypes = [ctypes.POINTER(ImageDesc)]
     lib.pb_remap_u8.restype = ctypes.c_int
@@ -137,6 +144,16 @@ def load():
     lib.pb_gather_from_map_px.argtypes = [ctypes.POINTER(ImageDesc), i32, i32, vp, i32, i32, vp, vp, vp]
     _lib = lib
     return lib
+
+
+def launch_counts() -> dict:
+    """Kernels launched per family (LAUNCH_FAMILIES) since the process started."""
+    lib = load()
+    counts = (ctypes.c_int64 * len(LAUNCH_FAMILIES))()
+    n = lib.pb_debug_launch_counts(counts, len(LAUNCH_FAMILIES))
+    if n != len(LAUNCH_FAMILIES):
+        raise RuntimeError(f"libpbremap counts {n} kernel families, this binding knows {len(LAUNCH_FAMILIES)}")
+    return dict(zip(LAUNCH_FAMILIES, counts))
 
 
 def check(code: int) -> None:

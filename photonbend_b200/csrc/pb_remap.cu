@@ -28,9 +28,15 @@ namespace pb {
 // ------------------------------------------------------------------------------------ errors
 
 static thread_local std::string g_last_error;
-// kernels this library has launched in this process (pb_kernel_launches)
+// kernels this library has launched in this process (pb_kernel_launches), in total and by family
+// (PB_LAUNCH_*, pb_debug_launch_counts)
 static std::atomic<long long> g_kernel_launches{0};
-#define PB_COUNT_LAUNCH() g_kernel_launches.fetch_add(1, std::memory_order_relaxed)
+static std::atomic<long long> g_family_launches[PB_LAUNCH_FAMILIES];
+#define PB_COUNT_LAUNCH(family)                                                        \
+    do {                                                                               \
+        g_kernel_launches.fetch_add(1, std::memory_order_relaxed);                     \
+        g_family_launches[(family)].fetch_add(1, std::memory_order_relaxed);           \
+    } while (0)
 
 static int fail(int code, const std::string& msg) {
     g_last_error = msg;
@@ -806,10 +812,11 @@ static void launch_direct(const RemapArgs& a, cudaStream_t st) {
         with_kind(a.out.kind, [&](auto o) {
             with_single_kind(a.src.kind, [&](auto s) { remap_direct32_kernel<o, s><<<grid, 256, 0, st>>>(a); });
         });
+        PB_COUNT_LAUNCH(PB_LAUNCH_DIRECT32);
     } else {
         with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) { remap_direct_kernel<o, s><<<grid, 256, 0, st>>>(a); });
+        PB_COUNT_LAUNCH(PB_LAUNCH_DIRECT);
     }
-    PB_COUNT_LAUNCH();
 }
 
 static void launch_generic(const RemapArgs& a, cudaStream_t st) {
@@ -818,7 +825,7 @@ static void launch_generic(const RemapArgs& a, cudaStream_t st) {
     with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
         with_channels(a.src.C, [&](auto c) { remap_generic_kernel<o, s, c><<<grid, block, 0, st>>>(a); });
     });
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_GENERIC);
 }
 
 // explicit-map gather: uint8 elements from any source, or elements of 2, 4 or 8 bytes from a
@@ -838,7 +845,7 @@ static void launch_gather(const SrcGeom& s, int elem_bytes, double* map, long lo
         with_kind(s.kind, [&](auto k) { gather(k, (unsigned char)0); });
     else
         with_single_kind(s.kind, [&](auto k) { with_elem(elem_bytes, [&](auto t) { gather(k, t); }); });
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_GATHER);
 }
 
 // The widest word (a power of two, at most 16 bytes) that divides the pixel size and every address
@@ -916,7 +923,8 @@ static cudaError_t launch_tiled_one(const TiledArgs& a, cudaStream_t st) {
     const int grid = a.tile_list ? a.n_list : a.tiles_x * a.tiles_y;
     if (grid <= 0) return cudaSuccess;
     remap_tiled_kernel<OUT_KIND, SRC_KIND, MODE, CLS><<<grid, kTileThreads, smem, st>>>(a);
-    PB_COUNT_LAUNCH();
+    // (a probe launch remaps nothing: it is the footprint census of pb_plan_create)
+    PB_COUNT_LAUNCH(a.probe ? PB_LAUNCH_PLAN : MODE == 1 ? PB_LAUNCH_TILED_SEP : PB_LAUNCH_TILED);
     return cudaGetLastError();
 }
 
@@ -936,7 +944,7 @@ static cudaError_t launch_chunk_one(const TiledArgs& a, cudaStream_t st) {
     const int grid = a.tile_list ? a.n_list : a.tiles_x * a.tiles_y;
     if (grid <= 0) return cudaSuccess;
     remap_chunk_kernel<SRC_KIND, CLS><<<grid, kTileThreads, smem, st>>>(a);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_CHUNK);
     return cudaGetLastError();
 }
 
@@ -946,7 +954,7 @@ static cudaError_t launch_two_lens(const TiledArgs& a, cudaStream_t st) {
     if (cudaError_t e = reserve_smem<remap_two_lens_kernel>(smem)) return e;
     if (a.n_list <= 0) return cudaSuccess;
     remap_two_lens_kernel<<<a.n_list, kTile2Threads, smem, st>>>(a);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_TWO_LENS);
     return cudaGetLastError();
 }
 
@@ -957,7 +965,7 @@ static cudaError_t launch_boxes(const TiledArgs& a, cudaStream_t st) {
     if (cudaError_t e = reserve_smem<remap_boxes_kernel<CLS>>(smem)) return e;
     if (a.n_list <= 0) return cudaSuccess;
     remap_boxes_kernel<CLS><<<a.n_list, BoxKernel<CLS>::kThreads, smem, st>>>(a);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(CLS == 1 ? PB_LAUNCH_BOXES1 : PB_LAUNCH_BOXES2);
     return cudaGetLastError();
 }
 
@@ -1007,7 +1015,7 @@ static cudaError_t launch_sep1_one(const TiledArgs& a, cudaStream_t st) {
     cfg.attrs = &attr;
     cfg.numAttrs = pdl ? 1 : 0;
     e = cudaLaunchKernelEx(&cfg, remap_sep1_kernel<SRC_KIND, NB, CLS>, a);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_SEP1);
     return e;
 }
 
@@ -1279,7 +1287,7 @@ static void classify_tiles(pb_plan& p, const int4* fp, cudaStream_t st) {
     if (cudaMalloc((void**)&boxes, sizeof(int4) * 2 * kMaxBoxes * (size_t)n_tiles) == cudaSuccess) {
         pb_box_kernel<<<(n_tiles + 7) / 8, 256, 0, st>>>(tiled_args(p, p.tables), footprint_table(p, p.tables), boxes, tx,
                                                         n_tiles);
-        PB_COUNT_LAUNCH();
+        PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
         if (cudaGetLastError() == cudaSuccess) p.boxes = boxes;
         else cudaFree(boxes);
     } else {
@@ -1295,12 +1303,12 @@ static void classify_tiles(pb_plan& p, const int4* fp, cudaStream_t st) {
     if (p.n_one > 0) {
         pb_sep1_table_kernel<<<(p.n_one + 255) / 256, 256, 0, st>>>(footprint_table(p, p.tables), cls, tx, ty, p.raster_band,
                                                                    2, lists, p.n_one, 1);
-        PB_COUNT_LAUNCH();
+        PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     }
     if (p.n_rest > 0) {
         pb_sep1_table_kernel<<<(p.n_rest + 255) / 256, 256, 0, st>>>(footprint_table(p, p.tables), cls + p.n_one, tx, ty,
                                                                     p.raster_band, 2, lists + p.n_one, p.n_rest, 0);
-        PB_COUNT_LAUNCH();
+        PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     }
     if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) {
         (void)cudaGetLastError();
@@ -1513,14 +1521,14 @@ static void tune_stage(pb_plan& p, cudaStream_t st) {
 static cudaError_t fill_tables(const pb_plan& p, double* tables, cudaStream_t st) {
     const int n = p.out.W > p.out.H ? p.out.W : p.out.H;
     pb_tables_kernel<<<(n + 255) / 256, 256, 0, st>>>(p.out, p.src, tables, tables + 2 * (size_t)p.out.W);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int n_entries = footprint_entries(p);
     pb_footprint_kernel<<<(n_entries + 7) / 8, 256, 0, st>>>(tiled_args(p, tables),
                                                            const_cast<int4*>(footprint_table(p, tables)), tiles_x(p),
                                                            n_entries);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int n_tiles = tiles_x(p) * tiles_y(p);
@@ -1532,7 +1540,7 @@ static cudaError_t fill_tables(const pb_plan& p, double* tables, cudaStream_t st
                                                               const_cast<int4*>(sep1_table(p, tables)), tiles_x(p),
                                                               tiles_y(p), p.src.kind == PB_KIND_CAMERA ? sep1_band : p.raster_band,
                                                               p.src.kind == PB_KIND_DOUBLE ? 2 : 1);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int n_slice = std::max(tiles_x(p) * kTileW, tiles_y(p) * kTileH);
@@ -1540,7 +1548,7 @@ static cudaError_t fill_tables(const pb_plan& p, double* tables, cudaStream_t st
                                                                const_cast<double*>(sep1_col(p, tables)),
                                                                const_cast<double*>(sep1_row(p, tables)), p.out.W, p.out.H,
                                                                tiles_x(p), tiles_y(p), (int)sep1_row_doubles(p));
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     return cudaGetLastError();
 }
 
@@ -1768,7 +1776,7 @@ static int plan_run_wide(const pb_plan& p, int elem_bytes, const void* src, int6
             });
         }
     });
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_WIDE);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "wide remap launch");
     return PB_OK;
@@ -1874,6 +1882,12 @@ int pb_version(void) { return PB_ABI_VERSION; }
 
 int64_t pb_kernel_launches(void) { return (int64_t)g_kernel_launches.load(std::memory_order_relaxed); }
 
+int pb_debug_launch_counts(int64_t* counts, int32_t capacity) {
+    for (int k = 0; counts && k < capacity && k < PB_LAUNCH_FAMILIES; ++k)
+        counts[k] = (int64_t)g_family_launches[k].load(std::memory_order_relaxed);
+    return PB_LAUNCH_FAMILIES;
+}
+
 const char* pb_last_error(void) { return g_last_error.c_str(); }
 
 int32_t pb_output_width(const pb_image_desc* out) {
@@ -1940,7 +1954,7 @@ static void calibrate_fast32(pb_plan& p, cudaStream_t st) {
     with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
         fast32_ratio_kernel<o, s><<<grid, block, 0, st>>>(a, gd, dev);
     });
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_PLAN);
     unsigned bits = 0;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(&bits, dev, sizeof(bits), cudaMemcpyDeviceToHost, st);
@@ -2071,7 +2085,7 @@ int pb_materialize_map_f64(const pb_remap_desc* desc, double* map, void* stream)
     if (cudaError_t eu = upload_lens_tables(&desc->out, &g, nullptr, nullptr, &luts, st, true))
         return cuda_fail(eu, "pb_materialize_map_f64 lens table");
     with_kind(g.kind, [&](auto k) { materialize_map_kernel<k><<<grid, block, 0, st>>>(g, rot, map); });
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_MAP);
     cudaError_t e = cudaGetLastError();
     if (luts) cudaFreeAsync(luts, st);
     if (e != cudaSuccess) return cuda_fail(e, "pb_materialize_map_f64 launch");
@@ -2093,9 +2107,9 @@ int pb_map_projection_u8(double* map, int32_t map_height, int32_t map_width, uin
     if (e == cudaSuccess) {
         const unsigned blocks = (unsigned)std::min<long long>((n + 255) / 256, 148 * 16);
         map_range_kernel<<<blocks, 256, 0, st>>>(map, n, range);
-        PB_COUNT_LAUNCH();
+        PB_COUNT_LAUNCH(PB_LAUNCH_MAP);
         map_projection_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(map, n, range, dst);
-        PB_COUNT_LAUNCH();
+        PB_COUNT_LAUNCH(PB_LAUNCH_MAP);
         e = cudaGetLastError();
     }
     cudaFreeAsync(range, st);
@@ -2121,7 +2135,7 @@ int pb_debug_fast32_stats(const pb_remap_desc* desc, double stats[6], void* stre
     with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
         fast32_stats_kernel<o, s><<<grid, block, 0, st>>>(a, gd, maxima, dev);
     });
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_DIAGNOSTIC);
     unsigned long long host[8];
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(host, dev, sizeof(host), cudaMemcpyDeviceToHost, st);
@@ -2147,7 +2161,7 @@ int pb_rotate_map_f64(const double matrix[9], double* map_in, double* map_out, i
     const long long blocks = (n_pixels + block - 1) / block;
     if (blocks > 0x7fffffffLL) return fail(PB_ERR_UNSUPPORTED, "pb_rotate_map_f64: map too large");
     rotate_map_kernel<<<(unsigned)blocks, block, 0, (cudaStream_t)stream>>>(m, map_in, map_out, n_pixels);
-    PB_COUNT_LAUNCH();
+    PB_COUNT_LAUNCH(PB_LAUNCH_MAP);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "pb_rotate_map_f64 launch");
     return PB_OK;

@@ -34,6 +34,17 @@ def product_remap(out_geom: dict, rotations, src_geom: dict, image):
     return product_image(src_geom, image).process_coordinate_map(product_map(out_geom, rotations))
 
 
+def remap_launches(fn):
+    """Run fn() -> (its result, {kernel family: grids launched}) for the kernels the library launched
+    during the call (pb_debug_launch_counts), without the plan-time kernels of a first call."""
+    from photonbend_b200 import _native
+
+    before = _native.launch_counts()
+    result = fn()
+    after = _native.launch_counts()
+    return result, {k: after[k] - before[k] for k in after if k != "plan" and after[k] != before[k]}
+
+
 def attribute_mismatches(got, want, image, idx):
     """Classify the pixels where ``got`` != ``want``.
 

@@ -41,6 +41,25 @@ def test_struct_layout_matches_header():
     assert _native.RemapDesc.rotations.offset == 120
 
 
+def test_launch_families_match_header():
+    """pb_debug_launch_counts: the PB_LAUNCH_* enum and _native.LAUNCH_FAMILIES name the same
+    families in the same order, and the families add up to pb_kernel_launches()."""
+    from photonbend_b200 import _native
+
+    with open(os.path.join(REPO, "include", "pb_remap.h")) as fh:
+        text = re.sub(r"/\*.*?\*/", "", fh.read(), flags=re.S)
+    values = {name: int(v) for name, v in re.findall(r"\bPB_LAUNCH_([A-Z0-9_]+)\s*=\s*(\d+)", text)}
+    n = values.pop("FAMILIES")
+    assert sorted(values.values()) == list(range(n))
+    assert tuple(name.lower() for name in sorted(values, key=values.get)) == _native.LAUNCH_FAMILIES
+    lib = _native.load()
+    assert lib.pb_debug_launch_counts(None, 0) == n
+    short = (ctypes.c_int64 * 2)(-1, -1)
+    assert lib.pb_debug_launch_counts(short, 1) == n and short[1] == -1  # writes no more than capacity
+    counts = _native.launch_counts()
+    assert min(counts.values()) >= 0 and sum(counts.values()) == lib.pb_kernel_launches()
+
+
 def test_argument_errors_need_no_gpu():
     from photonbend_b200 import _native
 

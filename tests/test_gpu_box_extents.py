@@ -123,9 +123,11 @@ def test_boxes_remap_like_rectangles(torch_cuda, name, og, sg, monkeypatch):
     frames = torch.from_numpy(np.stack(flat + noise + [ramp, case_matrix.case_image(sg, 77)])).cuda()
     assert frames.shape[0] == 16
     outs = {}
-    for switch in ("1", "0"):
+    for switch, families in (("1", {"boxes1", "boxes2"}), ("0", {"tiled_sep", "two_lens"})):
         monkeypatch.setenv("PB_BOX_EXTENTS", switch)
-        outs[switch] = helpers.product_image(sg, frames).process_coordinate_map(helpers.product_map(og, ())).cpu().numpy()
+        outs[switch], ran = helpers.remap_launches(
+            lambda: helpers.product_image(sg, frames).process_coordinate_map(helpers.product_map(og, ())).cpu().numpy())
+        assert ran and set(ran) <= families, (switch, ran)  # the box kernels, and without them the rectangle kernels
     for k in range(16):
         assert np.array_equal(outs["1"][k], outs["0"][k]), (name, k, mismatch_report(outs["1"][k], outs["0"][k]))
     if h <= 800:  # and against the oracle, where that is quick

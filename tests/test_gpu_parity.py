@@ -345,11 +345,29 @@ def test_double_source_batches_blend_band(torch_cuda, fov_deg, monkeypatch):
     ])
     want = [numpy_port.remap(og, (), sg, f) for f in frames]
     dev = torch.from_numpy(frames).cuda()
-    for env in ({}, {"PB_ONE_BYTES": "4096", "PB_REST_KIB": "8"}, {"PB_CLASS_SPLIT": "0"}, {"PB_CLS2_THREADS": "256"},
-                {"PB_CHUNK": "3"}):
+    # (switch, the kernels it runs): PB_BOX_EXTENTS=0 leads to remap_two_lens_kernel and, with
+    # PB_CLS2_THREADS=256, to the 256-thread class-2 remap_tiled_kernel; the one-lens class (CLS 1)
+    # then runs remap_tiled_kernel; either class may be empty
+    classes = None
+    for env, families in (({}, ("boxes1", "boxes2")), ({"PB_ONE_BYTES": "4096", "PB_REST_KIB": "8"}, ("boxes1", "boxes2")),
+                          ({"PB_CLASS_SPLIT": "0"}, ("tiled_sep", "tiled_sep")),
+                          ({"PB_CLS2_THREADS": "256", "PB_BOX_EXTENTS": "0"}, ("tiled_sep", "tiled_sep")),
+                          ({"PB_BOX_EXTENTS": "0"}, ("tiled_sep", "two_lens")), ({"PB_CHUNK": "3"}, ("chunk", "chunk"))):
         for k, v in env.items():
             monkeypatch.setenv(k, v)
-        out = helpers.product_image(sg, dev).process_coordinate_map(helpers.product_map(og, ())).cpu().numpy()
+        out, ran = helpers.remap_launches(
+            lambda: helpers.product_image(sg, dev).process_coordinate_map(helpers.product_map(og, ())).cpu().numpy())
+        if classes is None:  # the default run: which tile classes (one-lens, two-lens) have tiles
+            classes = ("boxes1" in ran, "boxes2" in ran)
+            assert any(classes) and set(ran) <= {"boxes1", "boxes2"}, ran
+        if env == {"PB_CLASS_SPLIT": "0"}:
+            assert ran == {"tiled_sep": 1}, ran
+        else:
+            expected = {}
+            for present, family in zip(classes, families):
+                if present:
+                    expected[family] = expected.get(family, 0) + 1
+            assert ran == expected, (env, ran, expected)
         for k in range(len(frames)):
             assert np.array_equal(out[k], want[k]), (fov_deg, env, k, mismatch_report(out[k], want[k]))
         for k in env:
@@ -928,10 +946,11 @@ def _random_geometry(rng, role):
 
 @pytest.mark.parametrize("fuzz_seed", [20261018, 7, 990])
 def test_random_mid_size_geometries(torch_cuda, fuzz_seed):
-    """Seeded fuzz (three seeds): 60 random (output, rotations, source) triples at sizes of several tiles -- every
-    kernel family gets some (separable batches and single frames when un-rotated, the FP32-first
-    rotated kernel, two-lens tiles, explicit maps for > 8 rotations never) -- against
-    oracle/numpy_port.py (bit-identical to the reference).  Same acceptance as the small matrix."""
+    """Seeded fuzz (three seeds): 60 random (output, rotations, source) triples at sizes of several tiles
+    against oracle/numpy_port.py (bit-identical to the reference).  Same acceptance as the small matrix.
+    Widths are rarely 16-byte aligned, so batches run remap_generic_kernel and single frames the
+    direct and single-frame separable kernels; the staged batch kernels are fuzzed by
+    tests/test_gpu_staged_batches.py::test_random_aligned_batches."""
     torch = torch_cuda
     from oracle import c_port, numpy_port
 
