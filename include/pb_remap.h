@@ -126,7 +126,8 @@ enum {
     PB_LAUNCH_PLAN = 12,      /* plan-time kernels: tables, footprints, boxes, census, calibration */
     PB_LAUNCH_MAP = 13,       /* coordinate-map kernels: materialise, rotate, map_projection */
     PB_LAUNCH_DIAGNOSTIC = 14, /* pb_debug_fast32_stats */
-    PB_LAUNCH_FAMILIES = 15
+    PB_LAUNCH_FRAMES = 15,    /* remap_frames_kernel: a rotation per frame (pb_plan_remap_frames_px) */
+    PB_LAUNCH_FAMILIES = 16
 };
 
 /* Kernels launched per family since the process started, for tests that must know which kernel
@@ -186,6 +187,21 @@ int pb_plan_remap_px(const pb_plan *plan, int32_t elem_bytes, const void *src, i
                      void *dst, int64_t dst_frame_stride, int32_t n_frames, void *stream);
 int pb_plan_remap_rows_px(const pb_plan *plan, int32_t elem_bytes, const void *src, void *dst_band,
                           int32_t row_begin, int32_t row_end, void *stream);
+/*
+ * A batch whose frames each have a rotation of their own (stabilised or levelled 360-degree video, a
+ * virtual camera moving through a panorama): frame k of the batch is remapped as if desc->rotations
+ * had frame_rotations[k] (row-major 3x3, HOST memory, n_frames x 9 doubles, read during the call)
+ * appended as its last rotation -- byte-identical to pb_plan_remap_px through a plan of that
+ * descriptor.  Strides, element widths and their errors as pb_plan_remap_px (elem_bytes == 1 is
+ * uint8); a source stride of 0 gives n_frames views of one image.  desc->n_rotations + 1 >
+ * PB_MAX_ROTATIONS -> PB_ERR_TOO_MANY_ROTATIONS before any device work.  A frame whose matrix is not
+ * orthonormal or not finite takes the exact float64 chain, as a plan of it would.  Kernel launches
+ * only (one per 128 frames): no allocation, no synchronisation, so the call can be captured into a
+ * CUDA graph.
+ */
+int pb_plan_remap_frames_px(const pb_plan *plan, int32_t elem_bytes, const double *frame_rotations,
+                            const void *src, int64_t src_frame_stride, void *dst, int64_t dst_frame_stride,
+                            int32_t n_frames, void *stream);
 void pb_plan_destroy(pb_plan *plan);
 
 /*

@@ -27,7 +27,7 @@ PB_ERR_TOO_MANY_ROTATIONS = 4
 
 # kernel families of pb_debug_launch_counts, in the order of the PB_LAUNCH_* enum
 LAUNCH_FAMILIES = ("direct", "direct32", "generic", "tiled", "tiled_sep", "two_lens", "boxes1", "boxes2", "sep1",
-                   "chunk", "wide", "gather", "plan", "map", "diagnostic")
+                   "chunk", "wide", "gather", "plan", "map", "diagnostic", "frames")
 
 # every symbol include/pb_remap.h declares
 EXPORTS = (
@@ -51,6 +51,7 @@ EXPORTS = (
     "pb_plan_remap_px",
     "pb_plan_remap_rows_px",
     "pb_gather_from_map_px",
+    "pb_plan_remap_frames_px",
 )
 
 
@@ -142,6 +143,8 @@ def load():
     lib.pb_plan_remap_rows_px.argtypes = [vp, i32, vp, vp, i32, i32, vp]
     lib.pb_gather_from_map_px.restype = ctypes.c_int
     lib.pb_gather_from_map_px.argtypes = [ctypes.POINTER(ImageDesc), i32, i32, vp, i32, i32, vp, vp, vp]
+    lib.pb_plan_remap_frames_px.restype = ctypes.c_int
+    lib.pb_plan_remap_frames_px.argtypes = [vp, i32, ctypes.POINTER(ctypes.c_double), vp, i64, vp, i64, i32, vp]
     _lib = lib
     return lib
 

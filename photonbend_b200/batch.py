@@ -70,16 +70,23 @@ def max_over_ranks(values, device="cpu"):
     return [float(v) for v in t.cpu()]
 
 
-def remap_batch(source, coordinate_map: CoordinateMap, frames, out=None):
+def remap_batch(source, coordinate_map: CoordinateMap, frames, out=None, frame_rotations=None):
     """Remap a device batch ``frames`` (CUDA tensor (N, H, W, C) of any dtype the remap takes, see
     ``engine.ELEM_BYTES``) that shares the geometry
     of ``source`` (a CameraImage / DoubleCameraImage / PanoramaImage whose own ``image`` is only
     used for its shape) along ``coordinate_map``.  One kernel launch; returns the (N, Ho, Wo, C)
-    CUDA tensor of the same dtype."""
+    CUDA tensor of the same dtype.
+
+    ``frame_rotations`` (N ``Rotation`` objects or an (N, 3, 3) array): frame k is remapped as if
+    ``frame_rotations[k]`` had been applied to ``coordinate_map`` after its own rotations
+    (stabilised or levelled video, a moving virtual camera)."""
     if not (isinstance(coordinate_map, CoordinateMap) and coordinate_map.is_lazy):
         raise ValueError("remap_batch needs the lazy CoordinateMap of get_coordinate_map()")
     if frames.dim() != 4 or not frames.is_cuda:
         raise ValueError("frames must be a CUDA tensor of shape (N, H, W, C)")
+    if frame_rotations is not None:
+        return engine.remap_frames_device(coordinate_map.rays, source._source_geometry(), frames.contiguous(),
+                                          frame_rotations, out)
     return engine.remap_device(coordinate_map.rays, source._source_geometry(), frames.contiguous(), out)
 
 
@@ -97,6 +104,11 @@ class FramePipeline:
 
     A host output buffer is complete after ``drain()`` or after the event its ``submit`` /
     ``flush`` returned; it must not be handed to another ``submit`` before that.
+
+    ``submit(..., rotation=R)`` remaps that frame as if ``R`` had been applied after the map's own
+    rotations (see ``remap_batch``'s ``frame_rotations``).  A pipeline takes a rotation with every
+    frame or with none: an identity rotation is not bit-identical to no rotation (it sends each
+    ray through acos / atan2 once more), so mixing the two would silently change some frames.
     """
 
     def __init__(self, source, coordinate_map: CoordinateMap, depth: int = 3, device: Optional[int] = None,
@@ -114,6 +126,8 @@ class FramePipeline:
         self._src_bufs: List = [None] * self._depth
         self._dst_bufs: List = [None] * self._depth
         self._pending: List[list] = [[] for _ in range(self._depth)]  # host outputs of the frames a slot holds
+        self._rotations: List[list] = [[] for _ in range(self._depth)]  # their rotations (pipelines that take them)
+        self._rotated: Optional[bool] = None  # fixed by the first submit
         self._slot = 0
         self.kernel_launches = 0
 
@@ -136,7 +150,9 @@ class FramePipeline:
                 self._dst_bufs[slot] = torch.empty((self._batch, oh, ow) + tuple(src_dev.shape[3:]), dtype=src_dev.dtype,
                                                    device=self._device)
             dst_dev = self._dst_bufs[slot]
-            if n == 1:  # one frame: the single-frame kernels
+            if self._rotated:
+                engine.remap_frames_device(self._rays, self._src_geom, src_dev[:n], self._rotations[slot], dst_dev[:n])
+            elif n == 1:  # one frame: the single-frame kernels
                 engine.remap_device(self._rays, self._src_geom, src_dev[0], dst_dev[0])
             else:
                 engine.remap_device(self._rays, self._src_geom, src_dev[:n], dst_dev[:n])
@@ -146,12 +162,21 @@ class FramePipeline:
             done = torch.cuda.Event()
             done.record(stream)
         self._pending[slot] = []
+        self._rotations[slot] = []
         return done
 
-    def submit(self, host_frame, host_out):
+    def submit(self, host_frame, host_out, rotation=None):
         """Enqueue one frame: host_frame (CPU tensor (H, W, C) of any dtype the remap takes) ->
-        host_out (CPU tensor (Ho, Wo, C) of the same dtype).  Returns immediately: the completion event of the launch when this
+        host_out (CPU tensor (Ho, Wo, C) of the same dtype), through ``rotation`` (a ``Rotation`` or
+        a 3x3 matrix) after the map's rotations when given.  Returns immediately: the completion event of the launch when this
         frame completed a batch, else None."""
+        rotated = rotation is not None
+        if self._rotated is None:
+            self._rotated = rotated
+        elif rotated != self._rotated:
+            raise ValueError("a FramePipeline takes a rotation with every frame or with none")
+        if rotated:
+            rotation = engine.frame_matrices([rotation])[0].reshape(3, 3)
         torch = self._torch
         slot = self._slot
         stream = self._streams[slot]
@@ -164,6 +189,8 @@ class FramePipeline:
                 self._dst_bufs[slot] = None
             self._src_bufs[slot][len(self._pending[slot])].copy_(host_frame, non_blocking=True)
         self._pending[slot].append(host_out)
+        if rotated:
+            self._rotations[slot].append(rotation)
         if len(self._pending[slot]) < self._batch:
             return None
         self._slot = (slot + 1) % self._depth

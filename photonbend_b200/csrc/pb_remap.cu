@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <string>
@@ -22,6 +23,7 @@
 #include "pb_tiled2.cuh"
 #include "pb_boxes.cuh"
 #include "pb_wide.cuh"
+#include "pb_frames.cuh"
 
 namespace pb {
 
@@ -1782,6 +1784,66 @@ static int plan_run_wide(const pb_plan& p, int elem_bytes, const void* src, int6
     return PB_OK;
 }
 
+// A batch with a rotation per frame (pb_frames.cuh): frame k as the plan of the descriptor with
+// frame_rotations[k] appended to its rotations.  The constants are what pb_plan_create derives for
+// that descriptor, less the plan's calibration of the FP32-first tier (K = 16, the bound that holds
+// for every geometry).  Launches of up to kFramesPerLaunch frames; nothing allocated, nothing awaited
+// (the plan's state is only read: no lock needed).
+static int plan_run_frames(const pb_plan& p, int elem_bytes, const double* frame_rotations, const void* src,
+                           int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames,
+                           cudaStream_t st) {
+    const long long tiles_y = (p.out.H + kTileH - 1) / kTileH;
+    if (tiles_y >= 65536) return fail(PB_ERR_UNSUPPORTED, "frames remap: more than 65535 x 64 output rows");
+    const int n = p.desc.n_rotations;
+    double rotations[PB_MAX_ROTATIONS][9];
+    std::memcpy(rotations, p.desc.rotations, sizeof(rotations));
+    // (~27 KB, the kernel's parameter block: off the stack of the caller's thread)
+    std::unique_ptr<FramesArgs> args(new (std::nothrow) FramesArgs);
+    if (!args) return fail(PB_ERR_INVALID_ARGUMENT, "frames remap: out of host memory");
+    FramesArgs& a = *args;
+    std::memset(&a, 0, sizeof(a));
+    a.out = p.out;
+    a.src = p.src;
+    a.rot.n = n + 1;
+    std::memcpy(a.rot.m, p.rot.m, sizeof(a.rot.m));
+    a.src_frame_stride = src_frame_stride;
+    a.dst_frame_stride = dst_frame_stride;
+    a.px_bytes = p.desc.channels * elem_bytes;
+    // wide_vec's words are at least 2 bytes: uint8 pixels of odd size or at odd addresses move bytewise
+    const bool multi = n_frames > 1;
+    const unsigned long long odd = (unsigned long long)a.px_bytes | reinterpret_cast<uintptr_t>(src) |
+                                   reinterpret_cast<uintptr_t>(dst) |
+                                   (multi ? (unsigned long long)(src_frame_stride | dst_frame_stride) : 0ull);
+    a.vec = (odd & 1) ? 1 : wide_vec(a.px_bytes, src, dst, src_frame_stride, dst_frame_stride, multi);
+    a.words = a.px_bytes / a.vec;
+    for (int f0 = 0; f0 < n_frames; f0 += kFramesPerLaunch) {
+        const int nf = std::min(kFramesPerLaunch, n_frames - f0);
+        for (int k = 0; k < nf; ++k) {
+            std::memcpy(rotations[n], frame_rotations + 9 * (size_t)(f0 + k), sizeof(rotations[n]));
+            const FastGeom g = derive_fast(p.desc.out, p.out, p.desc.src, p.src, n + 1, rotations);
+            const Fast32Geom g32 = fast32_to_float(derive_fast32(p.out, p.src, g));
+            if (f0 + k == 0) {  // everything but the per-frame fields is the same for every frame
+                a.fast = g;
+                a.fast.f32 = g32;
+            }
+            FrameRotation& fr = a.frame[k];
+            std::memcpy(fr.rot, g.rot, sizeof(fr.rot));
+            std::memcpy(fr.last, rotations[n], sizeof(fr.last));
+            std::memcpy(fr.rot32, g32.rot, sizeof(fr.rot32));
+            fr.enabled = g.enabled;
+            fr.enabled32 = g32.enabled;
+        }
+        a.src_px = static_cast<const unsigned char*>(src) + f0 * src_frame_stride;
+        a.dst_px = static_cast<unsigned char*>(dst) + f0 * dst_frame_stride;
+        const dim3 grid((p.out.W + kTileW - 1) / kTileW, (unsigned)tiles_y, nf);
+        with_kinds(p.out.kind, p.src.kind, [&](auto o, auto s) { remap_frames_kernel<o, s><<<grid, 256, 0, st>>>(a); });
+        PB_COUNT_LAUNCH(PB_LAUNCH_FRAMES);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return cuda_fail(e, "frames remap launch");
+    }
+    return PB_OK;
+}
+
 // Arguments of the entry points that need no device: the element width, then for elements wider
 // than a byte the source kind, and pointers and strides against the width.  -> PB_OK, or the code
 // with pb_last_error set.
@@ -1826,6 +1888,23 @@ static int plan_remap(const char* who, const pb_plan* plan, int32_t elem_bytes, 
                              (cudaStream_t)stream);
     return plan_run(*const_cast<pb_plan*>(plan), plan->tables, static_cast<const uint8_t*>(src), src_frame_stride,
                     static_cast<uint8_t*>(dst), dst_frame_stride, n_frames, (cudaStream_t)stream);
+}
+
+static int plan_remap_frames(const char* who, const pb_plan* plan, int32_t elem_bytes, const double* frame_rotations,
+                             const void* src, int64_t src_frame_stride, void* dst, int64_t dst_frame_stride,
+                             int32_t n_frames, void* stream) {
+    if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
+    if (!plan || !frame_rotations || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
+    if (elem_bytes > 1)  // (uint8 has nothing to check, and then the plan is not read before n_frames is)
+        if (int rc = check_wide(elem_bytes, plan->src.kind, src, src_frame_stride, dst, dst_frame_stride, who)) return rc;
+    if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": negative n_frames");
+    if (n_frames == 0) return PB_OK;
+    if (int rc = check_plan_device(plan, who)) return rc;
+    if (plan->desc.n_rotations + 1 > PB_MAX_ROTATIONS)
+        return fail(PB_ERR_TOO_MANY_ROTATIONS,
+                    std::string(who) + ": the plan's rotations and the frame's are more than PB_MAX_ROTATIONS");
+    return plan_run_frames(*plan, elem_bytes, frame_rotations, src, src_frame_stride, dst, dst_frame_stride, n_frames,
+                           (cudaStream_t)stream);
 }
 
 static int plan_remap_rows(const char* who, const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band,
@@ -2051,6 +2130,13 @@ int pb_plan_remap_px(const pb_plan* plan, int32_t elem_bytes, const void* src, i
 int pb_plan_remap_rows_px(const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band, int32_t row_begin,
                           int32_t row_end, void* stream) {
     return plan_remap_rows("pb_plan_remap_rows_px", plan, elem_bytes, src, dst_band, row_begin, row_end, stream);
+}
+
+int pb_plan_remap_frames_px(const pb_plan* plan, int32_t elem_bytes, const double* frame_rotations, const void* src,
+                            int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames,
+                            void* stream) {
+    return plan_remap_frames("pb_plan_remap_frames_px", plan, elem_bytes, frame_rotations, src, src_frame_stride, dst,
+                             dst_frame_stride, n_frames, stream);
 }
 
 void pb_plan_destroy(pb_plan* plan) {

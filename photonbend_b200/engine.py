@@ -330,6 +330,55 @@ def remap_device(rays: RayPlan, src: ImageGeometry, src_dev, out_dev=None):
     return out_dev
 
 
+def frame_matrices(matrices) -> np.ndarray:
+    """(N, 9) C-contiguous float64 rows of N per-frame rotations: ``Rotation`` objects (their
+    ``rotation_matrix``) or 3x3 matrices, or an (N, 3, 3) array."""
+    if not isinstance(matrices, np.ndarray):
+        matrices = [getattr(m, "rotation_matrix", m) for m in matrices]
+    arr = np.ascontiguousarray(np.asarray(matrices, dtype=np.float64))
+    if arr.ndim != 3 or arr.shape[1:] != (3, 3):
+        raise ValueError(f"frame rotations must be N rotations or an (N, 3, 3) array, got shape {arr.shape}")
+    return arr.reshape(-1, 9)
+
+
+def remap_frames_device(rays: RayPlan, src: ImageGeometry, src_dev, matrices, out_dev=None):
+    """Fused remap of a batch in which frame k has a rotation of its own (pb_plan_remap_frames_px):
+    frame k equals ``remap_device(rays.rotated(matrices[k]), src, frame k)`` byte for byte.
+    ``matrices``: N ``Rotation`` objects or an (N, 3, 3) float64 array.  src_dev: a CUDA batch
+    (N, H, W, C) of an accepted dtype (ELEM_BYTES), or ONE image (H, W[, C]) seen through all N
+    rotations (source frame stride 0).  Returns (and fills) the (N, Ho, Wo[, C]) CUDA output."""
+    torch = _torch()
+    lib = _native.load()
+    e = check_source(src, src_dev)
+    mats = frame_matrices(matrices)
+    frames = mats.shape[0]
+    batched = src_dev.dim() == 4
+    if batched and src_dev.shape[0] != frames:
+        raise ValueError(f"{src_dev.shape[0]} source frames but {frames} frame rotations")
+    h, w, c, had_c = image_layout(src_dev[0] if batched else src_dev)
+    if (h, w) != (src.height, src.width):
+        raise ValueError(f"source image is {h}x{w} but its geometry says {src.height}x{src.width}")
+    oh, ow = rays.out.height, rays.out.output_width
+    out_shape = (frames, oh, ow, c) if had_c else (frames, oh, ow)
+    if out_dev is None:
+        out_dev = torch.empty(out_shape, dtype=src_dev.dtype, device=src_dev.device)
+    else:
+        _check_out(out_dev, out_shape, src_dev)
+    if len(rays.rotations) + 1 > _native.PB_MAX_ROTATIONS:
+        raise _native.NativeError(_native.PB_ERR_TOO_MANY_ROTATIONS, "too many rotations to fuse")
+    if frames == 0:
+        return out_dev
+    desc = _remap_desc(rays, src, c)
+    with torch.cuda.device(src_dev.device):
+        plan = _plans.get(lib, desc, src_dev.device.index or 0, torch)
+        _native.check(lib.pb_plan_remap_frames_px(
+            plan, ctypes.c_int32(e), mats.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+            ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_int64(h * w * c * e if batched else 0),
+            ctypes.c_void_p(out_dev.data_ptr()), ctypes.c_int64(oh * ow * c * e), ctypes.c_int32(frames),
+            _stream_ptr(torch)))
+    return out_dev
+
+
 def remap_rows_device(rays: RayPlan, src: ImageGeometry, src_dev, row_begin: int, row_end: int, out_dev=None):
     """Output rows [row_begin, row_end) of one frame (pb_plan_remap_rows_u8 / _px): src_dev is the
     WHOLE source image on this device, the result is the band alone, (row_end - row_begin, Wo[, C]),

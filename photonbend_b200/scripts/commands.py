@@ -18,7 +18,10 @@ Same command names, arguments, options and exit behaviour as the reference
 A DIRECTORY as INPUT (an extension over the reference: the frames of a video, photos from one
 camera) converts every .jpg/.jpeg/.png in it with the same parameters into the OUTPUT directory,
 frames sharded over the visible GPUs (photonbend_b200/stream.py); ``--frames-per-launch`` sets how
-many frames share a kernel launch.
+many frames share a kernel launch.  ``--frame-rotations FILE`` gives every frame a rotation of its
+own, applied after the ``-r`` rotations (stabilised or levelled footage, a moving virtual camera):
+one line ``<file name> <pitch> <yaw> <roll>`` (degrees) per frame; blank lines and ``#`` comments
+are ignored.
 
 Everything between decode and encode runs on the GPU: the source array is uploaded once, the
 three-call protocol (get_coordinate_map / rotate_coordinate_map / process_coordinate_map) costs
@@ -141,9 +144,49 @@ def _remap(source, destination, rotations: List[Tuple[float, float, float]]) -> 
     return source.process_coordinate_map(coordinate_map)
 
 
-def _remap_directory(in_dir: Path, out_dir: Path, make_pair, rotations, frames_per_launch: int) -> None:
+def _exit_with(message: str) -> None:
+    print(message)
+    print("Exiting!")
+    sys.exit(1)
+
+
+def _read_frame_rotations(path: Path, files: List[Path]) -> List[Rotation]:
+    """The rotation of every frame of ``files`` from a ``--frame-rotations`` file, in frame order;
+    exits 1 on a malformed line, a name that is not a frame, a frame listed twice or not at all."""
+    try:
+        text = Path(path).read_text()
+    except (OSError, UnicodeDecodeError):
+        _exit_with(f"Error: frame rotations file {path} could not be read!")
+    names = {f.name for f in files}
+    angles = {}
+    for number, line in enumerate(text.splitlines(), 1):
+        fields = line.split("#", 1)[0].split()
+        if not fields:
+            continue
+        try:
+            if len(fields) != 4:
+                raise ValueError
+            pitch, yaw, roll = (float(v) for v in fields[1:])
+        except ValueError:
+            _exit_with(f"Error: {path}:{number}: expected <file name> <pitch> <yaw> <roll>, got {line.strip()!r}")
+        name = fields[0]
+        if name not in names:
+            _exit_with(f"Error: {path}:{number}: {name} is not a frame of the input directory")
+        if name in angles:
+            _exit_with(f"Error: {path}:{number}: frame {name} is listed twice")
+        angles[name] = (pitch, yaw, roll)
+    missing = [f.name for f in files if f.name not in angles]
+    if missing:
+        _exit_with(f"Error: {path} gives no rotation for frame {missing[0]}"
+                   + (f" (and {len(missing) - 1} more)" if len(missing) > 1 else ""))
+    return [Rotation(to_radians(p), to_radians(y), to_radians(r)) for p, y, r in (angles[f.name] for f in files)]
+
+
+def _remap_directory(in_dir: Path, out_dir: Path, make_pair, rotations, frames_per_launch: int,
+                     frame_rotations: Optional[Path] = None) -> None:
     """Every image of ``in_dir`` through the geometry ``make_pair(first_frame_pixels)`` ->
-    (source, destination) into ``out_dir`` (same file names), sharded over the visible GPUs."""
+    (source, destination) into ``out_dir`` (same file names), sharded over the visible GPUs; frame
+    k also through its own rotation from the ``frame_rotations`` file when given."""
     from photonbend_b200 import stream
 
     out_dir = Path(out_dir)
@@ -156,6 +199,7 @@ def _remap_directory(in_dir: Path, out_dir: Path, make_pair, rotations, frames_p
         print("Error: no .jpg / .jpeg / .png frames in the input directory!")
         print("Exiting!")
         sys.exit(1)
+    per_frame = None if frame_rotations is None else _read_frame_rotations(frame_rotations, files)
     outs = [out_dir / f.name for f in files]
     if any(o.exists() for o in outs):
         answer = ""
@@ -179,7 +223,8 @@ def _remap_directory(in_dir: Path, out_dir: Path, make_pair, rotations, frames_p
         coordinate_map = Rotation(to_radians(pitch), to_radians(yaw), to_radians(roll)).rotate_coordinate_map(
             coordinate_map)
     try:
-        stats = stream.remap_files(source, coordinate_map, files, outs, batch=max(1, frames_per_launch))
+        stats = stream.remap_files(source, coordinate_map, files, outs, batch=max(1, frames_per_launch),
+                                   frame_rotations=per_frame)
     except IOError:
         print("Could not read or save a frame!")
         print("Exiting!")
@@ -196,6 +241,22 @@ def _frames_option(fn):
 def _rotation_option(fn):
     return click.option("-r", "--rotation", required=False, type=click.FLOAT, nargs=3, default=[],
                         help=_ROTATION_HELP, multiple=True)(fn)
+
+
+def _frame_rotations_option(fn):
+    return click.option("--frame-rotations", required=False, default=None,
+                        type=click.Path(exists=True, dir_okay=False, path_type=Path),
+                        help="Directory input only: a file of '<file name> <pitch> <yaw> <roll>' lines (degrees), "
+                             "one rotation per frame, applied after the -r rotations.")(fn)
+
+
+def _single_image(input_image, frame_rotations) -> bool:
+    """True for a single-image INPUT; exits 1 when --frame-rotations was given with one."""
+    if Path(input_image).is_dir():
+        return False
+    if frame_rotations is not None:
+        _exit_with("Error: --frame-rotations needs a directory of frames as input.")
+    return True
 
 
 def _size_option(fn):
@@ -217,8 +278,9 @@ def _size_option(fn):
 @_rotation_option
 @_size_option
 @_frames_option
+@_frame_rotations_option
 @click.argument("output_image", type=click.Path(exists=False, path_type=Path))
-def make_pano(input_image, itype, lens, fov, output_image, rotation, size, frames_per_launch):
+def make_pano(input_image, itype, lens, fov, output_image, rotation, size, frames_per_launch, frame_rotations):
     """Make a panorama out of a photo.
 
     \b
@@ -230,8 +292,8 @@ def make_pano(input_image, itype, lens, fov, output_image, rotation, size, frame
         height = pixels.shape[0] if size is None else size
         return source, PanoramaImage(np.zeros((height, int(height * 2), CHANNELS), np.uint8))
 
-    if Path(input_image).is_dir():
-        return _remap_directory(input_image, output_image, pair, rotation, frames_per_launch)
+    if not _single_image(input_image, frame_rotations):
+        return _remap_directory(input_image, output_image, pair, rotation, frames_per_launch, frame_rotations)
     out = _checked_output(output_image)
     source, destination = pair(_load_pixels(input_image))
     _save_pixels(_remap(source, destination, rotation), out)
@@ -257,8 +319,9 @@ def make_pano(input_image, itype, lens, fov, output_image, rotation, size, frame
 @_rotation_option
 @_size_option
 @_frames_option
+@_frame_rotations_option
 @click.argument("output_image", type=click.Path(exists=False, path_type=Path))
-def alter_photo(input_image, itype, ilens, ifov, otype, olens, ofov, output_image, rotation, size, frames_per_launch):
+def alter_photo(input_image, itype, ilens, ifov, otype, olens, ofov, output_image, rotation, size, frames_per_launch, frame_rotations):
     """Change the the lens and FoV of a photo.
 
     \b
@@ -271,8 +334,8 @@ def alter_photo(input_image, itype, ilens, ifov, otype, olens, ofov, output_imag
         # output magnitude from the INPUT shape, as the reference does
         return source, _photo(canvas, otype, olens, _fov_radians(ofov, otype), _magnitude(otype, pixels.shape))
 
-    if Path(input_image).is_dir():
-        return _remap_directory(input_image, output_image, pair, rotation, frames_per_launch)
+    if not _single_image(input_image, frame_rotations):
+        return _remap_directory(input_image, output_image, pair, rotation, frames_per_launch, frame_rotations)
     out = _checked_output(output_image)
     source, destination = pair(_load_pixels(input_image))
     _save_pixels(_remap(source, destination, rotation), out)
@@ -292,8 +355,9 @@ def alter_photo(input_image, itype, ilens, ifov, otype, olens, ofov, output_imag
 @_rotation_option
 @_size_option
 @_frames_option
+@_frame_rotations_option
 @click.argument("output_image", type=click.Path(exists=False, path_type=Path))
-def make_photo(input_image, otype, lens, fov, output_image, rotation, size, frames_per_launch):
+def make_photo(input_image, otype, lens, fov, output_image, rotation, size, frames_per_launch, frame_rotations):
     """Make a photo out of a panorama.
 
     \b
@@ -305,8 +369,8 @@ def make_photo(input_image, otype, lens, fov, output_image, rotation, size, fram
         return PanoramaImage(pixels), _photo(np.zeros(shape, np.uint8), otype, lens, _fov_radians(fov, otype),
                                              _magnitude(otype, shape))
 
-    if Path(input_image).is_dir():
-        return _remap_directory(input_image, output_image, pair, rotation, frames_per_launch)
+    if not _single_image(input_image, frame_rotations):
+        return _remap_directory(input_image, output_image, pair, rotation, frames_per_launch, frame_rotations)
     out = _checked_output(output_image)
     source, destination = pair(_load_pixels(input_image))
     _save_pixels(_remap(source, destination, rotation), out)

@@ -52,8 +52,10 @@ def _encode_host(pixels: np.ndarray, path) -> None:
     Image.fromarray(pixels).save(path)
 
 
-def _host_worker(device: int, frames: Sequence[int], source, cmap, in_files, out_files, depth, batch, codec_threads, shape):
-    """Pillow codec: pinned host frames through a FramePipeline on GPU ``device``."""
+def _host_worker(device: int, frames: Sequence[int], source, cmap, in_files, out_files, depth, batch, codec_threads, shape,
+                 rotations=None):
+    """Pillow codec: pinned host frames through a FramePipeline on GPU ``device`` (frame k through
+    ``rotations[k]`` when given)."""
     torch = engine._torch()
     with torch.cuda.device(device):
         pipe = FramePipeline(source, cmap, depth=depth, device=device, batch=batch)
@@ -95,7 +97,7 @@ def _host_worker(device: int, frames: Sequence[int], source, cmap, in_files, out
                 ins[slot].numpy()[...] = pixels
                 group.append((slot, k))
                 launch_of[slot] = len(launches)
-                event = pipe.submit(ins[slot], outs[slot])
+                event = pipe.submit(ins[slot], outs[slot], None if rotations is None else rotations[k])
                 if event is not None:
                     launches.append([event, group])
                     group = []
@@ -116,12 +118,13 @@ def _default_decode_threads(batch: int, n_devices: int) -> int:
 
 
 def _compressed_pipeline(device: int, frames: Sequence[int], source, cmap, load, store, batch: int, decode_threads: int,
-                         shape) -> int:
+                         shape, rotations=None) -> int:
     """Frames ``frames`` on GPU ``device``, compressed on both sides of PCIe: ``load(k)`` gives the JPEG
     bytes of frame k, ``store(k, data)`` takes the JPEG bytes of its remap.  A producer (the calling
     thread) has batch n + 1 decoded into the other of two device buffers by ``decode_threads``
     workers -- one frame each, every worker its own decoder state and stream -- while a consumer
-    thread remaps batch n (ONE launch) and encodes it.  Returns the number of kernel launches."""
+    thread remaps batch n (ONE launch; frame k through ``rotations[k]`` when given) and encodes it.
+    Returns the number of kernel launches."""
     torch = engine._torch()
     chunks = [frames[c0:c0 + batch] for c0 in range(0, len(frames), batch)]
     if not chunks:
@@ -145,7 +148,9 @@ def _compressed_pipeline(device: int, frames: Sequence[int], source, cmap, load,
                         if failed:
                             return
                         k = len(chunk)
-                        if k == 1:
+                        if rotations is not None:
+                            engine.remap_frames_device(rays, geom, srcs[b][:k], [rotations[f] for f in chunk], dst[:k])
+                        elif k == 1:
                             engine.remap_device(rays, geom, srcs[b][0], dst[0])
                         else:
                             engine.remap_device(rays, geom, srcs[b][:k], dst[:k])
@@ -188,7 +193,8 @@ def _compressed_pipeline(device: int, frames: Sequence[int], source, cmap, load,
     return len(chunks)
 
 
-def _device_worker(device: int, frames: Sequence[int], source, cmap, in_files, out_files, batch, shape, n_devices=1):
+def _device_worker(device: int, frames: Sequence[int], source, cmap, in_files, out_files, batch, shape, n_devices=1,
+                   rotations=None):
     """nvJPEG codec on files: compressed bytes up, decode -> remap -> encode on GPU ``device``, compressed bytes down."""
 
     def load(k):
@@ -201,19 +207,31 @@ def _device_worker(device: int, frames: Sequence[int], source, cmap, in_files, o
 
     if batch <= 1:
         batch = 8  # (frames of a batch are decoded at once; one frame per launch would decode one at a time)
-    return _compressed_pipeline(device, frames, source, cmap, load, store, batch, _default_decode_threads(batch, n_devices), shape)
+    return _compressed_pipeline(device, frames, source, cmap, load, store, batch, _default_decode_threads(batch, n_devices), shape,
+                                rotations)
+
+
+def _frame_rotations(frame_rotations, n_frames: int):
+    """(N, 3, 3) float64 matrices of per-frame rotations, checked against the number of frames; None stays None."""
+    if frame_rotations is None:
+        return None
+    mats = engine.frame_matrices(frame_rotations).reshape(-1, 3, 3)
+    if mats.shape[0] != n_frames:
+        raise ValueError(f"{mats.shape[0]} frame rotations for {n_frames} frames")
+    return mats
 
 
 def remap_jpeg_stream(source, coordinate_map: CoordinateMap, jpegs: Sequence[bytes], devices: Optional[Sequence[int]] = None,
-                      batch: int = 8, decode_threads: Optional[int] = None) -> List[bytes]:
+                      batch: int = 8, decode_threads: Optional[int] = None, frame_rotations=None) -> List[bytes]:
     """Compressed stream in memory: JPEG bytes in -> nvJPEG decode on the device -> ONE remap launch
     per ``batch`` frames -> nvJPEG encode on the device -> JPEG bytes out.  Frame k on GPU
     ``devices[k mod G]``; per GPU a producer that decodes batch k + 1 with ``decode_threads`` host
     threads (each its own decoder state and stream; default: up to 8, at most one per frame of a
     batch and what the host's cores allow per GPU) while a consumer remaps and encodes batch k; raw
-    pixels never cross PCIe."""
+    pixels never cross PCIe.  ``frame_rotations``: one rotation per frame, as in ``remap_files``."""
     if not (isinstance(coordinate_map, CoordinateMap) and coordinate_map.is_lazy):
         raise ValueError("remap_jpeg_stream needs the lazy CoordinateMap of get_coordinate_map()")
+    rotations = _frame_rotations(frame_rotations, len(jpegs))
     torch = engine._torch()
     if devices is None:
         devices = list(range(torch.cuda.device_count()))
@@ -231,7 +249,7 @@ def remap_jpeg_stream(source, coordinate_map: CoordinateMap, jpegs: Sequence[byt
         try:
             frames = list(shard_frames(len(jpegs), g, len(devices)))
             _compressed_pipeline(devices[g], frames, source, coordinate_map, jpegs.__getitem__, store, batch,
-                                 decode_threads, shape)
+                                 decode_threads, shape, rotations)
         except BaseException as exc:  # noqa: BLE001
             errors.append(exc)
 
@@ -247,15 +265,19 @@ def remap_jpeg_stream(source, coordinate_map: CoordinateMap, jpegs: Sequence[byt
 
 def remap_files(source, coordinate_map: CoordinateMap, in_files: Sequence, out_files: Sequence,
                 devices: Optional[Sequence[int]] = None, depth: int = 3, batch: int = 1,
-                codec: Optional[str] = None, codec_threads: int = 4) -> dict:
+                codec: Optional[str] = None, codec_threads: int = 4, frame_rotations=None) -> dict:
     """Remap ``in_files[k]`` -> ``out_files[k]`` for files that all have the geometry of ``source``
     (a CameraImage / DoubleCameraImage / PanoramaImage; its own ``image`` only gives the frame
     shape) along the lazy ``coordinate_map``.  Frame k runs on ``devices[k mod G]`` (default: every
-    visible GPU), one host thread per GPU.  Returns {"frames", "gpus", "seconds", "kernel_launches"}."""
+    visible GPU), one host thread per GPU.  ``frame_rotations`` (one ``Rotation`` or 3x3 matrix per
+    file): frame k is remapped as if ``frame_rotations[k]`` had been applied after the map's own
+    rotations, and the rotation travels with the frame to its GPU.  Returns {"frames", "gpus",
+    "seconds", "kernel_launches"}."""
     if not (isinstance(coordinate_map, CoordinateMap) and coordinate_map.is_lazy):
         raise ValueError("remap_files needs the lazy CoordinateMap of get_coordinate_map()")
     if len(in_files) != len(out_files):
         raise ValueError("in_files and out_files differ in length")
+    rotations = _frame_rotations(frame_rotations, len(in_files))
     torch = engine._torch()
     codec = codec or image_io.selected_codec()
     if devices is None:
@@ -271,10 +293,10 @@ def remap_files(source, coordinate_map: CoordinateMap, in_files: Sequence, out_f
         try:
             if on_device:
                 results[g] = _device_worker(devices[g], frames, source, coordinate_map, in_files, out_files, max(1, batch), shape,
-                                            len(devices))
+                                            len(devices), rotations)
             else:
                 results[g] = _host_worker(devices[g], frames, source, coordinate_map, in_files, out_files, depth,
-                                          max(1, batch), codec_threads, shape)
+                                          max(1, batch), codec_threads, shape, rotations)
         except BaseException as exc:  # noqa: BLE001  (re-raised on the calling thread)
             errors.append(exc)
 
