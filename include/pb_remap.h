@@ -271,6 +271,16 @@ int pb_debug_plan_fast32(const pb_plan *plan, double out[2]);
  */
 int pb_debug_plan_boxes(const pb_plan *plan, int32_t *table, int64_t capacity, int32_t dims[3]);
 
+/*
+ * The staging sizes a plan picked from its footprint census at pb_plan_create, and those its batches
+ * launch with: out = {stage-buffer bytes of remap_tiled_kernel, widest staged row in 16-byte units
+ * (the plan's widest tensor map), stage buffers of a batch through remap_tiled_kernel, stage-buffer
+ * bytes of the single-frame kernel for a camera source, the same for a double-fisheye source's
+ * two-lens tiles (or every tile), the same for its one-lens tiles, frame-group ring bytes of
+ * remap_boxes_kernel for the one-lens tiles, the same for the rest}.  No reference counterpart.
+ */
+int pb_debug_plan_stage(const pb_plan *plan, int32_t out[8]);
+
 #ifdef __cplusplus
 }
 #endif

@@ -166,10 +166,13 @@ def coordinate_map(out_geom, rotations=(), threads=0):
     return cmap
 
 
-def source_index(out_geom, rotations, src_geom, threads=0):
-    """int64 (H, W, 2): linear source pixel offsets (left/only, right) or -1 for black."""
+def source_index(out_geom, rotations, src_geom, threads=0, rows=None):
+    """int64 (H, W, 2): linear source pixel offsets (left/only, right) or -1 for black.
+    ``rows=(r0, r1)`` returns only that band of output rows, (r1 - r0, W, 2)."""
     h, w = out_shape(out_geom)
-    idx = np.empty((h, w, 2), dtype=np.int64)
+    r0, r1 = (0, h) if rows is None else rows
+    band = np.empty((r1 - r0, w, 2), dtype=np.int64)
+    base = band.ctypes.data - r0 * w * 2 * 8  # C writes row i at offset i*w*2 int64s
     n, mats = _matrices(rotations)
     o, s = _describe(out_geom), _describe(src_geom)
     fn = lib().pbo_source_index_i64
@@ -180,10 +183,10 @@ def source_index(out_geom, rotations, src_geom, threads=0):
             ctypes.c_int(n),
             mats.ctypes.data_as(ctypes.c_void_p),
             ctypes.byref(s),
-            idx.ctypes.data_as(ctypes.c_void_p),
+            ctypes.c_void_p(base),
             ctypes.c_int(a),
             ctypes.c_int(b),
         )
 
-    _run_banded(call, 0, h, threads)
-    return idx
+    _run_banded(call, r0, r1, threads)
+    return band

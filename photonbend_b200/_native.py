@@ -48,6 +48,7 @@ EXPORTS = (
     "pb_debug_fast32_stats",
     "pb_debug_plan_fast32",
     "pb_debug_plan_boxes",
+    "pb_debug_plan_stage",
     "pb_plan_remap_px",
     "pb_plan_remap_rows_px",
     "pb_gather_from_map_px",
@@ -137,6 +138,8 @@ def load():
     lib.pb_debug_plan_fast32.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
     lib.pb_debug_plan_boxes.restype = ctypes.c_int
     lib.pb_debug_plan_boxes.argtypes = [vp, ctypes.POINTER(ctypes.c_int32), ctypes.c_int64, ctypes.POINTER(ctypes.c_int32)]
+    lib.pb_debug_plan_stage.restype = ctypes.c_int
+    lib.pb_debug_plan_stage.argtypes = [vp, ctypes.POINTER(ctypes.c_int32)]
     lib.pb_plan_remap_px.restype = ctypes.c_int
     lib.pb_plan_remap_px.argtypes = [vp, i32, vp, i64, vp, i64, i32, vp]
     lib.pb_plan_remap_rows_px.restype = ctypes.c_int

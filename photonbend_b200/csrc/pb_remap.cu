@@ -398,11 +398,7 @@ __device__ __forceinline__ void zero_px(T* __restrict__ d) {
 // Generic fused remap: one thread resolves one output pixel (float64, every polar round trip
 // of the reference kept), then applies the resolved lookup to every frame of the batch.
 template <int OUT_KIND, int SRC_KIND, int C>
-__global__ void __launch_bounds__(256) remap_generic_kernel(const __grid_constant__ RemapArgs a) {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = a.row_begin + blockIdx.y * blockDim.y + threadIdx.y;
-    if (i >= a.row_end || j >= a.out.W) return;
-
+__device__ __forceinline__ void generic_pixel(const RemapArgs& a, int i, int j) {
     const Lookup L = resolve_lookup<OUT_KIND, SRC_KIND>(a.out, a.fast, a.rot, a.src, i, j);
     const int off0 = xy_to_offset(L.xy0, a.src.W);
     const int off1 = xy_to_offset(L.xy1, a.src.W);
@@ -425,6 +421,16 @@ __global__ void __launch_bounds__(256) remap_generic_kernel(const __grid_constan
             }
         }
     }
+}
+
+template <int OUT_KIND, int SRC_KIND, int C>
+__global__ void __launch_bounds__(256) remap_generic_kernel(const __grid_constant__ RemapArgs a) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= a.out.W) return;
+    // (a grid has at most 65535 rows of blocks: taller outputs loop over row blocks, see grid_rows)
+    for (long long i = a.row_begin + blockIdx.y * blockDim.y + threadIdx.y; i < a.row_end;
+         i += (long long)gridDim.y * blockDim.y)
+        generic_pixel<OUT_KIND, SRC_KIND, C>(a, (int)i, j);
 }
 
 // ONE frame, any geometry (rotated remaps above all): every thread resolves two quads of four
@@ -543,13 +549,9 @@ __global__ void __launch_bounds__(256, PB_DIRECT_MIN_CTAS) remap_direct32_kernel
 // counters: [0] pixels, [1] undecided by tier 1, [2] decided by tier 1 but different from tiers 2/3,
 // [3] float and double evaluations disagree on a pixel's status (fov / no-pixel decisions)
 template <int OUT_KIND, int SRC_KIND>
-__global__ void __launch_bounds__(256) fast32_stats_kernel(const __grid_constant__ RemapArgs a,
-                                                           const __grid_constant__ Fast32GeomT<double> gd,
-                                                           unsigned* __restrict__ maxima,
-                                                           unsigned long long* __restrict__ counters) {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = blockIdx.y * blockDim.y + threadIdx.y;
-    if (i >= a.out.H || j >= a.out.W) return;
+__device__ __forceinline__ void fast32_stats_pixel(const RemapArgs& a, const Fast32GeomT<double>& gd,
+                                                   unsigned* __restrict__ maxima, unsigned long long* __restrict__ counters,
+                                                   int i, int j) {
     const Coords32<float> cf = coords32<float, OUT_KIND, SRC_KIND>(a.out, a.fast.f32, a.src, i, j);
     const Coords32<double> cd = coords32<double, OUT_KIND, SRC_KIND>(a.out, gd, a.src, i, j);
     const double eps = 5.9604644775390625e-08;
@@ -572,6 +574,18 @@ __global__ void __launch_bounds__(256) fast32_stats_kernel(const __grid_constant
     }
 }
 
+template <int OUT_KIND, int SRC_KIND>
+__global__ void __launch_bounds__(256) fast32_stats_kernel(const __grid_constant__ RemapArgs a,
+                                                           const __grid_constant__ Fast32GeomT<double> gd,
+                                                           unsigned* __restrict__ maxima,
+                                                           unsigned long long* __restrict__ counters) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= a.out.W) return;
+    // (taller outputs than the grid's 65535 rows of blocks loop over row blocks, see grid_rows)
+    for (long long i = blockIdx.y * blockDim.y + threadIdx.y; i < a.out.H; i += (long long)gridDim.y * blockDim.y)
+        fast32_stats_pixel<OUT_KIND, SRC_KIND>(a, gd, maxima, counters, (int)i, j);
+}
+
 // The calibration half of the above alone (pb_plan_create): largest |float - double| / (2^-24 * shape)
 // of a coordinate over the pixels both evaluations give coordinates for, as float bits.
 template <int OUT_KIND, int SRC_KIND>
@@ -579,20 +593,25 @@ __global__ void __launch_bounds__(256) fast32_ratio_kernel(const __grid_constant
                                                            const __grid_constant__ Fast32GeomT<double> gd,
                                                            unsigned* __restrict__ maxima) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = blockIdx.y * blockDim.y + threadIdx.y;
     float r = 0.0f;
-    if (i < a.out.H && j < a.out.W) {
+    // (taller outputs than the grid's 65535 rows of blocks loop over row blocks, see grid_rows; the
+    // 32 lanes of a warp share their rows, so they run the same trips)
+    for (long long ii = blockIdx.y * blockDim.y + threadIdx.y; ii < a.out.H; ii += (long long)gridDim.y * blockDim.y) {
+        const int i = (int)ii;
+        if (j >= a.out.W) break;
         const Coords32<float> cf = coords32<float, OUT_KIND, SRC_KIND>(a.out, a.fast.f32, a.src, i, j);
         if (cf.status != 2) {
             const Coords32<double> cd = coords32<double, OUT_KIND, SRC_KIND>(a.out, gd, a.src, i, j);
             const double eps = 5.9604644775390625e-08;
+            float q = 0.0f;  // this pixel's ratio
             if (cf.status == 0 && cd.status == 0)
-                r = fmaxf((float)(fabs((double)cf.vx - cd.vx) / (eps * (double)cf.ex)),
+                q = fmaxf((float)(fabs((double)cf.vx - cd.vx) / (eps * (double)cf.ex)),
                           (float)(fabs((double)cf.vy - cd.vy) / (eps * (double)cf.ey)));
             if (SRC_KIND == PB_KIND_DOUBLE && cd.status != 2 && cf.slot1 == 0 && cd.slot1 == 0)
-                r = fmaxf(r, fmaxf((float)(fabs((double)cf.wx - cd.wx) / (eps * (double)cf.fx_)),
+                q = fmaxf(q, fmaxf((float)(fabs((double)cf.wx - cd.wx) / (eps * (double)cf.fx_)),
                                    (float)(fabs((double)cf.wy - cd.wy) / (eps * (double)cf.fy_))));
-            if (!(r >= 0.0f)) r = INFINITY;  // a NaN must not hide behind the maximum
+            if (!(q >= 0.0f)) q = INFINITY;  // a NaN must not hide behind the maximum
+            r = fmaxf(r, q);
         }
     }
     const unsigned bits = __reduce_max_sync(0xffffffffu, __float_as_uint(r));  // (non-negative floats order like their bits)
@@ -605,14 +624,16 @@ __global__ void __launch_bounds__(256) materialize_map_kernel(const __grid_const
                                                               const __grid_constant__ Rotations rot,
                                                               double* __restrict__ map) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = blockIdx.y * blockDim.y + threadIdx.y;
-    if (i >= out.H || j >= out.W) return;
-    Ray r = output_ray<OUT_KIND>(out, i, j);
-    for (int k = 0; k < rot.n; ++k) r = rotate_ray(r, rot.m[k]);
-    double* m = map + ((long long)i * out.W + j) * 3;
-    m[0] = r.lat;
-    m[1] = r.lon;
-    m[2] = r.invalid ? 1.0 : 0.0;
+    if (j >= out.W) return;
+    // (taller maps than the grid's 65535 rows of blocks loop over row blocks, see grid_rows)
+    for (long long i = blockIdx.y * blockDim.y + threadIdx.y; i < out.H; i += (long long)gridDim.y * blockDim.y) {
+        Ray r = output_ray<OUT_KIND>(out, (int)i, j);
+        for (int k = 0; k < rot.n; ++k) r = rotate_ray(r, rot.m[k]);
+        double* m = map + (i * out.W + j) * 3;
+        m[0] = r.lat;
+        m[1] = r.lon;
+        m[2] = r.invalid ? 1.0 : 0.0;
+    }
 }
 
 struct Mat3 {
@@ -821,9 +842,13 @@ static void launch_direct(const RemapArgs& a, cudaStream_t st) {
     }
 }
 
+// Rows of blocks of a 2-D grid of (32, 8) blocks over rows output rows: at most 65535, the grid's
+// limit; the kernels that take it loop over the row blocks past it.
+static unsigned grid_rows(int rows) { return (unsigned)std::min(((long long)rows + 7) / 8, 65535LL); }
+
 static void launch_generic(const RemapArgs& a, cudaStream_t st) {
     dim3 block(32, 8);
-    dim3 grid((a.out.W + block.x - 1) / block.x, (a.row_end - a.row_begin + block.y - 1) / block.y);
+    dim3 grid((a.out.W + block.x - 1) / block.x, grid_rows(a.row_end - a.row_begin));
     with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
         with_channels(a.src.C, [&](auto c) { remap_generic_kernel<o, s, c><<<grid, block, 0, st>>>(a); });
     });
@@ -1554,6 +1579,30 @@ static cudaError_t fill_tables(const pb_plan& p, double* tables, cudaStream_t st
     return cudaGetLastError();
 }
 
+// Stage buffers of a launch of remap_tiled_kernel through plan p: a second one lets the loads of the
+// next (frame, slot) item overlap the current gather; taken when three CTAs per SM still fit.
+// multi: more than one frame (two output tile buffers); mode1: the separable tables.
+static int tiled_buffers(const pb_plan& p, bool multi, bool mode1) {
+    const bool dbl = p.src.kind == PB_KIND_DOUBLE;
+    if (!multi && !dbl) return 1;
+    const int n_out = multi ? 2 : 1;
+    int two;
+    if (dbl) two = mode1 ? tiled_smem_bytes<PB_KIND_DOUBLE, 1>(p.stage_bytes, 2, n_out)
+                         : tiled_smem_bytes<PB_KIND_DOUBLE, 0>(p.stage_bytes, 2, n_out);
+    else two = mode1 ? tiled_smem_bytes<PB_KIND_CAMERA, 1>(p.stage_bytes, 2, n_out)
+                     : tiled_smem_bytes<PB_KIND_CAMERA, 0>(p.stage_bytes, 2, n_out);
+    int limit_kib = 75;  // three CTAs per SM
+    if (const char* e = std::getenv("PB_TWO_BUF_LIMIT_KIB")) limit_kib = std::atoi(e);  // tuning experiments
+    return two <= limit_kib * 1024 ? 2 : 1;
+}
+// A batch through a double-fisheye plan: the stage buffer of the tiles that see one lens (four CTAs
+// per SM) and of the rest (two CTAs per SM, twice the stage area)
+static int one_stage_bytes() { return env_int("PB_ONE_BYTES", 21 * 1024); }
+static int rest_stage_bytes() { return env_int("PB_REST_KIB", 50) * 1024; }
+// ... and the ring of frame groups of remap_boxes_kernel of tile class cls: what were the two stage
+// buffers of remap_tiled_kernel (one lens), or of remap_two_lens_kernel (the rest)
+static int boxes_stage_bytes(int cls) { return cls == 1 ? 2 * one_stage_bytes() + 128 : 2 * rest_stage_bytes(); }
+
 // tables: the plan's own, a transient stream-ordered allocation, or null (generic rays)
 // [row_begin, row_end): the output rows to produce; dst points at row row_begin (a band of a
 // single frame, or the whole image)
@@ -1620,18 +1669,7 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
         // a second stage buffer lets the loads of the next (frame, slot) item overlap the current
         // gather; taken when three CTAs per SM still fit
         a.n_out = multi ? 2 : 1;
-        a.n_buffers = 1;
-        if (multi || dbl) {
-            const int mode = (p.separable && tables != nullptr) ? 1 : 0;
-            int two;
-            if (dbl) two = mode ? tiled_smem_bytes<PB_KIND_DOUBLE, 1>(a.stage_bytes, 2, a.n_out)
-                                : tiled_smem_bytes<PB_KIND_DOUBLE, 0>(a.stage_bytes, 2, a.n_out);
-            else two = mode ? tiled_smem_bytes<PB_KIND_CAMERA, 1>(a.stage_bytes, 2, a.n_out)
-                            : tiled_smem_bytes<PB_KIND_CAMERA, 0>(a.stage_bytes, 2, a.n_out);
-            int limit_kib = 75;  // three CTAs per SM
-            if (const char* e = std::getenv("PB_TWO_BUF_LIMIT_KIB")) limit_kib = std::atoi(e);  // tuning experiments
-            if (two <= limit_kib * 1024) a.n_buffers = 2;
-        }
+        a.n_buffers = tiled_buffers(p, multi, p.separable && tables != nullptr);
         if (cached_src_maps(p, src, src_pitch, n_frames, src_frame_stride, a.max_units, a.src_maps) &&
             cached_dst_map(p, dst, dst_pitch, row_end - row_begin, n_frames, dst_frame_stride, &a.dst_map)) {
             const bool sep = p.separable && tables != nullptr;
@@ -1679,12 +1717,12 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
                 a.n_out = 2;
                 a.tile_list = p.tile_lists + p.n_one;
                 a.n_list = p.n_rest;
-                a.stage_bytes = env_int("PB_REST_KIB", 50) * 1024;
+                a.stage_bytes = rest_stage_bytes();
                 pb_plan::SideLane* lane = fork_side(p, st);
                 TiledArgs b = a;
                 b.tile_list = p.tile_lists;
                 b.n_list = p.n_one;
-                b.stage_bytes = env_int("PB_ONE_BYTES", 21 * 1024);  // four CTAs per SM
+                b.stage_bytes = one_stage_bytes();
                 // the two-lens / blend-band tiles stage the chunks their pixels touch instead of bounding
                 // rectangles (pb_chunk.cuh); PB_CHUNK: bit 0 = that class, bit 1 = the one-lens class too
                 const int chunk = env_int("PB_CHUNK", 0);
@@ -1699,7 +1737,7 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
                     a.stage_bytes = env_int("PB_CHUNK_REST_KIB", 94) * 1024;
                     e = launch_chunk_one<PB_KIND_DOUBLE, 2>(a, lane ? lane->side : st);
                 } else if (boxed) {
-                    a.stage_bytes = 2 * a.stage_bytes;  // the ring of frame groups of remap_two_lens_kernel
+                    a.stage_bytes = boxes_stage_bytes(2);
                     e = launch_boxes<2>(a, lane ? lane->side : st);
                 } else if (env_int("PB_CLS2_THREADS", 512) == 512) {
                     // 16 warps per CTA, one quad per thread: twice the warps per SM for the same shared memory
@@ -1714,7 +1752,7 @@ static int plan_run(pb_plan& p, const double* tables, const uint8_t* src, int64_
                         b.stage_bytes = env_int("PB_CHUNK_ONE_KIB", 38) * 1024;
                         e = launch_chunk_one<PB_KIND_DOUBLE, 1>(b, st);
                     } else if (boxed) {
-                        b.stage_bytes = 2 * b.stage_bytes + 128;  // the ring of the two stage buffers of remap_tiled_kernel
+                        b.stage_bytes = boxes_stage_bytes(1);
                         e = launch_boxes<1>(b, st);
                     } else {
                         e = launch_tiled_one<PB_KIND_EQUIRECT, PB_KIND_DOUBLE, 1, 1>(b, st);
@@ -2029,7 +2067,7 @@ static void calibrate_fast32(pb_plan& p, cudaStream_t st) {
     }
     cudaMemsetAsync(dev, 0, sizeof(unsigned), st);
     dim3 block(32, 8);
-    dim3 grid((a.out.W + block.x - 1) / block.x, (a.out.H + block.y - 1) / block.y);
+    dim3 grid((a.out.W + block.x - 1) / block.x, grid_rows(a.out.H));
     with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
         fast32_ratio_kernel<o, s><<<grid, block, 0, st>>>(a, gd, dev);
     });
@@ -2111,6 +2149,19 @@ int pb_debug_plan_boxes(const pb_plan* plan, int32_t* table, int64_t capacity, i
     return PB_OK;
 }
 
+int pb_debug_plan_stage(const pb_plan* plan, int32_t out[8]) {
+    if (!plan || !out) return fail(PB_ERR_INVALID_ARGUMENT, "pb_debug_plan_stage: null pointer");
+    out[0] = plan->stage_bytes;
+    out[1] = plan->max_units;
+    out[2] = tiled_buffers(*plan, true, plan->separable && plan->tables != nullptr);
+    out[3] = plan->src.kind == PB_KIND_CAMERA && plan->sep1_cap3 > 0 ? plan->sep1_cap3 : plan->sep1_cap;
+    out[4] = plan->sep1_cap;
+    out[5] = plan->sep1_cap_one;
+    out[6] = boxes_stage_bytes(1);
+    out[7] = boxes_stage_bytes(2);
+    return PB_OK;
+}
+
 int pb_plan_remap_u8(const pb_plan* plan, const uint8_t* src, int64_t src_frame_stride, uint8_t* dst,
                      int64_t dst_frame_stride, int32_t n_frames, void* stream) {
     return plan_remap("pb_plan_remap_u8", plan, 1, src, src_frame_stride, dst, dst_frame_stride, n_frames, stream);
@@ -2165,7 +2216,7 @@ int pb_materialize_map_f64(const pb_remap_desc* desc, double* map, void* stream)
     rot.n = desc->n_rotations;
     std::memcpy(rot.m, desc->rotations, sizeof(rot.m));
     dim3 block(32, 8);
-    dim3 grid((g.W + block.x - 1) / block.x, (g.H + block.y - 1) / block.y);
+    dim3 grid((g.W + block.x - 1) / block.x, grid_rows(g.H));
     cudaStream_t st = (cudaStream_t)stream;
     double* luts = nullptr;
     if (cudaError_t eu = upload_lens_tables(&desc->out, &g, nullptr, nullptr, &luts, st, true))
@@ -2217,7 +2268,7 @@ int pb_debug_fast32_stats(const pb_remap_desc* desc, double stats[6], void* stre
     cudaMemsetAsync(dev, 0, 8 * sizeof(unsigned long long), st);
     unsigned* maxima = reinterpret_cast<unsigned*>(dev + 4);
     dim3 block(32, 8);
-    dim3 grid((a.out.W + block.x - 1) / block.x, (a.out.H + block.y - 1) / block.y);
+    dim3 grid((a.out.W + block.x - 1) / block.x, grid_rows(a.out.H));
     with_kinds(a.out.kind, a.src.kind, [&](auto o, auto s) {
         fast32_stats_kernel<o, s><<<grid, block, 0, st>>>(a, gd, maxima, dev);
     });
