@@ -22,7 +22,8 @@
  *  - images are HWC, tightly packed (row pitch = width * channels elements): uint8 for the _u8
  *    entry points; the _px entry points take elements of 1, 2, 4 or 8 bytes of any type (a pixel
  *    is copied as bytes, never converted), except from a double-fisheye source, whose blend is
- *    uint8 arithmetic;
+ *    uint8 arithmetic; the _typed entry points take a PB_ELEM_* type and blend a double-fisheye
+ *    source in that type;
  *  - coordinate maps are float64 (H, W, 3) = (latitude, longitude, invalid != 0), tightly packed
  *    (photonbend/core/__init__.py:42-49);
  *  - all work is enqueued on `stream` (a cudaStream_t, NULL = the default stream) and the call
@@ -127,7 +128,25 @@ enum {
     PB_LAUNCH_MAP = 13,       /* coordinate-map kernels: materialise, rotate, map_projection */
     PB_LAUNCH_DIAGNOSTIC = 14, /* pb_debug_fast32_stats */
     PB_LAUNCH_FRAMES = 15,    /* remap_frames_kernel: a rotation per frame (pb_plan_remap_frames_px) */
-    PB_LAUNCH_FAMILIES = 16
+    PB_LAUNCH_BLEND = 16,     /* remap_blend_kernel: a double-fisheye batch blended in its own type */
+    PB_LAUNCH_FAMILIES = 17
+};
+
+/* Element types of the _typed entry points (NumPy's names; bfloat16 as torch's). */
+enum {
+    PB_ELEM_UINT8 = 0,
+    PB_ELEM_INT8 = 1,
+    PB_ELEM_BOOL = 2,
+    PB_ELEM_UINT16 = 3,
+    PB_ELEM_INT16 = 4,
+    PB_ELEM_FLOAT16 = 5,
+    PB_ELEM_UINT32 = 6,
+    PB_ELEM_INT32 = 7,
+    PB_ELEM_FLOAT32 = 8,
+    PB_ELEM_UINT64 = 9,
+    PB_ELEM_INT64 = 10,
+    PB_ELEM_FLOAT64 = 11,
+    PB_ELEM_BFLOAT16 = 12
 };
 
 /* Kernels launched per family since the process started, for tests that must know which kernel
@@ -202,6 +221,26 @@ int pb_plan_remap_rows_px(const pb_plan *plan, int32_t elem_bytes, const void *s
 int pb_plan_remap_frames_px(const pb_plan *plan, int32_t elem_bytes, const double *frame_rotations,
                             const void *src, int64_t src_frame_stride, void *dst, int64_t dst_frame_stride,
                             int32_t n_frames, void *stream);
+/*
+ * The _px entry points with an element TYPE (PB_ELEM_*) in place of a width.  For a camera or
+ * equirect source they are the _px call with the type's width.  For a double-fisheye source the
+ * two lenses are blended in the source's own type: every output element is
+ *     (double)left * w_left + (double)right * w_right          (products rounded, no FMA)
+ * cast to the element type as NumPy's astype does on x86-64 (bfloat16: as torch's cast, through
+ * float32), with a missing lens sample counting as 0 and pixels outside the output's fov 0 -- the
+ * reference's blend (projection.py:459) with its final cast to uint8 replaced.  PB_ELEM_UINT8 is
+ * exactly the uint8 path.  A batch through a double-fisheye source is one launch of
+ * remap_blend_kernel whatever n_frames is.  Errors, before any device work: an unknown type ->
+ * PB_ERR_UNSUPPORTED; a null pointer, or a pointer / stride not a multiple of the type's width ->
+ * PB_ERR_INVALID_ARGUMENT; the rest as the _px call.
+ */
+int pb_plan_remap_typed(const pb_plan *plan, int32_t elem_type, const void *src, int64_t src_frame_stride, void *dst,
+                        int64_t dst_frame_stride, int32_t n_frames, void *stream);
+int pb_plan_remap_rows_typed(const pb_plan *plan, int32_t elem_type, const void *src, void *dst_band,
+                             int32_t row_begin, int32_t row_end, void *stream);
+int pb_plan_remap_frames_typed(const pb_plan *plan, int32_t elem_type, const double *frame_rotations,
+                               const void *src, int64_t src_frame_stride, void *dst, int64_t dst_frame_stride,
+                               int32_t n_frames, void *stream);
 void pb_plan_destroy(pb_plan *plan);
 
 /*
@@ -230,6 +269,9 @@ int pb_gather_from_map_u8(const pb_image_desc *src_desc, int32_t channels, doubl
 /* The same for elements of elem_bytes (1, 2, 4 or 8) bytes, with the errors of pb_plan_remap_px. */
 int pb_gather_from_map_px(const pb_image_desc *src_desc, int32_t channels, int32_t elem_bytes, double *map,
                           int32_t map_height, int32_t map_width, const void *src, void *dst, void *stream);
+/* The same for elements of type elem_type (PB_ELEM_*), as pb_plan_remap_typed. */
+int pb_gather_from_map_typed(const pb_image_desc *src_desc, int32_t channels, int32_t elem_type, double *map,
+                             int32_t map_height, int32_t map_width, const void *src, void *dst, void *stream);
 
 /*
  * map_projection (projection.py:550-599) on an explicit map (device, float64 map_height x

@@ -25,9 +25,15 @@ PB_ERR_UNSUPPORTED = 2
 PB_ERR_CUDA = 3
 PB_ERR_TOO_MANY_ROTATIONS = 4
 
+# element types of the _typed entry points (PB_ELEM_*), by NumPy / torch dtype name
+ELEM_TYPES = {
+    "uint8": 0, "int8": 1, "bool": 2, "uint16": 3, "int16": 4, "float16": 5, "uint32": 6, "int32": 7,
+    "float32": 8, "uint64": 9, "int64": 10, "float64": 11, "bfloat16": 12,
+}
+
 # kernel families of pb_debug_launch_counts, in the order of the PB_LAUNCH_* enum
 LAUNCH_FAMILIES = ("direct", "direct32", "generic", "tiled", "tiled_sep", "two_lens", "boxes1", "boxes2", "sep1",
-                   "chunk", "wide", "gather", "plan", "map", "diagnostic", "frames")
+                   "chunk", "wide", "gather", "plan", "map", "diagnostic", "frames", "blend")
 
 # every symbol include/pb_remap.h declares
 EXPORTS = (
@@ -53,6 +59,10 @@ EXPORTS = (
     "pb_plan_remap_rows_px",
     "pb_gather_from_map_px",
     "pb_plan_remap_frames_px",
+    "pb_plan_remap_typed",
+    "pb_plan_remap_rows_typed",
+    "pb_plan_remap_frames_typed",
+    "pb_gather_from_map_typed",
 )
 
 
@@ -148,6 +158,14 @@ def load():
     lib.pb_gather_from_map_px.argtypes = [ctypes.POINTER(ImageDesc), i32, i32, vp, i32, i32, vp, vp, vp]
     lib.pb_plan_remap_frames_px.restype = ctypes.c_int
     lib.pb_plan_remap_frames_px.argtypes = [vp, i32, ctypes.POINTER(ctypes.c_double), vp, i64, vp, i64, i32, vp]
+    lib.pb_plan_remap_typed.restype = ctypes.c_int
+    lib.pb_plan_remap_typed.argtypes = [vp, i32, vp, i64, vp, i64, i32, vp]
+    lib.pb_plan_remap_rows_typed.restype = ctypes.c_int
+    lib.pb_plan_remap_rows_typed.argtypes = [vp, i32, vp, vp, i32, i32, vp]
+    lib.pb_plan_remap_frames_typed.restype = ctypes.c_int
+    lib.pb_plan_remap_frames_typed.argtypes = [vp, i32, ctypes.POINTER(ctypes.c_double), vp, i64, vp, i64, i32, vp]
+    lib.pb_gather_from_map_typed.restype = ctypes.c_int
+    lib.pb_gather_from_map_typed.argtypes = [ctypes.POINTER(ImageDesc), i32, i32, vp, i32, i32, vp, vp, vp]
     _lib = lib
     return lib
 

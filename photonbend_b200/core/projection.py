@@ -12,8 +12,9 @@ asynchronous copies) or torch CUDA tensors (device resident: no copies at all, a
 elements may be bool, int8, uint8, int16, uint16, float16, bfloat16 (torch), int32, uint32,
 float32, int64, uint64 or float64: like the reference's fancy indexing, every output pixel is a
 bit-for-bit copy of the source pixel its index picks (0 where there is none).  A double-fisheye
-source must be uint8 (the reference casts its blend to uint8).  The result comes back in the same
-dtype and flavour as the source image.
+source blends its two lenses: the reference casts that blend to uint8, so a source of another
+dtype is refused unless it is made with ``keep_dtype=True``, which casts the blend to the source's
+own dtype instead.  The result comes back in the same dtype and flavour as the source image.
 """
 
 from __future__ import annotations
@@ -189,16 +190,22 @@ class DoubleCameraImage(_DeviceSampler):
     """A 360-degree camera frame: two opposite fisheye sensors stored side by side.
 
     Attributes:
-        image: the uint8 image, shape (height, width, channels); each half is width // 2 wide
-            (uint8 only: the reference blends the two lenses and casts the blend to uint8).
+        image: the image, shape (height, width, channels); each half is width // 2 wide.
         sensor_fov (float): field of view of ONE sensor in radians (> pi for full coverage).
         lens (Lens), forward_lens, reverse_lens: the lens model of both sensors.
         magnitude (float): always height / 2 (a ``magnitude=`` keyword is accepted and ignored).
         f_distance (float): focal distance in pixels.
+        keep_dtype (bool): how the two lenses' samples are blended.  False (the default, the
+            reference's behaviour): into uint8, and only a uint8 image is accepted (the reference
+            casts the float64 blend to uint8 whatever the input dtype, which would wrap wider
+            values mod 256).  True: into the image's own dtype -- any dtype the remap takes --
+            as ``(left.astype(float64) * w_left + right.astype(float64) * w_right).astype(dtype)``
+            with NumPy's casts (bfloat16: torch's); a uint8 image gives the default's bytes.
     """
 
-    def __init__(self, image_arr, sensor_fov: float, lens: Lens, **kwargs):
+    def __init__(self, image_arr, sensor_fov: float, lens: Lens, keep_dtype: bool = False, **kwargs):
         self.image = image_arr
+        self.keep_dtype = bool(keep_dtype)
         self.sensor_fov = sensor_fov
         self.lens = lens
         self.forward_lens = lens.forward_function
@@ -216,7 +223,7 @@ class DoubleCameraImage(_DeviceSampler):
         return engine.ImageGeometry(
             kind=_native.KIND_DOUBLE, height=height, width=width, lens=lens,
             fov=float(self.sensor_fov), f_distance=float(self.f_distance), table=table, table_max=table_max,
-            table_key=table_key)
+            table_key=table_key, keep_dtype=self.keep_dtype and role == "source")
 
     def _source_geometry(self):
         return self._geometry("source")

@@ -300,4 +300,119 @@ __device__ __forceinline__ unsigned char blend_u8(unsigned a, double wa, unsigne
     return cast_u8(__dadd_rn(__dmul_rn((double)a, wa), __dmul_rn((double)b, wb)));
 }
 
+// ---------------------------------------------------------------------------------- typed blend
+//
+// A double-fisheye source that keeps its dtype (pb_plan_remap_typed ...): the reference's blend
+// with its final cast to uint8 replaced by a cast to the source's own element type,
+//     (left.astype(float64) * wl + right.astype(float64) * wr).astype(image.dtype)
+// Elements travel as raw bits, zero-extended to 64; the type code (PB_ELEM_*) is uniform over a
+// launch, so its switches do not diverge.
+
+__host__ __device__ __forceinline__ int elem_type_bytes(int type) {
+    switch (type) {
+        case PB_ELEM_UINT8: case PB_ELEM_INT8: case PB_ELEM_BOOL: return 1;
+        case PB_ELEM_UINT16: case PB_ELEM_INT16: case PB_ELEM_FLOAT16: case PB_ELEM_BFLOAT16: return 2;
+        case PB_ELEM_UINT32: case PB_ELEM_INT32: case PB_ELEM_FLOAT32: return 4;
+        case PB_ELEM_UINT64: case PB_ELEM_INT64: case PB_ELEM_FLOAT64: return 8;
+        default: return 0;
+    }
+}
+
+// ndarray.astype(float64) of one element: exact for every type but the 64-bit integers, which
+// round to nearest (cvtsi2sd, and gcc's uint64 sequence, on x86-64)
+__device__ __forceinline__ double elem_to_f64(unsigned long long bits, int type) {
+    switch (type) {
+        case PB_ELEM_INT8: return (double)(signed char)bits;
+        case PB_ELEM_BOOL: return (bits & 0xffu) != 0 ? 1.0 : 0.0;
+        case PB_ELEM_UINT16: return (double)(unsigned short)bits;
+        case PB_ELEM_INT16: return (double)(short)bits;
+        case PB_ELEM_FLOAT16: {
+            double d;
+            asm("cvt.f64.f16 %0, %1;" : "=d"(d) : "h"((unsigned short)bits));
+            return d;
+        }
+        case PB_ELEM_BFLOAT16: return (double)__uint_as_float((unsigned)bits << 16);
+        case PB_ELEM_UINT32: return (double)(unsigned)bits;
+        case PB_ELEM_INT32: return (double)(int)(unsigned)bits;
+        case PB_ELEM_FLOAT32: return (double)__uint_as_float((unsigned)bits);
+        case PB_ELEM_UINT64: return __ull2double_rn(bits);
+        case PB_ELEM_INT64: return __ll2double_rn((long long)bits);
+        case PB_ELEM_FLOAT64: return __longlong_as_double((long long)bits);
+        default: return (double)(unsigned char)bits;
+    }
+}
+
+// ndarray.astype(type) of one float64 on x86-64 (NumPy's casts, bfloat16: torch's):
+//   8 / 16-bit integers  truncation to int32 (cvttsd2si), low bits kept; NaN, |v| >= 2^31 -> 0
+//   int32 / int64        truncation; NaN and out of range -> INT32_MIN / INT64_MIN
+//   uint32               truncation to int64, low 32 bits kept
+//   uint64               v < 2^63 (or NaN): truncation to int64; else trunc(v - 2^63) ^ 2^63
+//   float32 / float16    ONE rounding to nearest even (float16 straight from float64)
+//   bfloat16             two: to float32, then to bfloat16, both to nearest even
+//   bool                 v != 0 (NaN is True)
+__device__ __forceinline__ unsigned long long f64_to_elem(double v, int type) {
+    switch (type) {
+        case PB_ELEM_BOOL: return v != 0.0 ? 1ull : 0ull;
+        case PB_ELEM_UINT16: case PB_ELEM_INT16:
+            return fabs(v) < 2147483648.0 ? (unsigned long long)(__double2int_rz(v) & 0xffff) : 0ull;
+        case PB_ELEM_FLOAT16: {
+            unsigned short h;
+            asm("cvt.rn.f16.f64 %0, %1;" : "=h"(h) : "d"(v));
+            return h;
+        }
+        case PB_ELEM_BFLOAT16: {
+            unsigned short h;
+            asm("cvt.rn.bf16.f32 %0, %1;" : "=h"(h) : "f"(__double2float_rn(v)));
+            return h;
+        }
+        case PB_ELEM_INT32:
+            return (unsigned)(v > -2147483649.0 && v < 2147483648.0 ? __double2int_rz(v) : (int)0x80000000u);
+        case PB_ELEM_UINT32: return (unsigned)(unsigned long long)trunc_i64(v);
+        case PB_ELEM_FLOAT32: return __float_as_uint(__double2float_rn(v));
+        case PB_ELEM_INT64: return (unsigned long long)trunc_i64(v);
+        case PB_ELEM_UINT64:
+            if (!(v >= 9223372036854775808.0)) return (unsigned long long)trunc_i64(v);
+            return (unsigned long long)trunc_i64(__dadd_rn(v, -9223372036854775808.0)) ^ 0x8000000000000000ull;
+        case PB_ELEM_FLOAT64: return (unsigned long long)__double_as_longlong(v);
+        default: return cast_u8(v);  // uint8, int8
+    }
+}
+
+// One element of the blend: the products are rounded before the sum (no FMA, as blend_u8); a lens
+// without a sample contributes 0 * its weight
+__device__ __forceinline__ unsigned long long blend_elem(unsigned long long a, double wa, unsigned long long b, double wb,
+                                                         int type) {
+    return f64_to_elem(__dadd_rn(__dmul_rn(elem_to_f64(a, type), wa), __dmul_rn(elem_to_f64(b, type), wb)), type);
+}
+
+// raw element of `bytes` (1, 2, 4, 8) bytes at p, zero-extended; and the store of its low bytes
+__device__ __forceinline__ unsigned long long load_elem(const unsigned char* p, int bytes) {
+    switch (bytes) {
+        case 1: return __ldg(p);
+        case 2: return __ldg(reinterpret_cast<const unsigned short*>(p));
+        case 4: return __ldg(reinterpret_cast<const unsigned*>(p));
+        default: return __ldg(reinterpret_cast<const unsigned long long*>(p));
+    }
+}
+__device__ __forceinline__ void store_elem(unsigned char* p, int bytes, unsigned long long v) {
+    switch (bytes) {
+        case 1: *p = (unsigned char)v; break;
+        case 2: *reinterpret_cast<unsigned short*>(p) = (unsigned short)v; break;
+        case 4: *reinterpret_cast<unsigned*>(p) = (unsigned)v; break;
+        default: *reinterpret_cast<unsigned long long*>(p) = v; break;
+    }
+}
+
+// One pixel of C elements of a double-fisheye source, element type `type`: p0 / p1 the two lenses'
+// pixels (null: no sample), o the output pixel
+__device__ __forceinline__ void blend_px_typed(const unsigned char* p0, double w0, const unsigned char* p1, double w1,
+                                               unsigned char* o, int C, int type) {
+    const int E = elem_type_bytes(type);
+    for (int c = 0; c < C; ++c) {
+        const unsigned long long v0 = p0 ? load_elem(p0 + c * E, E) : 0ull;
+        const unsigned long long v1 = p1 ? load_elem(p1 + c * E, E) : 0ull;
+        store_elem(o + c * E, E, blend_elem(v0, w0, v1, w1, type));
+    }
+}
+
 }  // namespace pb

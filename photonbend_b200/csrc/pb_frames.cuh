@@ -17,8 +17,9 @@
 //                              (remap_direct32_kernel / remap_wide_kernel), indices parked in shared
 //                              memory; then the gather of remap_wide_kernel: a warp moves 32
 //                              consecutive pixels of a row as naturally aligned words of VEC bytes.
-//   double-fisheye source      resolve_lookup in place and the uint8 blend of the two lenses
-//                              (remap_direct_kernel), channel by channel.
+//   double-fisheye source      resolve_lookup in place and the blend of the two lenses
+//                              (remap_direct_kernel), channel by channel: blend_u8, or for a source
+//                              that keeps its type the typed blend (blend_px_typed).
 // The per-pixel functions are the ones every other kernel calls, so frame k is byte-identical to
 // the plan path for a descriptor with M_k appended to its rotations.
 //
@@ -59,6 +60,7 @@ struct FramesArgs {
     int px_bytes;    // P = channels x element bytes
     int vec;         // gather word: 1, 2, 4, 8 or 16 bytes
     int words;       // NW = P / VEC (<= 4)
+    int elem_type;   // double-fisheye source: PB_ELEM_* of its blend (uint8: blend_u8)
     FrameRotation frame[kFramesPerLaunch];
 };
 static_assert(sizeof(FramesArgs) <= 32764, "kernel parameters are limited to 32764 bytes");
@@ -148,6 +150,13 @@ __global__ void __launch_bounds__(256, PB_WIDE_MIN_CTAS) remap_frames_kernel(con
                 if (j >= a.out.W) break;
                 const Lookup L = resolve_lookup<OUT_KIND, SRC_KIND>(a.out, fast, rot, a.src, i, j);
                 const int off0 = xy_to_offset(L.xy0, a.src.W), off1 = xy_to_offset(L.xy1, a.src.W);
+                if (a.elem_type != PB_ELEM_UINT8) {
+                    const int P = a.px_bytes;
+                    blend_px_typed(off0 >= 0 ? sp + (long long)off0 * P : nullptr, L.w0,
+                                   off1 >= 0 ? sp + (long long)off1 * P : nullptr, L.w1,
+                                   dp + ((long long)i * a.out.W + j) * P, C, a.elem_type);
+                    continue;
+                }
                 const unsigned char* p0 = sp + (long long)max(off0, 0) * C;
                 const unsigned char* p1 = sp + (long long)max(off1, 0) * C;
                 unsigned char* o = dp + ((long long)i * a.out.W + j) * C;

@@ -24,6 +24,7 @@
 #include "pb_boxes.cuh"
 #include "pb_wide.cuh"
 #include "pb_frames.cuh"
+#include "pb_blend.cuh"
 
 namespace pb {
 
@@ -659,13 +660,14 @@ __global__ void __launch_bounds__(256) rotate_map_kernel(const __grid_constant__
 }
 
 // T: one element of the image (unsigned char; for a camera / equirect source also the unsigned
-// integer of a 2, 4 or 8-byte element -- the copy moves bytes, it converts nothing)
+// integer of a 2, 4 or 8-byte element -- the copy moves bytes, it converts nothing).  A
+// double-fisheye source is addressed in bytes and blends in elem_type (PB_ELEM_*: uint8 is blend_u8).
 template <int SRC_KIND, int C, typename T = unsigned char>
 __global__ void __launch_bounds__(256) gather_from_map_kernel(const __grid_constant__ SrcGeom src,
                                                               double* __restrict__ map, long long n,
                                                               const T* __restrict__ sp,
-                                                              T* __restrict__ dst) {
-    static_assert(SRC_KIND != PB_KIND_DOUBLE || sizeof(T) == 1, "the double-fisheye blend is uint8 arithmetic");
+                                                              T* __restrict__ dst, int elem_type) {
+    static_assert(SRC_KIND != PB_KIND_DOUBLE || sizeof(T) == 1, "a double-fisheye source is addressed in bytes");
     const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
     Ray r;
@@ -684,6 +686,17 @@ __global__ void __launch_bounds__(256) gather_from_map_kernel(const __grid_const
         if (off0 >= 0) copy_px<C, T>(dp, sp + (long long)off0 * C);
         else zero_px<C, T>(dp);
     } else {
+        if (elem_type != PB_ELEM_UINT8) {
+            const int P = C * elem_type_bytes(elem_type);
+            unsigned char* o = dst + p * P;
+            if (r.invalid) {
+                for (int k = 0; k < P; ++k) o[k] = 0;
+                return;
+            }
+            blend_px_typed(off0 >= 0 ? sp + (long long)off0 * P : nullptr, L.w0, off1 >= 0 ? sp + (long long)off1 * P : nullptr,
+                           L.w1, o, C, elem_type);
+            return;
+        }
         if (r.invalid) {
             zero_px<C>(dp);
             return;
@@ -855,20 +868,22 @@ static void launch_generic(const RemapArgs& a, cudaStream_t st) {
     PB_COUNT_LAUNCH(PB_LAUNCH_GENERIC);
 }
 
-// explicit-map gather: uint8 elements from any source, or elements of 2, 4 or 8 bytes from a
-// camera / equirect source
-static void launch_gather(const SrcGeom& s, int elem_bytes, double* map, long long n, const void* src, void* dst,
-                          cudaStream_t st) {
+// explicit-map gather: uint8 elements from any source, elements of 2, 4 or 8 bytes from a
+// camera / equirect source, or a double-fisheye source blended in elem_type (PB_ELEM_*)
+static void launch_gather(const SrcGeom& s, int elem_bytes, int elem_type, double* map, long long n, const void* src,
+                          void* dst, cudaStream_t st) {
     const int block = 256;
     const unsigned grid = (unsigned)((n + block - 1) / block);
     auto gather = [&](auto k, auto t) {
         using T = decltype(t);
         with_channels(s.C, [&](auto c) {
             gather_from_map_kernel<k, c, T><<<grid, block, 0, st>>>(s, map, n, static_cast<const T*>(src),
-                                                                      static_cast<T*>(dst));
+                                                                      static_cast<T*>(dst), elem_type);
         });
     };
-    if (elem_bytes == 1)
+    if (s.kind == PB_KIND_DOUBLE)
+        gather(Int<PB_KIND_DOUBLE>{}, (unsigned char)0);
+    else if (elem_bytes == 1)
         with_kind(s.kind, [&](auto k) { gather(k, (unsigned char)0); });
     else
         with_single_kind(s.kind, [&](auto k) { with_elem(elem_bytes, [&](auto t) { gather(k, t); }); });
@@ -1822,14 +1837,60 @@ static int plan_run_wide(const pb_plan& p, int elem_bytes, const void* src, int6
     return PB_OK;
 }
 
+// plan_run for a double-fisheye source blended in its own element type (pb_blend.cuh): ONE launch of
+// remap_blend_kernel for the whole batch (the plan's state is only read: no lock needed)
+static int plan_run_blend(const pb_plan& p, int elem_type, const void* src, int64_t src_frame_stride, void* dst,
+                          int64_t dst_frame_stride, int32_t n_frames, cudaStream_t st, int row_begin = 0,
+                          int row_end = -1) {
+    if (row_end < 0) row_end = p.out.H;
+    const long long tiles_y = (row_end - row_begin + kTileH - 1) / kTileH;
+    if (tiles_y >= 65536) return fail(PB_ERR_UNSUPPORTED, "blend remap: more than 65535 x 64 output rows in one call");
+    BlendArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.out = p.out;
+    a.src = p.src;
+    a.rot = p.rot;
+    a.fast = p.fast;
+    const bool sep = p.separable && p.tables != nullptr;
+    a.col_tab = sep ? p.tables : nullptr;
+    a.row_tab = sep ? p.tables + 2 * (size_t)p.out.W : nullptr;
+    a.src_px = static_cast<const unsigned char*>(src);
+    a.dst_px = static_cast<unsigned char*>(dst);
+    a.src_frame_stride = src_frame_stride;
+    a.dst_frame_stride = dst_frame_stride;
+    a.n_frames = n_frames;
+    a.row_begin = row_begin;
+    a.row_end = row_end;
+    a.channels = p.desc.channels;
+    a.elem_type = elem_type;
+    const dim3 grid((p.out.W + kTileW - 1) / kTileW, (unsigned)tiles_y);
+    auto launch = [&](auto e) {
+        if (sep) {
+            remap_blend_kernel<PB_KIND_EQUIRECT, true, e><<<grid, 256, 0, st>>>(a);
+        } else {
+            with_kind(p.out.kind, [&](auto o) { remap_blend_kernel<o, false, e><<<grid, 256, 0, st>>>(a); });
+        }
+    };
+    switch (elem_type_bytes(elem_type)) {
+        case 1: launch(Int<1>{}); break;
+        case 2: launch(Int<2>{}); break;
+        case 4: launch(Int<4>{}); break;
+        default: launch(Int<8>{}); break;
+    }
+    PB_COUNT_LAUNCH(PB_LAUNCH_BLEND);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "blend remap launch");
+    return PB_OK;
+}
+
 // A batch with a rotation per frame (pb_frames.cuh): frame k as the plan of the descriptor with
 // frame_rotations[k] appended to its rotations.  The constants are what pb_plan_create derives for
 // that descriptor, less the plan's calibration of the FP32-first tier (K = 16, the bound that holds
 // for every geometry).  Launches of up to kFramesPerLaunch frames; nothing allocated, nothing awaited
 // (the plan's state is only read: no lock needed).
-static int plan_run_frames(const pb_plan& p, int elem_bytes, const double* frame_rotations, const void* src,
-                           int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames,
-                           cudaStream_t st) {
+static int plan_run_frames(const pb_plan& p, int elem_bytes, int elem_type, const double* frame_rotations,
+                           const void* src, int64_t src_frame_stride, void* dst, int64_t dst_frame_stride,
+                           int32_t n_frames, cudaStream_t st) {
     const long long tiles_y = (p.out.H + kTileH - 1) / kTileH;
     if (tiles_y >= 65536) return fail(PB_ERR_UNSUPPORTED, "frames remap: more than 65535 x 64 output rows");
     const int n = p.desc.n_rotations;
@@ -1847,6 +1908,7 @@ static int plan_run_frames(const pb_plan& p, int elem_bytes, const double* frame
     a.src_frame_stride = src_frame_stride;
     a.dst_frame_stride = dst_frame_stride;
     a.px_bytes = p.desc.channels * elem_bytes;
+    a.elem_type = elem_type;
     // wide_vec's words are at least 2 bytes: uint8 pixels of odd size or at odd addresses move bytewise
     const bool multi = n_frames > 1;
     const unsigned long long odd = (unsigned long long)a.px_bytes | reinterpret_cast<uintptr_t>(src) |
@@ -1885,16 +1947,27 @@ static int plan_run_frames(const pb_plan& p, int elem_bytes, const double* frame
 // Arguments of the entry points that need no device: the element width, then for elements wider
 // than a byte the source kind, and pointers and strides against the width.  -> PB_OK, or the code
 // with pb_last_error set.
+// The element of a call: a width (the _u8 / _px entry points: type kUntyped) or a PB_ELEM_* type.
+constexpr int kUntyped = -1;
 static int check_elem_bytes(int32_t elem_bytes, const char* who) {
     if (elem_bytes != 1 && elem_bytes != 2 && elem_bytes != 4 && elem_bytes != 8)
         return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": elem_bytes must be 1, 2, 4 or 8 (got " +
                                             std::to_string(elem_bytes) + ")");
     return PB_OK;
 }
-static int check_wide(int32_t elem_bytes, int src_kind, const void* src, long long src_stride, const void* dst,
-                      long long dst_stride, const char* who) {
+static int check_elem_type(int32_t elem_type, const char* who) {
+    if (elem_type_bytes(elem_type) == 0)
+        return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": unknown element type " + std::to_string(elem_type));
+    return PB_OK;
+}
+// a double-fisheye source blended in its own type (remap_blend_kernel and the typed branches)
+static bool typed_blend(int src_kind, int elem_type) {
+    return src_kind == PB_KIND_DOUBLE && elem_type != kUntyped && elem_type != PB_ELEM_UINT8;
+}
+static int check_wide(int32_t elem_bytes, int elem_type, int src_kind, const void* src, long long src_stride,
+                      const void* dst, long long dst_stride, const char* who) {
     if (elem_bytes == 1) return PB_OK;
-    if (src_kind == PB_KIND_DOUBLE)
+    if (src_kind == PB_KIND_DOUBLE && elem_type == kUntyped)
         return fail(PB_ERR_UNSUPPORTED, std::string(who) +
                                             ": a double-fisheye source blends its two lenses into uint8 "
                                             "(projection.py:459); only elem_bytes == 1 is supported for it");
@@ -1912,15 +1985,20 @@ static int check_plan_device(const pb_plan* plan, const char* who) {
     return PB_OK;
 }
 
-// The bodies of the _u8 (elem_bytes == 1) and _px entry points; who names the entry point.
-static int plan_remap(const char* who, const pb_plan* plan, int32_t elem_bytes, const void* src,
+// The bodies of the _u8 (elem_bytes == 1), _px and _typed (elem_type != kUntyped, elem_bytes its
+// width) entry points; who names the entry point.
+static int plan_remap(const char* who, const pb_plan* plan, int32_t elem_bytes, int elem_type, const void* src,
                       int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames, void* stream) {
     if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
     if (!plan || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
-    if (int rc = check_wide(elem_bytes, plan->src.kind, src, src_frame_stride, dst, dst_frame_stride, who)) return rc;
+    if (int rc = check_wide(elem_bytes, elem_type, plan->src.kind, src, src_frame_stride, dst, dst_frame_stride, who))
+        return rc;
     if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": negative n_frames");
     if (n_frames == 0) return PB_OK;
     if (int rc = check_plan_device(plan, who)) return rc;
+    if (typed_blend(plan->src.kind, elem_type))
+        return plan_run_blend(*plan, elem_type, src, src_frame_stride, dst, dst_frame_stride, n_frames,
+                              (cudaStream_t)stream);
     if (elem_bytes > 1)
         return plan_run_wide(*plan, elem_bytes, src, src_frame_stride, dst, dst_frame_stride, n_frames,
                              (cudaStream_t)stream);
@@ -1928,32 +2006,35 @@ static int plan_remap(const char* who, const pb_plan* plan, int32_t elem_bytes, 
                     static_cast<uint8_t*>(dst), dst_frame_stride, n_frames, (cudaStream_t)stream);
 }
 
-static int plan_remap_frames(const char* who, const pb_plan* plan, int32_t elem_bytes, const double* frame_rotations,
-                             const void* src, int64_t src_frame_stride, void* dst, int64_t dst_frame_stride,
-                             int32_t n_frames, void* stream) {
+static int plan_remap_frames(const char* who, const pb_plan* plan, int32_t elem_bytes, int elem_type,
+                             const double* frame_rotations, const void* src, int64_t src_frame_stride, void* dst,
+                             int64_t dst_frame_stride, int32_t n_frames, void* stream) {
     if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
     if (!plan || !frame_rotations || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
     if (elem_bytes > 1)  // (uint8 has nothing to check, and then the plan is not read before n_frames is)
-        if (int rc = check_wide(elem_bytes, plan->src.kind, src, src_frame_stride, dst, dst_frame_stride, who)) return rc;
+        if (int rc = check_wide(elem_bytes, elem_type, plan->src.kind, src, src_frame_stride, dst, dst_frame_stride, who))
+            return rc;
     if (n_frames < 0) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": negative n_frames");
     if (n_frames == 0) return PB_OK;
     if (int rc = check_plan_device(plan, who)) return rc;
     if (plan->desc.n_rotations + 1 > PB_MAX_ROTATIONS)
         return fail(PB_ERR_TOO_MANY_ROTATIONS,
                     std::string(who) + ": the plan's rotations and the frame's are more than PB_MAX_ROTATIONS");
-    return plan_run_frames(*plan, elem_bytes, frame_rotations, src, src_frame_stride, dst, dst_frame_stride, n_frames,
-                           (cudaStream_t)stream);
+    return plan_run_frames(*plan, elem_bytes, typed_blend(plan->src.kind, elem_type) ? elem_type : PB_ELEM_UINT8,
+                           frame_rotations, src, src_frame_stride, dst, dst_frame_stride, n_frames, (cudaStream_t)stream);
 }
 
-static int plan_remap_rows(const char* who, const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band,
-                           int32_t row_begin, int32_t row_end, void* stream) {
+static int plan_remap_rows(const char* who, const pb_plan* plan, int32_t elem_bytes, int elem_type, const void* src,
+                           void* dst_band, int32_t row_begin, int32_t row_end, void* stream) {
     if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
     if (!plan || !src || !dst_band) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
-    if (int rc = check_wide(elem_bytes, plan->src.kind, src, 0, dst_band, 0, who)) return rc;
+    if (int rc = check_wide(elem_bytes, elem_type, plan->src.kind, src, 0, dst_band, 0, who)) return rc;
     if (row_begin < 0 || row_end > plan->out.H || row_begin > row_end)
         return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": rows outside the output image");
     if (row_begin == row_end) return PB_OK;
     if (int rc = check_plan_device(plan, who)) return rc;
+    if (typed_blend(plan->src.kind, elem_type))
+        return plan_run_blend(*plan, elem_type, src, 0, dst_band, 0, 1, (cudaStream_t)stream, row_begin, row_end);
     if (elem_bytes > 1)
         return plan_run_wide(*plan, elem_bytes, src, 0, dst_band, 0, 1, (cudaStream_t)stream, row_begin, row_end);
     return plan_run(*const_cast<pb_plan*>(plan), plan->tables, static_cast<const uint8_t*>(src), 0,
@@ -1961,12 +2042,12 @@ static int plan_remap_rows(const char* who, const pb_plan* plan, int32_t elem_by
 }
 
 static int gather_from_map(const char* who, const pb_image_desc* src_desc, int32_t channels, int32_t elem_bytes,
-                           double* map, int32_t map_height, int32_t map_width, const void* src, void* dst,
-                           void* stream) {
+                           int elem_type, double* map, int32_t map_height, int32_t map_width, const void* src,
+                           void* dst, void* stream) {
     if (int rc = check_elem_bytes(elem_bytes, who)) return rc;
     if (!src_desc || !map || !src || !dst) return fail(PB_ERR_INVALID_ARGUMENT, std::string(who) + ": null pointer");
     if (int rc = check_image(*src_desc, "src")) return rc;
-    if (int rc = check_wide(elem_bytes, src_desc->kind, src, 0, dst, 0, who)) return rc;
+    if (int rc = check_wide(elem_bytes, elem_type, src_desc->kind, src, 0, dst, 0, who)) return rc;
     // source_lookup packs a source pixel as row << 16 | column
     if (src_desc->height > 32767 || src_desc->width > 65535)
         return fail(PB_ERR_UNSUPPORTED, std::string(who) + ": source larger than 32767 rows x 65535 columns");
@@ -1980,7 +2061,8 @@ static int gather_from_map(const char* who, const pb_image_desc* src_desc, int32
     double* luts = nullptr;
     if (cudaError_t eu = upload_lens_tables(nullptr, nullptr, src_desc, &s, &luts, st, true))
         return cuda_fail(eu, (std::string(who) + " lens table").c_str());
-    launch_gather(s, elem_bytes, map, n, src, dst, st);
+    launch_gather(s, elem_bytes, typed_blend(src_desc->kind, elem_type) ? elem_type : PB_ELEM_UINT8, map, n, src, dst,
+                  st);
     cudaError_t e = cudaGetLastError();
     if (luts) cudaFreeAsync(luts, st);
     if (e != cudaSuccess) return cuda_fail(e, (std::string(who) + " launch").c_str());
@@ -2164,29 +2246,29 @@ int pb_debug_plan_stage(const pb_plan* plan, int32_t out[8]) {
 
 int pb_plan_remap_u8(const pb_plan* plan, const uint8_t* src, int64_t src_frame_stride, uint8_t* dst,
                      int64_t dst_frame_stride, int32_t n_frames, void* stream) {
-    return plan_remap("pb_plan_remap_u8", plan, 1, src, src_frame_stride, dst, dst_frame_stride, n_frames, stream);
+    return plan_remap("pb_plan_remap_u8", plan, 1, kUntyped, src, src_frame_stride, dst, dst_frame_stride, n_frames, stream);
 }
 
 int pb_plan_remap_rows_u8(const pb_plan* plan, const uint8_t* src, uint8_t* dst_band, int32_t row_begin, int32_t row_end,
                           void* stream) {
-    return plan_remap_rows("pb_plan_remap_rows_u8", plan, 1, src, dst_band, row_begin, row_end, stream);
+    return plan_remap_rows("pb_plan_remap_rows_u8", plan, 1, kUntyped, src, dst_band, row_begin, row_end, stream);
 }
 
 int pb_plan_remap_px(const pb_plan* plan, int32_t elem_bytes, const void* src, int64_t src_frame_stride, void* dst,
                      int64_t dst_frame_stride, int32_t n_frames, void* stream) {
-    return plan_remap("pb_plan_remap_px", plan, elem_bytes, src, src_frame_stride, dst, dst_frame_stride, n_frames,
+    return plan_remap("pb_plan_remap_px", plan, elem_bytes, kUntyped, src, src_frame_stride, dst, dst_frame_stride, n_frames,
                       stream);
 }
 
 int pb_plan_remap_rows_px(const pb_plan* plan, int32_t elem_bytes, const void* src, void* dst_band, int32_t row_begin,
                           int32_t row_end, void* stream) {
-    return plan_remap_rows("pb_plan_remap_rows_px", plan, elem_bytes, src, dst_band, row_begin, row_end, stream);
+    return plan_remap_rows("pb_plan_remap_rows_px", plan, elem_bytes, kUntyped, src, dst_band, row_begin, row_end, stream);
 }
 
 int pb_plan_remap_frames_px(const pb_plan* plan, int32_t elem_bytes, const double* frame_rotations, const void* src,
                             int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames,
                             void* stream) {
-    return plan_remap_frames("pb_plan_remap_frames_px", plan, elem_bytes, frame_rotations, src, src_frame_stride, dst,
+    return plan_remap_frames("pb_plan_remap_frames_px", plan, elem_bytes, kUntyped, frame_rotations, src, src_frame_stride, dst,
                              dst_frame_stride, n_frames, stream);
 }
 
@@ -2306,13 +2388,43 @@ int pb_rotate_map_f64(const double matrix[9], double* map_in, double* map_out, i
 
 int pb_gather_from_map_u8(const pb_image_desc* src_desc, int32_t channels, double* map, int32_t map_height,
                           int32_t map_width, const uint8_t* src, uint8_t* dst, void* stream) {
-    return gather_from_map("pb_gather_from_map_u8", src_desc, channels, 1, map, map_height, map_width, src, dst, stream);
+    return gather_from_map("pb_gather_from_map_u8", src_desc, channels, 1, kUntyped, map, map_height, map_width, src, dst, stream);
 }
 
 int pb_gather_from_map_px(const pb_image_desc* src_desc, int32_t channels, int32_t elem_bytes, double* map,
                           int32_t map_height, int32_t map_width, const void* src, void* dst, void* stream) {
-    return gather_from_map("pb_gather_from_map_px", src_desc, channels, elem_bytes, map, map_height, map_width, src, dst,
-                           stream);
+    return gather_from_map("pb_gather_from_map_px", src_desc, channels, elem_bytes, kUntyped, map, map_height, map_width,
+                           src, dst, stream);
+}
+
+// The _typed entry points: the _px bodies with the type's width, and the type
+int pb_plan_remap_typed(const pb_plan* plan, int32_t elem_type, const void* src, int64_t src_frame_stride, void* dst,
+                        int64_t dst_frame_stride, int32_t n_frames, void* stream) {
+    if (int rc = check_elem_type(elem_type, "pb_plan_remap_typed")) return rc;
+    return plan_remap("pb_plan_remap_typed", plan, elem_type_bytes(elem_type), elem_type, src, src_frame_stride, dst,
+                      dst_frame_stride, n_frames, stream);
+}
+
+int pb_plan_remap_rows_typed(const pb_plan* plan, int32_t elem_type, const void* src, void* dst_band, int32_t row_begin,
+                             int32_t row_end, void* stream) {
+    if (int rc = check_elem_type(elem_type, "pb_plan_remap_rows_typed")) return rc;
+    return plan_remap_rows("pb_plan_remap_rows_typed", plan, elem_type_bytes(elem_type), elem_type, src, dst_band,
+                           row_begin, row_end, stream);
+}
+
+int pb_plan_remap_frames_typed(const pb_plan* plan, int32_t elem_type, const double* frame_rotations, const void* src,
+                               int64_t src_frame_stride, void* dst, int64_t dst_frame_stride, int32_t n_frames,
+                               void* stream) {
+    if (int rc = check_elem_type(elem_type, "pb_plan_remap_frames_typed")) return rc;
+    return plan_remap_frames("pb_plan_remap_frames_typed", plan, elem_type_bytes(elem_type), elem_type, frame_rotations,
+                             src, src_frame_stride, dst, dst_frame_stride, n_frames, stream);
+}
+
+int pb_gather_from_map_typed(const pb_image_desc* src_desc, int32_t channels, int32_t elem_type, double* map,
+                             int32_t map_height, int32_t map_width, const void* src, void* dst, void* stream) {
+    if (int rc = check_elem_type(elem_type, "pb_gather_from_map_typed")) return rc;
+    return gather_from_map("pb_gather_from_map_typed", src_desc, channels, elem_type_bytes(elem_type), elem_type, map,
+                           map_height, map_width, src, dst, stream);
 }
 
 }  // extern "C"

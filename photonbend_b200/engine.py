@@ -34,6 +34,10 @@ class ImageGeometry:
     table: Optional[np.ndarray] = field(default=None, compare=False)
     table_max: float = 0.0
     table_key: bytes = b""  # digest of ``table``: what two geometries with user lenses are compared by
+    # double-fisheye source: blend the two lenses in the image's own dtype instead of refusing
+    # anything but uint8 (see check_source).  A property of the calls, not of the descriptor: one
+    # cached plan serves both settings.
+    keep_dtype: bool = False
 
     @property
     def output_width(self) -> int:
@@ -234,16 +238,27 @@ def elem_bytes(image) -> int:
 
 def check_source(src: ImageGeometry, image) -> int:
     """elem_bytes(image), after refusing what a source of geometry ``src`` cannot be: a
-    double-fisheye source must be uint8.  The reference blends its two lenses in float64 and casts
-    the blend to uint8 whatever the input dtype (projection.py:459), so a wider source would come
-    back as a uint8 image wrapped mod 256; neither that nor a dtype-preserving blend is offered."""
+    double-fisheye source must be uint8 unless its geometry has ``keep_dtype``.  The reference
+    blends its two lenses in float64 and casts the blend to uint8 whatever the input dtype
+    (projection.py:459), so a wider source would come back as a uint8 image wrapped mod 256; with
+    ``keep_dtype`` the blend is cast to the source's own dtype instead (``typed_blend``)."""
     width = elem_bytes(image)
     name = _dtype_name(image)
-    if src.kind == _native.KIND_DOUBLE and name != "uint8":
+    if src.kind == _native.KIND_DOUBLE and name != "uint8" and not src.keep_dtype:
         raise NotImplementedError(
             f"a double-fisheye source must be uint8 (got {name}): the reference blends the two lenses and "
-            "casts the blend to uint8 whatever the input dtype, which would wrap other values mod 256")
+            "casts the blend to uint8 whatever the input dtype, which would wrap other values mod 256; "
+            "pass keep_dtype=True to blend in the source's own dtype")
     return width
+
+
+def typed_blend(src: ImageGeometry, image) -> Optional[int]:
+    """The PB_ELEM_* type of ``image`` when a remap from ``src`` blends a double-fisheye source in
+    that type (the _typed entry points), else None (uint8, or no blend: the _u8 / _px ones)."""
+    name = _dtype_name(image)
+    if src.kind == _native.KIND_DOUBLE and src.keep_dtype and name != "uint8":
+        return _native.ELEM_TYPES[name]
+    return None
 
 
 def to_device(image):
@@ -298,7 +313,8 @@ def _check_out(out_dev, out_shape, src_dev) -> None:
 def remap_device(rays: RayPlan, src: ImageGeometry, src_dev, out_dev=None):
     """Fused remap on device tensors.  src_dev: CUDA tensor (H, W[, C]) or a batch (N, H, W, C) of
     an accepted dtype (ELEM_BYTES); returns (and fills) the CUDA output tensor of the same dtype.
-    One-byte elements take the uint8 kernels (pb_plan_remap_u8), wider ones pb_plan_remap_px."""
+    One-byte elements take the uint8 kernels (pb_plan_remap_u8), wider ones pb_plan_remap_px; a
+    double-fisheye source blended in its own dtype pb_plan_remap_typed."""
     torch = _torch()
     lib = _native.load()
     e = check_source(src, src_dev)
@@ -321,7 +337,11 @@ def remap_device(rays: RayPlan, src: ImageGeometry, src_dev, out_dev=None):
         stream = _stream_ptr(torch)
         src_ptr, dst_ptr = ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_void_p(out_dev.data_ptr())
         src_stride, dst_stride = ctypes.c_int64(h * w * c * e), ctypes.c_int64(oh * ow * c * e)
-        if e == 1:  # uint8, int8, bool: the same bytes
+        typed = typed_blend(src, src_dev)
+        if typed is not None:
+            _native.check(lib.pb_plan_remap_typed(plan, ctypes.c_int32(typed), src_ptr, src_stride, dst_ptr, dst_stride,
+                                                  ctypes.c_int32(frames), stream))
+        elif e == 1:  # uint8, int8, bool: the same bytes
             _native.check(lib.pb_plan_remap_u8(plan, src_ptr, src_stride, dst_ptr, dst_stride,
                                                ctypes.c_int32(frames), stream))
         else:
@@ -371,8 +391,10 @@ def remap_frames_device(rays: RayPlan, src: ImageGeometry, src_dev, matrices, ou
     desc = _remap_desc(rays, src, c)
     with torch.cuda.device(src_dev.device):
         plan = _plans.get(lib, desc, src_dev.device.index or 0, torch)
-        _native.check(lib.pb_plan_remap_frames_px(
-            plan, ctypes.c_int32(e), mats.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+        typed = typed_blend(src, src_dev)
+        call, elem = (lib.pb_plan_remap_frames_px, e) if typed is None else (lib.pb_plan_remap_frames_typed, typed)
+        _native.check(call(
+            plan, ctypes.c_int32(elem), mats.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
             ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_int64(h * w * c * e if batched else 0),
             ctypes.c_void_p(out_dev.data_ptr()), ctypes.c_int64(oh * ow * c * e), ctypes.c_int32(frames),
             _stream_ptr(torch)))
@@ -406,7 +428,10 @@ def remap_rows_device(rays: RayPlan, src: ImageGeometry, src_dev, row_begin: int
         plan = _plans.get(lib, desc, src_dev.device.index or 0, torch)
         src_ptr, dst_ptr = ctypes.c_void_p(src_dev.data_ptr()), ctypes.c_void_p(out_dev.data_ptr())
         rows = (ctypes.c_int32(row_begin), ctypes.c_int32(row_end), _stream_ptr(torch))
-        if e == 1:
+        typed = typed_blend(src, src_dev)
+        if typed is not None:
+            _native.check(lib.pb_plan_remap_rows_typed(plan, ctypes.c_int32(typed), src_ptr, dst_ptr, *rows))
+        elif e == 1:
             _native.check(lib.pb_plan_remap_rows_u8(plan, src_ptr, dst_ptr, *rows))
         else:
             _native.check(lib.pb_plan_remap_rows_px(plan, ctypes.c_int32(e), src_ptr, dst_ptr, *rows))
@@ -469,8 +494,14 @@ def gather_from_map_device(src: ImageGeometry, cmap_dev, src_dev, out_dev=None):
         raise ValueError(f"out must be a contiguous {_dtype_name(src_dev)} tensor of shape {out_shape} on {src_dev.device}")
     d = _native.ImageDesc()
     src.fill(d)
+    typed = typed_blend(src, src_dev)
     with torch.cuda.device(src_dev.device):
-        if e == 1:
+        if typed is not None:
+            _native.check(lib.pb_gather_from_map_typed(
+                ctypes.byref(d), ctypes.c_int32(c), ctypes.c_int32(typed), ctypes.c_void_p(cmap_dev.data_ptr()),
+                ctypes.c_int32(mh), ctypes.c_int32(mw), ctypes.c_void_p(src_dev.data_ptr()),
+                ctypes.c_void_p(out_dev.data_ptr()), _stream_ptr(torch)))
+        elif e == 1:
             _native.check(lib.pb_gather_from_map_u8(
                 ctypes.byref(d), ctypes.c_int32(c), ctypes.c_void_p(cmap_dev.data_ptr()),
                 ctypes.c_int32(mh), ctypes.c_int32(mw), ctypes.c_void_p(src_dev.data_ptr()),
