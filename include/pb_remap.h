@@ -80,8 +80,9 @@ typedef struct pb_image_desc {
     int32_t width;     /* pixels (a double image holds two width/2 halves side by side) */
     double fov;        /* radians: full field of view (camera) or per-sensor fov (double) */
     double f_distance; /* pixels per focal unit = magnitude / lens_forward(fov / 2) */
-    /* PB_LENS_TABLE only (otherwise NULL / 0): lens_table_n >= 2 float64 samples in HOST memory of
-     * the one lens function this side of the remap evaluates, at x_k = k * lens_table_max /
+    /* PB_LENS_TABLE only (otherwise NULL / 0): 2 <= lens_table_n <= 2^24 float64 samples in HOST
+     * memory of the one lens function this side of the remap evaluates (lens_table_max finite and
+     * > 0, else PB_ERR_INVALID_ARGUMENT), at x_k = k * lens_table_max /
      * (lens_table_n - 1): as `out`, the lens's reverse function (radius in focal units ->
      * latitude); as `src`, its forward function (latitude -> radius in focal units).  The kernel
      * interpolates linearly and clamps x to [0, lens_table_max].  Copied during the call (plans

@@ -72,6 +72,7 @@ def gather_px(e, sd=image(), ch=3, m=FAKE, mh=4, mw=4, src=FAKE, dst=FAKE):
 
 BIG = 2**31 - 1
 TABLE_MSG = "PB_LENS_TABLE needs lens_table (>= 2 samples) and lens_table_max > 0"
+TABLE = ctypes.cast(FAKE, ctypes.POINTER(ctypes.c_double))  # never dereferenced: the checks come first
 DOUBLE_MSG = ("a double-fisheye source blends its two lenses into uint8 (projection.py:459); "
               "only elem_bytes == 1 is supported for it")
 ALIGN_MSG = "pointer or stride not a multiple of elem_bytes"
@@ -93,6 +94,18 @@ CASES = {
     "remap-src-kind+channels": (remap(desc(src=image(3), channels=0)), INVALID, "src: unknown image kind"),
     "remap-src-lens+size": (remap(desc(src=image(lens=7, height=40000))), INVALID, "src: unknown lens"),
     "remap-src-table": (remap(desc(src=image(lens=N.LENS_TABLE))), INVALID, "src: " + TABLE_MSG),
+    "remap-src-table-2^24+1": (remap(desc(src=image(lens=N.LENS_TABLE, lens_table=TABLE, lens_table_n=(1 << 24) + 1,
+                                                    lens_table_max=3.0))), INVALID, "src: " + TABLE_MSG),
+    "remap-out-table-inf-max": (remap(desc(out=image(lens=N.LENS_TABLE, lens_table=TABLE, lens_table_n=2,
+                                                     lens_table_max=float("inf"))), n=0), INVALID, "out: " + TABLE_MSG),
+    "remap-src-table-nan-max": (remap(desc(src=image(lens=N.LENS_TABLE, lens_table=TABLE, lens_table_n=17,
+                                                     lens_table_max=float("nan")))), INVALID, "src: " + TABLE_MSG),
+    "remap-src-table-zero-max": (remap(desc(src=image(N.KIND_DOUBLE, lens=N.LENS_TABLE, lens_table=TABLE,
+                                                      lens_table_n=17, lens_table_max=0.0))), INVALID, "src: " + TABLE_MSG),
+    "remap-out-table-neg-max": (remap(desc(out=image(lens=N.LENS_TABLE, lens_table=TABLE, lens_table_n=1 << 24,
+                                                     lens_table_max=-1.0))), INVALID, "out: " + TABLE_MSG),
+    "gather-table-2^24+1": (gather_u8(sd=image(lens=N.LENS_TABLE, lens_table=TABLE, lens_table_n=(1 << 24) + 1,
+                                               lens_table_max=3.0)), INVALID, "src: " + TABLE_MSG),
     "remap-src-double-width": (remap(desc(src=image(N.KIND_DOUBLE, width=1))), INVALID,
                                "src: a double image needs width >= 2"),
     "remap-equirect-ignores-lens": (remap(desc(src=image(N.KIND_EQUIRECT, lens=99)), n=0), N.PB_OK, None),

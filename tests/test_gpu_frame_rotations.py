@@ -10,6 +10,7 @@ import pytest
 
 import case_matrix
 import helpers
+import table_oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -56,16 +57,31 @@ def _matrices(n, seed):
     return np.stack(mats[:n])
 
 
-def _rays_geom(og, rots, sg, shape, user_lens=False):
+def _user_source(sg, shape):
+    """a camera source of sg's geometry with equisolid as a Lens of user callables: PB_LENS_TABLE"""
     from photonbend_b200.core.lens import Lens
     from photonbend_b200.core.projection import CameraImage
 
-    if user_lens:  # equisolid as a Lens of user callables: PB_LENS_TABLE
-        lens = Lens(lambda t: 2 * np.sin(t / 2), lambda r: 2 * np.arcsin(r / 2))
-        src = CameraImage(np.zeros(shape, np.uint8), sg["fov"], lens, magnitude=sg.get("magnitude"))
-    else:
-        src = helpers.product_image(sg, np.zeros(shape, np.uint8))
+    lens = Lens(lambda t: 2 * np.sin(t / 2), lambda r: 2 * np.arcsin(r / 2))
+    return CameraImage(np.zeros(shape, np.uint8), sg["fov"], lens, magnitude=sg.get("magnitude"))
+
+
+def _rays_geom(og, rots, sg, shape, user_lens=False):
+    src = _user_source(sg, shape) if user_lens else helpers.product_image(sg, np.zeros(shape, np.uint8))
     return helpers.product_map(og, rots).rays, src._source_geometry()
+
+
+def _check_table_oracle(got, frames, og, rots, sg, mats, what):
+    """frame k of a user-lens remap against the table oracle of the map rotated by mats[k] (any 9
+    doubles: numpy_port.rotate_map is the reference's arithmetic, orthonormal or not)"""
+    from oracle import numpy_port
+
+    got = got.cpu().numpy()
+    with table_oracle.patched():
+        for k, m in enumerate(mats):
+            oracle = helpers.Oracle(og, rots, sg)
+            oracle.cmap = numpy_port.rotate_map(oracle.cmap, np.asarray(m, dtype=np.float64))
+            oracle.check(got[k], frames[k], f"{what}: frame {k}")
 
 
 def _per_frame(torch, rays, geom, src_dev, mats, stride0=False):
@@ -167,8 +183,11 @@ def test_non_orthonormal_frame_lens_table_and_stride_zero(torch_cuda):
         for rots in ROTATION_SETS[:2]:
             rays, geom = _rays_geom(og, rots, sg, shape, user_lens)
             what = f"user lens {user_lens} {rots}"
-            _assert_frames_equal(engine.remap_frames_device(rays, geom, batch, mats),
-                                 _per_frame(torch, rays, geom, batch, mats), what)
+            got = engine.remap_frames_device(rays, geom, batch, mats)
+            _assert_frames_equal(got, _per_frame(torch, rays, geom, batch, mats), what)
+            if user_lens:
+                sg_table = table_oracle.geom_of(_user_source(sg, shape))
+                _check_table_oracle(got, batch.cpu().numpy(), og, rots, sg_table, mats, what)
             # source stride 0: seven views of one image
             _assert_frames_equal(engine.remap_frames_device(rays, geom, one, mats),
                                  _per_frame(torch, rays, geom, one, mats, stride0=True), what + " stride 0")
@@ -177,11 +196,14 @@ def test_non_orthonormal_frame_lens_table_and_stride_zero(torch_cuda):
     from photonbend_b200.core.projection import CameraImage, PanoramaImage
 
     lens = Lens(lambda t: 2 * np.sin(t / 2), lambda r: 2 * np.arcsin(r / 2))
-    rays = CameraImage(np.zeros((OUT_H, OUT_W, 3), np.uint8), rad(180), lens, magnitude=150.5).get_coordinate_map().rays
+    out_image = CameraImage(np.zeros((OUT_H, OUT_W, 3), np.uint8), rad(180), lens, magnitude=150.5)
+    rays = out_image.get_coordinate_map().rays
     geom = PanoramaImage(np.zeros((192, 384, 3), np.uint8))._source_geometry()
     pano = torch.from_numpy(rng.integers(0, 256, (7, 192, 384, 3), dtype=np.uint8)).cuda()
-    _assert_frames_equal(engine.remap_frames_device(rays, geom, pano, mats),
-                         _per_frame(torch, rays, geom, pano, mats), "output lens table")
+    got = engine.remap_frames_device(rays, geom, pano, mats)
+    _assert_frames_equal(got, _per_frame(torch, rays, geom, pano, mats), "output lens table")
+    _check_table_oracle(got, pano.cpu().numpy(), table_oracle.geom_of(out_image), (), _src_geom("equirect"), mats,
+                        "output lens table")
 
 
 # ------------------------------------------------------------------------------------ 4. NumPy oracle
